@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- benchmark of the grad / curvature stencil path (BASELINE.json metric: Gcells/s over all AMR levels).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference] [--dump-outputs DIR]
 
 Workloads (--workload; the default, config2, is the configuration the metric is quoted on):
   config2      grad, uniform 512^3, 64 boxes of 128^3, 5 components                         (BASELINE configs[1])
@@ -43,6 +43,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the tree as it found it (it may be read-only)
 
 UNIT = "Gcells/s"
 HASH_FILE = os.path.join(ROOT, "tests", "golden", "bench_hashes.json")
@@ -283,9 +284,49 @@ class Ctx:
         return int(t.item()) & (2 ** 64 - 1)
 
 
-def measure(cx, spec, steps, warmup, e2e_steps=0, sampler=None):
+DUMP_BYTES = 60_000_000          # --dump-outputs: the values of all files together; with the .npy headers they stay below 64 MB
+DUMP_SEED = 20261020
+
+
+def output_names(spec):
+    """Names of the output components in Field order: gx, gy, gz, |grad| per variable, or the five curvature outputs."""
+    if spec["kind"] == "grad":
+        return ["%s_%s" % (v, k) for v in spec["names"] for k in ("gx", "gy", "gz", "gradmag")]
+    v = spec["names"][0]
+    return ["Progress", "MeanCurvature_" + v, "FlameNormalX_" + v, "FlameNormalY_" + v, "FlameNormalZ_" + v]
+
+
+def dump_cells(cells, ncomp):
+    """Host-concat indices of the cells --dump-outputs writes: all of them, or a sorted seeded sample within DUMP_BYTES."""
+    n = min(cells, DUMP_BYTES // (8 * ncomp))
+    return np.arange(cells) if n == cells else np.sort(np.random.default_rng(DUMP_SEED).choice(cells, n, replace=False))
+
+
+def dump_outputs(spec, H, fout, out_dir):
+    """Write every output component of the last step as out_dir/<name>.npy (float64, valid cells in host-concat order:
+    levels, boxes, z-y-x).  Workloads larger than DUMP_BYTES keep the same seeded sample of cells in every component, so
+    two builds run with the same arguments can be compared value for value."""
+    names = output_names(spec)
+    idx = dump_cells(H.num_cells, len(names))
+    os.makedirs(out_dir, exist_ok=True)
+    vals = np.empty((len(names), idx.size))
+    off = 0
+    for l, lv in enumerate(H.levels):
+        for b, (lo, hi) in enumerate(lv.boxes):
+            m = (hi[0] - lo[0] + 1) * (hi[1] - lo[1] + 1) * (hi[2] - lo[2] + 1)
+            i0, i1 = np.searchsorted(idx, [off, off + m])
+            if i1 > i0:
+                for c in range(len(names)):
+                    vals[c, i0:i1] = fout.download_box(l, b, c).ravel()[idx[i0:i1] - off]
+            off += m
+    for c, name in enumerate(names):
+        np.save(os.path.join(out_dir, name + ".npy"), vals[c])
+
+
+def measure(cx, spec, steps, warmup, e2e_steps=0, sampler=None, dump_dir=None):
     """Run one workload on the current rank layout.  Returns a dict with the device-resident timing, the dominant kernel's
-    share, the optional host-buffer (e2e) timing and the output fingerprint."""
+    share, the optional host-buffer (e2e) timing and the output fingerprint; with dump_dir, also writes the outputs of the
+    last timed step there (dump_outputs)."""
     torch, dist, capi, multigpu = cx.torch, cx.dist, cx.capi, cx.multigpu
     rank, world, stream = cx.rank, cx.world, cx.stream
     kind, names = spec["kind"], spec["names"]
@@ -372,6 +413,8 @@ def measure(cx, spec, steps, warmup, e2e_steps=0, sampler=None):
 
     # ---- fingerprint of the outputs of the last step ----
     res["output_hash"] = "%016x" % cx.sum_hash(fout.hash(0, nout))
+    if dump_dir is not None:
+        dump_outputs(spec, H, fout, dump_dir)
 
     # ---- e2e: host buffers through the C ABI (pinned H2D of inputs, hot path, D2H of all outputs) -------------
     if e2e_steps > 0:
@@ -548,9 +591,16 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary workloads")
     ap.add_argument("--only-extra", default=None, help="run just one workload device-resident and print its short record (profiling aid)")
     ap.add_argument("--write-hashes", action="store_true", help="(N=1) record this run's fingerprints in tests/golden/bench_hashes.json")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="(N=1) write the outputs of the last timed step of the workload as DIR/<name>.npy (float64; a fixed seeded "
+                         "sample of cells when all of them would exceed %d MB)" % (DUMP_BYTES // 1000000))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     filter_only = args.only_extra == "filter3"
+    if args.dump_outputs and (filter_only or args.impl == "reference" or args.gpus > 1):
+        ap.error("--dump-outputs covers the grad and curvature workloads of the B200 arm on one GPU")
     spec = workload_spec("config2" if filter_only else (args.only_extra or args.workload))
     if args.impl == "reference":
         return reference_arm(args, spec)
@@ -586,7 +636,7 @@ def main():
         print(json.dumps(measure_filter(cx, args.steps, args.warmup, cpu_baseline=not args.no_cpu_baseline)))
         return
     if args.only_extra:
-        r = measure(cx, spec, args.steps, args.warmup)
+        r = measure(cx, spec, args.steps, args.warmup, dump_dir=args.dump_outputs)
         r["steps"] = args.steps
         if rank == 0:
             print(json.dumps(short(args.only_extra, r)))
@@ -595,7 +645,7 @@ def main():
         return
 
     sampler = ClockSampler(local_rank) if rank == 0 else None
-    r = measure(cx, spec, args.steps, args.warmup, e2e_steps=args.e2e_steps, sampler=sampler)
+    r = measure(cx, spec, args.steps, args.warmup, e2e_steps=args.e2e_steps, sampler=sampler, dump_dir=args.dump_outputs)
     r["steps"] = args.steps
     if sampler is not None:
         sampler.stop_flag = True

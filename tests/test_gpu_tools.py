@@ -174,19 +174,19 @@ def test_amrex_linked_curvature_do_smooth(amrex_exes, tmp_path):
         assert bit_equal(_flat(a, n), _flat(b, n)), n
 
 
-# ---- BASELINE-size parity against the compiled, unmodified reference run on the same box ----------------------------------
+# ---- BASELINE-size parity: the C restatement of the reference's arithmetic (oracle/, bit-exact against the reference's
+#      golden vectors in tests/test_oracle_golden.py) on the same hierarchy; also the compiled reference itself where it was built
 def _big_tmp():
     import tempfile
     base = "/dev/shm" if os.path.isdir("/dev/shm") else None
     return tempfile.TemporaryDirectory(prefix="pa_full_", dir=base)
 
 
-@pytest.mark.skipif(not O.have_ref(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("config", ["configs1_512", "configs4_small_boxes"])
 def test_full_size_grad_vs_reference_executable(exes, config):
     """BASELINE configs[1] (uniform 512^3 in 128^3 boxes, one of its variables) and configs[4] (4 levels, ratios 2/4/2,
-    128^3 base, 16^3 boxes) at FULL size: the reference tool and the B200 tool read the same plotfile, AMReX's own fcompare
-    must print PLOTFILE AGREE (every output bit equal)."""
+    128^3 base, 16^3 boxes) at FULL size: every output bit of the B200 tool equals the oracle's; where the reference tool
+    was built, it reads the same plotfile and AMReX's own fcompare must print PLOTFILE AGREE."""
     from peleanalysis_b200 import synth
     if config == "configs1_512":
         pf, var = synth.make_hierarchy(512, [], [], 128, ("temp",)), "temp"
@@ -196,30 +196,43 @@ def test_full_size_grad_vs_reference_executable(exes, config):
     with _big_tmp() as tmp:
         d = os.path.join(tmp, "plt")
         plotfile.write_plotfile(d, pf)
+        OH = O.OracleHier(pf)
+        want = OH.grad(OH.flatten(pf.comp(var)))
         del pf
         _run(exes[0], "infile=" + d, "gradVar=" + var, "outfile=" + os.path.join(tmp, "b200"), cwd=tmp)
-        O.run_ref("grad", d, os.path.join(tmp, "ref"), gradVar=var)
-        p = subprocess.run([O.ref_exe("fcompare.ref.ex"), os.path.join(tmp, "b200"), os.path.join(tmp, "ref")], capture_output=True, text=True)
-        assert "PLOTFILE AGREE" in p.stdout, p.stdout[-1500:]
+        for c, n in enumerate([var + "_gx", var + "_gy", var + "_gz", "||grad%s||" % var]):
+            got = _flat(plotfile.read_plotfile(os.path.join(tmp, "b200"), comps=[n]), n)
+            assert bit_equal(got, want[c]), (config, n, max_rel(got, want[c]))
+        del want
+        if O.have_ref():
+            O.run_ref("grad", d, os.path.join(tmp, "ref"), gradVar=var)
+            p = subprocess.run([O.ref_exe("fcompare.ref.ex"), os.path.join(tmp, "b200"), os.path.join(tmp, "ref")], capture_output=True, text=True)
+            assert "PLOTFILE AGREE" in p.stdout, p.stdout[-1500:]
 
 
-@pytest.mark.skipif(not O.have_ref(), reason="oracle/_ref not built")
 def test_full_size_curvature_vs_reference_executable(exes):
     """BASELINE configs[2] at full size (3 levels, 256^3 base, ratio 2, 64^3 boxes): every output the reference initialises
-    (it leaves SmoothedProgress and, without do_gaussCurv, GaussianCurvature unset) bit for bit."""
+    (it leaves SmoothedProgress and, without do_gaussCurv, GaussianCurvature unset) bit for bit, against the oracle and,
+    where it was built, the reference tool."""
     from peleanalysis_b200 import synth
     pf = synth.config3(256, 64)
+    names = ["Progress", "MeanCurvature_temp", "FlameNormalX_temp", "FlameNormalY_temp", "FlameNormalZ_temp"]
     with _big_tmp() as tmp:
         d = os.path.join(tmp, "plt")
         plotfile.write_plotfile(d, pf)
+        OH = O.OracleHier(pf)
+        pmin, pmax = plotfile.file_min_max(d, "temp", len(pf.levels))      # the tool's default progMin / progMax
+        want = OH.curvature(OH.flatten(pf.comp("temp")), pmin, pmax)
         del pf
         _run(exes[1], "infile=" + d, "progressName=temp", "outfile=" + os.path.join(tmp, "b200"), cwd=tmp)
-        O.run_ref("curvature", d, os.path.join(tmp, "ref"), progressName="temp")
-        names = ["Progress", "MeanCurvature_temp", "FlameNormalX_temp", "FlameNormalY_temp", "FlameNormalZ_temp"]
         a = plotfile.read_plotfile(os.path.join(tmp, "b200"), comps=names)
-        b = plotfile.read_plotfile(os.path.join(tmp, "ref"), comps=names)
-        for n in names:
-            assert bit_equal(_flat(a, n), _flat(b, n)), n
+        for c, n in enumerate(names):
+            assert bit_equal(_flat(a, n), want[c]), (n, max_rel(_flat(a, n), want[c]))
+        if O.have_ref():
+            O.run_ref("curvature", d, os.path.join(tmp, "ref"), progressName="temp")
+            b = plotfile.read_plotfile(os.path.join(tmp, "ref"), comps=names)
+            for n in names:
+                assert bit_equal(_flat(a, n), _flat(b, n)), n
 
 
 @pytest.mark.parametrize("name", ["filter_c1", "filter_c1_corner_gauss", "filter_c3", "filter_c3_subset", "filter_c3_pc_samefgr", "filter_ratio4"])

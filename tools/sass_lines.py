@@ -5,6 +5,7 @@ Joins `ncu -i X.ncu-rep --page source --csv --kernel-name ... --launch-count 1` 
 usage: tools/sass_lines.py source_page.csv cubin mangled_name_fragment [top]"""
 import collections
 import csv
+import os
 import re
 import subprocess
 import sys
@@ -49,7 +50,7 @@ def main():
         per[lines[i]] += ex[i]
         pst[lines[i]] += st[i]
     tot, tst = sum(per.values()) or 1, sum(pst.values()) or 1
-    src = open("/root/repo/peleanalysis_b200/csrc/stencil_tma.cu").read().splitlines()
+    src = open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "peleanalysis_b200", "csrc", "stencil_tma.cu")).read().splitlines()
     for ln, c in per.most_common(top):
         text = src[ln - 1].strip()[:110] if ln and ln <= len(src) else "?"
         print("%5s %6.2f%% inst %6.2f%% stall | %s" % (ln, 100.0 * c / tot, 100.0 * pst[ln] / tst, text))
