@@ -204,7 +204,8 @@ int pa_curvature_scratch(pa_hier *h, int which, pa_field **f);
  * layers of every level by FillPatch rules on a NON-periodic geometry (PP/Utility/PltFileManager/PltFileManager.cpp:118-120)
  * and applies PelePhysics' Filter box by box.  Create the hierarchy with is_per = {0,0,0} on the re-chopped grids, allocate the
  * input field with nghost >= the widest level's nGrow and upload the plotfile's valid data; then per level
- * pa_fill_patch + pa_filter.  Results are bit-identical to the reference tool's.  Single-rank. */
+ * pa_fill_patch + pa_filter.  Results are bit-identical to the reference tool's.  On several ranks (boxes of every level
+ * distributed, e.g. by pa_sfc_distribute) each pa_fill_patch is preceded by its exchange, below. */
 /* Filter::Filter(type, fgr) (PP/Utility/Filter/Filter.H:56-111 + Filter.cpp:3-404): ghost width and the 2*ngrow+1 weights of
  * filter_types 0..10 (1 box, 2 Gaussian, 3-10 the Sagaut & Grohens approximations).  Returns the number of weights
  * (weights may be NULL to query) or a negative pa_status. */
@@ -217,8 +218,23 @@ int pa_boxes_max_size(int nboxes, const int *boxes, int max_grid_size, int *out_
  * cell; else interpolation from the VALID cells of level lev-1 (interp_type 1: MFCellConsLinInterp with the monotonised-central
  * slope, AX/AmrCore/AMReX_MFInterp_3D_C.H:178-260; 0: MFPCInterp); first-order extrapolation outside the domain
  * (AX/Base/AMReX_PhysBCFunct.H:406-640, AMReX_FilCC_3D_C.H), on the coarse patch as well.  Levels are independent of each
- * other (only valid coarse data is read).  PA_ERR_ARG if the coarse level does not cover a needed coarse patch. */
+ * other (only valid coarse data is read).  PA_ERR_ARG if the coarse level does not cover a needed coarse patch (decided over
+ * every box of the level: on several ranks all fail or none does), or, on several ranks, if this rank receives cells for the
+ * fill and the recv slab was not marked for exactly this (field, comp, ncomp, lev, nghost, interp_type). */
 int pa_fill_patch(pa_field *f, int comp, int ncomp, int lev, int nghost, int interp_type);
+/* Several ranks: the communication of FabArray::FillPatchTwoLevels (ParallelCopy of the coarse patches and FillBoundary of
+ * the fine level, AX/AmrCore/AMReX_FillPatchUtil_I.H; AX/Base/AMReX_FabArrayCommI.H) as one packed-slab exchange per fill:
+ *   pa_fill_patch_pack -> transport (NCCL send/recv or pa_copy_async of each peer's segment) -> pa_fill_patch_mark_received
+ *   -> pa_fill_patch
+ * Sources owned by another rank than their destination box's -- same-level neighbours and coarse cells of the patches --
+ * travel [cell][comp] in doubles; offsets (nranks+1 each) locate each peer's segment.  The slabs are shared by every fill
+ * of the hierarchy and grow to the largest plan asked for: query the buffers again after asking for another plan.  Any pack
+ * invalidates the mark of the previous fill.  On one rank the offsets are all zero, the slabs NULL and pack / mark do
+ * nothing, so callers need a single code path. */
+int pa_fill_patch_exchange_buffers(pa_field *f, int ncomp, int lev, int nghost, int interp_type, double **send_slab, double **recv_slab,
+                                   int64_t *send_offsets /*nranks+1*/, int64_t *recv_offsets /*nranks+1*/);
+int pa_fill_patch_pack(pa_field *f, int comp, int ncomp, int lev, int nghost, int interp_type);
+int pa_fill_patch_mark_received(pa_field *f, int comp, int ncomp, int lev, int nghost, int interp_type);
 /* Filter::apply_filter on every box of level `lev` (PP/Utility/Filter/Filter.H:28-50, Filter.cpp:462-491):
  * out = sum over (n, m, l) of w[l]*w[m]*w[n] * in(i+l, j+m, k+n), the reference's summation order.  `in` must hold ngrow
  * filled ghost layers (pa_fill_patch); out's ghost cells are not written. */
@@ -274,6 +290,9 @@ int pa_debug_links(pa_hier *h, int lev, int box, int out[30]);
  * each recv-slab slot expects, encoded (source level << 56 | global box << 32 | linear index in the box's valid
  * region).  which = 0: send slab, 1: recv slab.  Returns the slab length in cells (writes min(len, out_len)). */
 int64_t pa_debug_exchange_ids(pa_hier *h, int which, int64_t *out, int64_t out_len);
+/* The same for the exchange of pa_fill_patch(lev, nghost, interp_type) (pa_fill_patch_pack's send slab, the recv slab it
+ * unpacks).  Returns a negative pa_status if the level is not properly nested for that ghost width. */
+int64_t pa_debug_fill_patch_exchange_ids(pa_hier *h, int lev, int nghost, int interp_type, int which, int64_t *out, int64_t out_len);
 
 /* Device self-test of the stencil kernels' branch-free IEEE sqrt / reciprocal / quotient forms (the flame normal's
  * nrm = -max(1e-14, sqrt(G.G)), n = G / nrm of Src/curvature.cpp:467-502) against the plain operators on n pseudo-random

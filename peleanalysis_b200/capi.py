@@ -80,6 +80,9 @@ SYMBOLS = {
     "pa_filter_weights": (_i, [_i, _i, C.POINTER(_i), C.POINTER(_d), _i]),
     "pa_boxes_max_size": (_i, [_i, C.POINTER(_i), _i, C.POINTER(_i), _i]),
     "pa_fill_patch": (_i, [_vp, _i, _i, _i, _i, _i]),
+    "pa_fill_patch_exchange_buffers": (_i, [_vp, _i, _i, _i, _i, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_i64), C.POINTER(_i64)]),
+    "pa_fill_patch_pack": (_i, [_vp, _i, _i, _i, _i, _i]), "pa_fill_patch_mark_received": (_i, [_vp, _i, _i, _i, _i, _i]),
+    "pa_debug_fill_patch_exchange_ids": (_i64, [_vp, _i, _i, _i, _i, _vp, _i64]),
     "pa_filter": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _i]),
 }
 
@@ -241,6 +244,15 @@ class Hierarchy:
         n = lib().pa_debug_exchange_ids(self.h, which, None, 0)
         out = np.empty(n, dtype=np.int64)
         lib().pa_debug_exchange_ids(self.h, which, _ptr(out) if n else None, n)
+        return out
+
+    def fill_patch_exchange_ids(self, lev: int, nghost: int, interp_type: int, which: int) -> np.ndarray:
+        """pa_fill_patch's exchange plan: identity of the cell in every send- (which=0) / recv-slab (1) slot."""
+        n = lib().pa_debug_fill_patch_exchange_ids(self.h, lev, nghost, interp_type, which, None, 0)
+        if n < 0:
+            check(int(n))
+        out = np.empty(n, dtype=np.int64)
+        lib().pa_debug_fill_patch_exchange_ids(self.h, lev, nghost, interp_type, which, _ptr(out) if n else None, n)
         return out
 
     def exchange_prefix(self, ncomp: int = 1):
@@ -455,6 +467,23 @@ def fp64_rate_gops() -> float:
 
 def fill_patch(f: Field, comp: int, ncomp: int, lev: int, nghost: int, interp_type: int = 1) -> None:
     check(lib().pa_fill_patch(f.f, comp, ncomp, lev, nghost, interp_type))
+
+
+def fill_patch_exchange_buffers(f: Field, ncomp: int, lev: int, nghost: int, interp_type: int = 1):
+    """(send slab pointer, recv slab pointer, send offsets, recv offsets) of pa_fill_patch's exchange, offsets in doubles"""
+    n = f.hier.nranks
+    sp, rp = C.c_void_p(), C.c_void_p()
+    so, ro = (C.c_int64 * (n + 1))(), (C.c_int64 * (n + 1))()
+    check(lib().pa_fill_patch_exchange_buffers(f.f, ncomp, lev, nghost, interp_type, C.byref(sp), C.byref(rp), so, ro))
+    return sp.value, rp.value, list(so), list(ro)
+
+
+def fill_patch_pack(f: Field, comp: int, ncomp: int, lev: int, nghost: int, interp_type: int = 1) -> None:
+    check(lib().pa_fill_patch_pack(f.f, comp, ncomp, lev, nghost, interp_type))
+
+
+def fill_patch_mark_received(f: Field, comp: int, ncomp: int, lev: int, nghost: int, interp_type: int = 1) -> None:
+    check(lib().pa_fill_patch_mark_received(f.f, comp, ncomp, lev, nghost, interp_type))
 
 
 def filter_level(inp: Field, comp_in: int, out: Field, comp_out: int, ncomp: int, lev: int, filter_type: int, fgr: int) -> None:

@@ -118,9 +118,13 @@ struct pa_hier {
     cudaStream_t side = nullptr;
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     // filterPlt path: FillPatch tables per (level, ghost width, interpolater stencil), coarse-patch scratch, filter work prefix
-    struct FpDev { DevBuf<PaFpPiece> pieces; DevBuf<PaFpCopy> copies; DevBuf<PaFpClamp> clamps; };
+    struct FpDev { DevBuf<PaFpPiece> pieces; DevBuf<PaFpCopy> copies; DevBuf<PaFpClamp> clamps; DevBuf<PaPackTag> pack; DevBuf<PaFpUnpack> unpack; };
     std::map<std::array<int, 3>, std::unique_ptr<FpDev>> fp;
     DevBuf<double> fp_scratch;
+    // several ranks: slabs of the FillPatch exchange ([cell][comp], sized for the largest plan asked for) and the fill whose
+    // data the recv slab holds right now (field, comp, ncomp, level, nghost, cgrow); any pack clears it
+    DevBuf<double> fp_send, fp_recv;
+    struct FpMark { const pa_field* f = nullptr; int comp = -1, ncomp = 0, lev = -1, ng = -1, cgrow = -1; } fp_mark;
     std::map<int, std::unique_ptr<DevBuf<long long>>> filter_prefix;   // per level
     std::map<int, long long> filter_nwork;
     DevBuf<double> filter_w3;
@@ -785,6 +789,7 @@ int pa_field_alloc(pa_hier* h, int ncomp, int nghost, pa_field** out) {
 int pa_field_free(pa_field* f) {
     if (!f) return PA_OK;
     if (f->h && f->h->recv_owner == f) f->h->recv_owner = nullptr;
+    if (f->h && f->h->fp_mark.f == f) f->h->fp_mark = pa_hier::FpMark();
     for (void* p : f->ipc_mapped) cudaIpcCloseMemHandle(p);
     for (double* p : f->slab) if (p) cudaFree(p);
     delete f;
@@ -1677,17 +1682,138 @@ int pa_boxes_max_size(int nboxes, const int* boxes, int max_grid_size, int* out_
     return (int)out.size();
 }
 
+// ---- FillPatch on several ranks ------------------------------------------------------------------------------------------
+// Arguments every FillPatch entry shares; (lev, nghost, interp_type) names the fill and its exchange plan.
+static int fp_check(const pa_field* f, int comp, int ncomp, int lev, int nghost, const std::string& who) {
+    CHK(check_field(f, comp, ncomp, who.c_str()));
+    const Hier& H = f->h->H;
+    if (lev < 0 || lev >= H.nlev) return fail(PA_ERR_ARG, who + ": level out of range");
+    if (nghost < 0 || nghost > f->ng) return fail(PA_ERR_ARG, who + ": the field has fewer ghost layers than asked for");
+    if (H.is_per[0] || H.is_per[1] || H.is_per[2])
+        return fail(PA_ERR_UNSUPPORTED, who + ": periodic directions are not served -- the reference tool's PltFileManager geometry is never periodic");
+    return PA_OK;
+}
+
+// Host tables of the fill and their device copy.  The nesting verdict is taken over every box of the level, so on several
+// ranks all of them fail here, before any communication, or none does.
+static int fp_tables(pa_hier* h, int lev, int nghost, int interp_type, const FillPatchTable** T, pa_hier::FpDev** D, const std::string& who) {
+    const int cgrow = interp_type == 1 ? 1 : 0;
+    const FillPatchTable& X = h->H.fill_patch(lev, nghost, cgrow);
+    if (!X.err.empty()) return fail(PA_ERR_ARG, who + ": " + X.err);
+    std::array<int, 3> key{lev, nghost, cgrow};
+    auto it = h->fp.find(key);
+    if (it == h->fp.end()) {
+        auto d = std::make_unique<pa_hier::FpDev>();
+        CU(d->pieces.upload(X.pieces, t_stream));
+        CU(d->copies.upload(X.copies, t_stream));
+        CU(d->clamps.upload(X.clamps, t_stream));
+        CU(d->pack.upload(X.pack, t_stream));
+        CU(d->unpack.upload(X.unpack, t_stream));
+        it = h->fp.emplace(key, std::move(d)).first;
+    }
+    *T = &X;
+    *D = it->second.get();
+    return PA_OK;
+}
+
+// send / recv slabs large enough for this plan; growing one must not free memory a queued pack or unpack still uses
+static int fp_slabs(pa_hier* h, const FillPatchTable& T, int ncomp) {
+    const int n = h->H.nranks;
+    const size_t ns = (size_t)std::max<long long>(T.send_prefix[n] * ncomp, 1), nr = (size_t)std::max<long long>(T.recv_prefix[n] * ncomp, 1);
+    if (h->fp_send.n < ns || h->fp_recv.n < nr) {
+        CU(cudaStreamSynchronize(t_stream));
+        CU(h->fp_send.reserve(ns));
+        CU(h->fp_recv.reserve(nr));
+    }
+    return PA_OK;
+}
+
+// FabArray::FillPatchTwoLevels' communication (ParallelCopy of the coarse patches, FillBoundary of the fine level) as one
+// slab exchange per fill: pa_fill_patch_pack -> transport (NCCL send/recv, pa_copy_async, ...) -> pa_fill_patch_mark_received
+// -> pa_fill_patch.  On one rank the offsets are all zero and pack / mark do nothing.
+int pa_fill_patch_exchange_buffers(pa_field* f, int ncomp, int lev, int nghost, int interp_type, double** send_slab, double** recv_slab,
+                                   int64_t* send_offsets, int64_t* recv_offsets) {
+    const std::string who = "pa_fill_patch_exchange_buffers";
+    CHK(fp_check(f, 0, ncomp, lev, nghost, who));
+    pa_hier* h = f->h;
+    const int n = h->H.nranks;
+    if (send_slab) *send_slab = nullptr;
+    if (recv_slab) *recv_slab = nullptr;
+    for (int p = 0; p <= n; ++p) {
+        if (send_offsets) send_offsets[p] = 0;
+        if (recv_offsets) recv_offsets[p] = 0;
+    }
+    if (n <= 1 || nghost == 0) return PA_OK;
+    CHK(ensure_device(h));
+    const FillPatchTable* T;
+    pa_hier::FpDev* D;
+    CHK(fp_tables(h, lev, nghost, interp_type, &T, &D, who));
+    CHK(fp_slabs(h, *T, ncomp));
+    if (send_slab) *send_slab = h->fp_send.p;
+    if (recv_slab) *recv_slab = h->fp_recv.p;
+    for (int p = 0; p <= n; ++p) {
+        if (send_offsets) send_offsets[p] = T->send_prefix[p] * ncomp;
+        if (recv_offsets) recv_offsets[p] = T->recv_prefix[p] * ncomp;
+    }
+    return PA_OK;
+}
+
+int pa_fill_patch_pack(pa_field* f, int comp, int ncomp, int lev, int nghost, int interp_type) {
+    const std::string who = "pa_fill_patch_pack";
+    CHK(fp_check(f, comp, ncomp, lev, nghost, who));
+    pa_hier* h = f->h;
+    h->fp_mark = pa_hier::FpMark();                  // the transport that follows overwrites the recv slab
+    if (h->H.nranks <= 1 || nghost == 0) return PA_OK;
+    CHK(ensure_device(h));
+    const FillPatchTable* T;
+    pa_hier::FpDev* D;
+    CHK(fp_tables(h, lev, nghost, interp_type, &T, &D, who));
+    CHK(fp_slabs(h, *T, ncomp));
+    if (T->npack == 0) return PA_OK;
+    GridArgs ga;
+    CHK(grid_args_inplace(f, comp, ga));
+    CU(launch_exchange_pack(D->pack.p, 0, (long long)T->pack.size(), 0, T->npack, ga, ncomp, h->fp_send.p, t_stream));
+    return PA_OK;
+}
+
+int pa_fill_patch_mark_received(pa_field* f, int comp, int ncomp, int lev, int nghost, int interp_type) {
+    CHK(fp_check(f, comp, ncomp, lev, nghost, "pa_fill_patch_mark_received"));
+    pa_hier* h = f->h;
+    if (h->H.nranks <= 1) return PA_OK;
+    pa_hier::FpMark m;
+    m.f = f; m.comp = comp; m.ncomp = ncomp; m.lev = lev; m.ng = nghost; m.cgrow = interp_type == 1 ? 1 : 0;
+    h->fp_mark = m;
+    return PA_OK;
+}
+
+int64_t pa_debug_fill_patch_exchange_ids(pa_hier* h, int lev, int nghost, int interp_type, int which, int64_t* out, int64_t out_len) {
+    if (!h || lev < 0 || lev >= h->H.nlev || nghost < 0) { fail(PA_ERR_ARG, "pa_debug_fill_patch_exchange_ids: bad argument"); return PA_ERR_ARG; }
+    const FillPatchTable& T = h->H.fill_patch(lev, nghost, interp_type == 1 ? 1 : 0);
+    if (!T.err.empty()) { fail(PA_ERR_ARG, "pa_debug_fill_patch_exchange_ids: " + T.err); return PA_ERR_ARG; }
+    const std::vector<long long>& v = which ? T.recv_ids : T.send_ids;
+    if (out) for (int64_t i = 0; i < (int64_t)v.size() && i < out_len; ++i) out[i] = v[i];
+    return (int64_t)v.size();
+}
+
 int pa_fill_patch(pa_field* f, int comp, int ncomp, int lev, int nghost, int interp_type) {
-    CHK(check_field(f, comp, ncomp, "pa_fill_patch"));
+    CHK(fp_check(f, comp, ncomp, lev, nghost, "pa_fill_patch"));
     pa_hier* h = f->h;
     Hier& H = h->H;
-    if (lev < 0 || lev >= H.nlev) return fail(PA_ERR_ARG, "pa_fill_patch: level out of range");
-    if (nghost < 0 || nghost > f->ng) return fail(PA_ERR_ARG, "pa_fill_patch: the field has fewer ghost layers than asked for");
-    if (H.nranks > 1) return fail(PA_ERR_UNSUPPORTED, "pa_fill_patch is single-rank (shard whole plotfiles / variables over ranks instead)");
-    if (H.is_per[0] || H.is_per[1] || H.is_per[2])
-        return fail(PA_ERR_UNSUPPORTED, "pa_fill_patch: periodic directions are not served -- the reference tool's PltFileManager geometry is never periodic");
     CHK(ensure_device(h));
     if (nghost == 0) return PA_OK;
+    const int cgrow = interp_type == 1 ? 1 : 0;
+    const FillPatchTable* Tp;
+    pa_hier::FpDev* Dp;
+    CHK(fp_tables(h, lev, nghost, interp_type, &Tp, &Dp, "pa_fill_patch"));
+    const FillPatchTable& T = *Tp;
+    const double* recv = nullptr;
+    if (T.nunpack > 0) {
+        const pa_hier::FpMark& m = h->fp_mark;
+        if (m.f != f || m.comp != comp || m.ncomp != ncomp || m.lev != lev || m.ng != nghost || m.cgrow != cgrow)
+            return fail(PA_ERR_ARG, "pa_fill_patch: this rank receives cells for the fill, but the recv slab does not hold them: exchange this "
+                                    "(field, comp, ncomp, lev, nghost, interp_type) first (pa_fill_patch_pack -> transport -> pa_fill_patch_mark_received)");
+        recv = h->fp_recv.p;
+    }
     int err = PA_OK;
     const PaLayDev* lay = dev_layout(h, lev, f->ng, &err);
     if (!lay) return err;
@@ -1710,35 +1836,32 @@ int pa_fill_patch(pa_field* f, int comp, int ncomp, int lev, int nghost, int int
         const int slices = (int)std::min<long long>(16, std::max<long long>(1, per_tag / 2048));
         CU(launch_halo_blocks(it->second->p, (int)T.tags.size(), slices, h->lev[lev]->boxes.p, lay, base, f->cs[lev], ncomp, t_stream));
     }
-    // 2. the rest of the in-domain ghost cells from the next coarser level, 3. the out-of-domain ones by extrapolation
-    const int cgrow = interp_type == 1 ? 1 : 0;
-    const FillPatchTable& T = H.fill_patch(lev, nghost, cgrow);
-    if (!T.err.empty()) return fail(PA_ERR_ARG, "pa_fill_patch: " + T.err);
-    std::array<int, 3> key{lev, nghost, cgrow};
-    auto it = h->fp.find(key);
-    if (it == h->fp.end()) {
-        auto d = std::make_unique<pa_hier::FpDev>();
-        CU(d->pieces.upload(T.pieces, t_stream));
-        CU(d->copies.upload(T.copies, t_stream));
-        CU(d->clamps.upload(T.clamps, t_stream));
-        it = h->fp.emplace(key, std::move(d)).first;
-    }
+    // 2. the rest of the in-domain ghost cells from the next coarser level, 3. the out-of-domain ones by extrapolation.
+    //    Several ranks: the unpack (cells of other ranks into ghost cells and coarse patches) joins 1. and 2. before the
+    //    interpolation reads the patches; the clamp reads in-domain ghost cells, so it comes last.
+    const pa_hier::FpDev* D = Dp;
     if (T.nfine > 0) {
-        const Level& Cv = H.lev[lev - 1];
-        const PaLayDev* clay = dev_layout(h, lev - 1, f->ng, &err);
-        if (!clay) return err;
         const size_t need = (size_t)T.ncrse * ncomp;
         if (h->fp_scratch.n < need) {
             CU(cudaStreamSynchronize(t_stream));          // an earlier fill may still read the buffer this replaces
             CU(h->fp_scratch.reserve(need));
         }
-        const double* cbase = f->slab[lev - 1] + (long long)comp * f->cs[lev - 1];
-        CU(launch_fp_gather(it->second->copies.p, (int)T.copies.size(), T.ncopy, it->second->pieces.p, h->lev[lev - 1]->boxes.p, clay, cbase,
-                            f->cs[lev - 1], ncomp, h->fp_scratch.p, T.ncrse, t_stream));
-        CU(launch_fp_interp(interp_type == 1, it->second->pieces.p, (int)T.pieces.size(), T.nfine, h->fp_scratch.p, T.ncrse, Cv.dom.lo, Cv.dom.hi,
+        if (T.ncopy > 0) {                                // several ranks: the coarse boxes of a patch may all be remote
+            const PaLayDev* clay = dev_layout(h, lev - 1, f->ng, &err);
+            if (!clay) return err;
+            const double* cbase = f->slab[lev - 1] + (long long)comp * f->cs[lev - 1];
+            CU(launch_fp_gather(D->copies.p, (int)T.copies.size(), T.ncopy, D->pieces.p, h->lev[lev - 1]->boxes.p, clay, cbase,
+                                f->cs[lev - 1], ncomp, h->fp_scratch.p, T.ncrse, t_stream));
+        }
+    }
+    CU(launch_fp_unpack(D->unpack.p, (int)T.unpack.size(), T.nunpack, recv, D->pieces.p, h->fp_scratch.p, T.ncrse, h->lev[lev]->boxes.p, lay,
+                        base, f->cs[lev], ncomp, t_stream));
+    if (T.nfine > 0) {
+        const Level& Cv = H.lev[lev - 1];
+        CU(launch_fp_interp(interp_type == 1, D->pieces.p, (int)T.pieces.size(), T.nfine, h->fp_scratch.p, T.ncrse, Cv.dom.lo, Cv.dom.hi,
                             V.ratio, h->lev[lev]->boxes.p, lay, base, f->cs[lev], ncomp, t_stream));
     }
-    CU(launch_fp_clamp(it->second->clamps.p, (int)T.clamps.size(), T.nclamp, V.dom.lo, V.dom.hi, nghost, h->lev[lev]->boxes.p, lay, base,
+    CU(launch_fp_clamp(D->clamps.p, (int)T.clamps.size(), T.nclamp, V.dom.lo, V.dom.hi, nghost, h->lev[lev]->boxes.p, lay, base,
                        f->cs[lev], ncomp, t_stream));
     return PA_OK;
 }

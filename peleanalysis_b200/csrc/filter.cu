@@ -3,6 +3,8 @@
 //
 //   k_fp_gather   coarse VALID cells -> coarse patches of the pieces (FillPatchSingleLevel into mf_crse_patch,
 //                 AX/AmrCore/AMReX_FillPatchUtil_I.H), one thread per coarse cell over the copy-tag table
+//   k_fp_unpack   several ranks: cells of other ranks' boxes (packed by the exchange pack kernel, moved by the caller) ->
+//                 ghost cells of local boxes and coarse patches (FillPatchTwoLevels' ParallelCopy / FillBoundary data)
 //   k_fp_interp   pieces <- coarse patches: MFCellConsLinInterp with the monotonised-central slope
 //                 (AX/AmrCore/AMReX_MFInterp_3D_C.H:178-260) or MFPCInterp; coarse reads clamp their index into the coarse
 //                 domain, which IS the first-order extrapolation the reference applies to the patch (AMReX_FilCC_3D_C.H)
@@ -62,6 +64,32 @@ __global__ void k_fp_gather(const PaFpCopy* __restrict__ copies, int ncopies, lo
         const PaBoxDev sb = cboxes[t.sbox];
         const long long sa = lay_addr(clay[t.sbox], ci - sb.lo[0], cj - sb.lo[1], ck - sb.lo[2]);
         for (int m = 0; m < ncomp; ++m) scratch[dst + m * ncrse] = cbase[sa + m * ccs];
+    }
+}
+
+// Several ranks: the fill's sources owned by another rank arrive packed in the recv slab ([cell][comp], the exchange pack
+// kernel's layout).  One thread per slab cell over the unpack table: into a ghost cell of a local box (same-level source) or a
+// coarse-patch cell of a piece (coarse source).  Runs before the interpolation, which reads the coarse patches.
+__global__ void k_fp_unpack(const PaFpUnpack* __restrict__ recs, int nrecs, long long ncells, const double* __restrict__ recv,
+                            const PaFpPiece* __restrict__ pieces, double* __restrict__ scratch, long long ncrse,
+                            const PaBoxDev* __restrict__ fboxes, const PaLayDev* __restrict__ flay, double* __restrict__ fbase,
+                            long long fcs, int ncomp) {
+    for (long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x; c < ncells; c += (long long)gridDim.x * blockDim.x) {
+        const PaFpUnpack t = recs[last_le(recs, nrecs, c, [](const PaFpUnpack& x) { return x.start; })];
+        const long long q = c - t.start;
+        const int i = t.lo[0] + (int)(q % t.n[0]);
+        const long long r = q / t.n[0];
+        const int j = t.lo[1] + (int)(r % t.n[1]), k = t.lo[2] + (int)(r / t.n[1]);
+        const double* s = recv + (t.rsrc + q) * ncomp;
+        if (t.box >= 0) {
+            const PaBoxDev b = fboxes[t.box];
+            const long long da = lay_addr(flay[t.box], i - b.lo[0], j - b.lo[1], k - b.lo[2]);
+            for (int m = 0; m < ncomp; ++m) fbase[da + m * fcs] = s[m];
+        } else {
+            const PaFpPiece P = pieces[-1 - t.box];
+            const long long dst = P.cstart + ((long long)(k - P.clo[2]) * P.cn[1] + (j - P.clo[1])) * P.cn[0] + (i - P.clo[0]);
+            for (int m = 0; m < ncomp; ++m) scratch[dst + m * ncrse] = s[m];
+        }
     }
 }
 
@@ -339,6 +367,15 @@ cudaError_t launch_fp_gather(const PaFpCopy* copies, int ncopies, long long ncel
                              cudaStream_t st) {
     if (ncells <= 0 || ncopies <= 0) return cudaSuccess;
     PA_LAUNCH(blocks_for(ncells, 256), 256, 0, st, k_fp_gather)(copies, ncopies, ncells, pieces, cboxes, clay, cbase, ccs, ncomp, scratch, ncrse);
+    ++g_launches;
+    return cudaGetLastError();
+}
+
+cudaError_t launch_fp_unpack(const PaFpUnpack* recs, int nrecs, long long ncells, const double* recv, const PaFpPiece* pieces,
+                             double* scratch, long long ncrse, const PaBoxDev* fboxes, const PaLayDev* flay, double* fbase, long long fcs,
+                             int ncomp, cudaStream_t st) {
+    if (ncells <= 0 || nrecs <= 0) return cudaSuccess;
+    PA_LAUNCH(blocks_for(ncells, 256), 256, 0, st, k_fp_unpack)(recs, nrecs, ncells, recv, pieces, scratch, ncrse, fboxes, flay, fbase, fcs, ncomp);
     ++g_launches;
     return cudaGetLastError();
 }

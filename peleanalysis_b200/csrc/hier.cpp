@@ -122,8 +122,12 @@ std::string Hier::init(int nlev_, const pa_level_desc_host* L, const int* per, c
     xplan.send_prefix.assign(nranks + 1, 0);
     xplan.recv_prefix.assign(nranks + 1, 0);
     xplan.pack_level_begin.assign(nlev + 1, 0);
-    if (nranks > 1) build_exchange();          // fixes recv/send slab offsets first
-    for (int l = 0; l < nlev; ++l) build_halo(l, 1, true, halo_cross[l], true);
+    // a filter-only hierarchy on several ranks moves its cross-rank cells through fill_patch's own plan: the width-1 cross
+    // tables (and the ratio-aligned coarse needs they assume) would never be used
+    const bool cross_tables = !(filter_only && nranks > 1);
+    if (nranks > 1 && cross_tables) build_exchange();          // fixes recv/send slab offsets first
+    if (cross_tables)
+        for (int l = 0; l < nlev; ++l) build_halo(l, 1, true, halo_cross[l], true);
     if (filter_only) {                             // FillPatch needs no face masks / BC records; grids may be unaligned
         faces = FaceTable();
         faces.level_rec_begin.assign(nlev + 1, 0);
@@ -515,6 +519,7 @@ void Hier::build_halo(int l, int ng, bool cross, HaloTable& out, bool allow_remo
                 V.hash.query(grown.shifted(s.data()), [&](int k, const Box& ib) { is.emplace_back(k, ib); });
                 sort_isects(is);
                 for (auto& e : is) {
+                    if (V.owner[e.first] != rank) continue;        // several ranks: fill_patch's exchange moves these
                     int neg[3] = {-s[0], -s[1], -s[2]};
                     Box dst = e.second.shifted(neg);
                     parts.clear();
@@ -523,7 +528,7 @@ void Hier::build_halo(int l, int ng, bool cross, HaloTable& out, bool allow_remo
                         PaHaloTag t;
                         std::memset(&t, 0, sizeof(t));
                         t.dbox = V.g2l[gb];
-                        t.sbox = V.g2l[e.first];       // caller guarantees single rank
+                        t.sbox = V.g2l[e.first];
                         t.srank = rank;
                         t.rsrc = -1;
                         for (int d = 0; d < 3; ++d) { t.dlo[d] = p.lo[d]; t.n[d] = p.len(d); t.shift[d] = s[d]; }
@@ -597,12 +602,38 @@ void box_max_size(int nboxes, const int* boxes, int max_grid_size, std::vector<B
 // its grown region that lies inside the domain and that no box of the level covers is cut into boxes ("pieces",
 // BoxArray::complementIn); each piece is interpolated from a coarse patch that is gathered from the coarse level's valid
 // cells.  Ghost cells outside the (non-periodic) domain are first-order extrapolated afterwards: `clamps`.
+// On several ranks the walk goes over every box of the level (global id order): a source owned by the destination box's
+// owner is a local table entry there, any other source joins the slab stream (source owner -> destination owner), which the
+// source's owner packs (`pack`) and the destination's owner unpacks (`unpack`) -- what ParallelCopy / FillBoundary
+// communicate inside FillPatchTwoLevels.
 const FillPatchTable& Hier::fill_patch(int l, int ng, int cgrow) {
     std::array<int, 3> key{l, ng, cgrow};
     auto it = fill_patch_.find(key);
     if (it != fill_patch_.end()) return it->second;
     FillPatchTable T;
     const Level& V = lev[l];
+    struct XSend { int peer; PaPackTag t; };
+    struct XRecv { int peer; int slev, sgb; PaFpUnpack u; };
+    std::vector<XSend> xs;
+    std::vector<XRecv> xr;
+    // a source region (index space of level slev, cells [r.lo, r.hi]) of global box sgb for destination `dst` (>= 0: local
+    // fine box, < 0: piece) of a box owned by `downer`
+    auto cross = [&](int downer, int slev, int sgb, const Box& r, int dst) {
+        const int sowner = lev[slev].owner[sgb];
+        if (downer == rank) {
+            XRecv e; e.peer = sowner; e.slev = slev; e.sgb = sgb;
+            std::memset(&e.u, 0, sizeof(e.u));
+            e.u.box = dst;
+            for (int d = 0; d < 3; ++d) { e.u.lo[d] = r.lo[d]; e.u.n[d] = r.len(d); }
+            xr.push_back(e);
+        } else if (sowner == rank) {
+            XSend e; e.peer = downer;
+            std::memset(&e.t, 0, sizeof(e.t));
+            e.t.sbox = lev[slev].g2l[sgb]; e.t.slev = slev;
+            for (int d = 0; d < 3; ++d) { e.t.slo[d] = r.lo[d]; e.t.n[d] = r.len(d); }
+            xs.push_back(e);
+        }
+    };
     for (size_t lb = 0; lb < V.local.size(); ++lb) {
         const Box g = V.boxes[V.local[lb]].grown(ng);
         bool out = false;
@@ -614,45 +645,100 @@ const FillPatchTable& Hier::fill_patch(int l, int ng, int cgrow) {
             T.clamps.push_back(c);
         }
     }
-    if (l > 0) {
-        const Level& Cv = lev[l - 1];
-        const int r = V.ratio;
-        std::vector<Box> cur, nxt;
-        for (size_t lb = 0; lb < V.local.size(); ++lb) {
-            const Box region = V.boxes[V.local[lb]].grown(ng).isect(V.dom);
-            cur.assign(1, region);
-            V.hash.query(region, [&](int idx, const Box&) {
-                nxt.clear();
-                for (const Box& b : cur) box_diff(b, V.boxes[idx], nxt);
-                cur.swap(nxt);
-            });
-            for (const Box& pc : cur) {
-                PaFpPiece P;
-                P.box = (int)lb;
-                Box cp;
-                for (int d = 0; d < 3; ++d) {
-                    P.lo[d] = pc.lo[d]; P.n[d] = pc.len(d);
-                    cp.lo[d] = coarsen(pc.lo[d], r) - cgrow; cp.hi[d] = coarsen(pc.hi[d], r) + cgrow;
-                    P.clo[d] = cp.lo[d]; P.cn[d] = cp.len(d);
-                }
-                P.cstart = T.ncrse; P.fstart = T.nfine;
-                const Box cpd = cp.isect(Cv.dom);
-                long long got = 0;
-                const int piece = (int)T.pieces.size();
-                Cv.hash.query(cpd, [&](int idx, const Box& is) {
-                    PaFpCopy c;
-                    c.piece = piece; c.sbox = Cv.g2l[idx];
-                    for (int d = 0; d < 3; ++d) { c.lo[d] = is.lo[d]; c.n[d] = is.len(d); }
-                    c.start = T.ncopy;
-                    T.ncopy += is.npts(); got += is.npts();
-                    T.copies.push_back(c);
-                });
-                if (got != cpd.npts() && T.err.empty())
-                    T.err = "level " + std::to_string(l) + ": ghost cells of box " + std::to_string(V.local[lb]) +
-                            " need coarse cells that level " + std::to_string(l - 1) + " does not cover (grids not properly nested for this ghost width)";
-                T.ncrse += cp.npts(); T.nfine += pc.npts();
-                T.pieces.push_back(P);
+    // one rank: the local boxes are all boxes, in the same order
+    const std::vector<int> every = [&] { std::vector<int> v(V.boxes.size()); for (size_t b = 0; b < v.size(); ++b) v[b] = (int)b; return v; }();
+    const std::vector<int>& walk = nranks > 1 ? every : V.local;
+    std::vector<std::pair<int, Box>> is;
+    std::vector<Box> parts;
+    const Level* Cv = l > 0 ? &lev[l - 1] : nullptr;
+    std::vector<Box> cur, nxt;
+    for (int gb : walk) {
+        const int downer = V.owner[gb];
+        const bool mine = downer == rank;
+        // 1. same-level sources of another rank, in halo_full's order (grown(ng) against every box, minus the own box)
+        if (nranks > 1) {
+            is.clear();
+            V.hash.query(V.boxes[gb].grown(ng), [&](int k, const Box& ib) { is.emplace_back(k, ib); });
+            sort_isects(is);
+            for (auto& e : is) {
+                if (V.owner[e.first] == downer) continue;
+                parts.clear();
+                box_diff(e.second, V.boxes[gb], parts);
+                for (const Box& p : parts) cross(downer, l, e.first, p, mine ? V.g2l[gb] : 0);
             }
+        }
+        if (!Cv) continue;
+        // 2. coarse patches of the pieces
+        const int r = V.ratio;
+        const Box region = V.boxes[gb].grown(ng).isect(V.dom);
+        cur.assign(1, region);
+        V.hash.query(region, [&](int idx, const Box&) {
+            nxt.clear();
+            for (const Box& b : cur) box_diff(b, V.boxes[idx], nxt);
+            cur.swap(nxt);
+        });
+        for (const Box& pc : cur) {
+            PaFpPiece P;
+            P.box = mine ? V.g2l[gb] : -1;
+            Box cp;
+            for (int d = 0; d < 3; ++d) {
+                P.lo[d] = pc.lo[d]; P.n[d] = pc.len(d);
+                cp.lo[d] = coarsen(pc.lo[d], r) - cgrow; cp.hi[d] = coarsen(pc.hi[d], r) + cgrow;
+                P.clo[d] = cp.lo[d]; P.cn[d] = cp.len(d);
+            }
+            P.cstart = T.ncrse; P.fstart = T.nfine;
+            const Box cpd = cp.isect(Cv->dom);
+            long long got = 0;
+            const int piece = (int)T.pieces.size();
+            Cv->hash.query(cpd, [&](int idx, const Box& ib) {
+                got += ib.npts();
+                if (Cv->owner[idx] != downer) { cross(downer, l - 1, idx, ib, -1 - piece); return; }
+                if (!mine) return;
+                PaFpCopy c;
+                c.piece = piece; c.sbox = Cv->g2l[idx];
+                for (int d = 0; d < 3; ++d) { c.lo[d] = ib.lo[d]; c.n[d] = ib.len(d); }
+                c.start = T.ncopy;
+                T.ncopy += ib.npts();
+                T.copies.push_back(c);
+            });
+            if (got != cpd.npts() && T.err.empty())
+                T.err = "level " + std::to_string(l) + ": ghost cells of box " + std::to_string(gb) +
+                        " need coarse cells that level " + std::to_string(l - 1) + " does not cover (grids not properly nested for this ghost width)";
+            if (!mine) continue;
+            T.ncrse += cp.npts(); T.nfine += pc.npts();
+            T.pieces.push_back(P);
+        }
+    }
+    if (nranks > 1) {
+        // slab layout: per peer contiguous, walk order inside a peer's block
+        T.send_prefix.assign(nranks + 1, 0);
+        T.recv_prefix.assign(nranks + 1, 0);
+        for (const XSend& e : xs) T.send_prefix[e.peer + 1] += (long long)e.t.n[0] * e.t.n[1] * e.t.n[2];
+        for (const XRecv& e : xr) T.recv_prefix[e.peer + 1] += (long long)e.u.n[0] * e.u.n[1] * e.u.n[2];
+        for (int p = 0; p < nranks; ++p) { T.send_prefix[p + 1] += T.send_prefix[p]; T.recv_prefix[p + 1] += T.recv_prefix[p]; }
+        std::vector<long long> sc(T.send_prefix.begin(), T.send_prefix.end() - 1), rc(T.recv_prefix.begin(), T.recv_prefix.end() - 1);
+        T.send_ids.assign((size_t)T.send_prefix[nranks], -1);
+        T.recv_ids.assign((size_t)T.recv_prefix[nranks], -1);
+        auto ids = [&](std::vector<long long>& out, long long at, int slev, int sgb, const int* lo, const int* n) {
+            const Box& B = lev[slev].boxes[sgb];
+            long long q = 0;
+            for (int k = 0; k < n[2]; ++k)
+                for (int j = 0; j < n[1]; ++j)
+                    for (int i = 0; i < n[0]; ++i, ++q) out[(size_t)(at + q)] = cell_id(slev, sgb, B, lo[0] + i, lo[1] + j, lo[2] + k);
+        };
+        for (XSend& e : xs) {
+            const long long c = (long long)e.t.n[0] * e.t.n[1] * e.t.n[2];
+            e.t.dense = T.npack; e.t.start = sc[e.peer];
+            ids(T.send_ids, e.t.start, e.t.slev, lev[e.t.slev].local[e.t.sbox], e.t.slo, e.t.n);
+            sc[e.peer] += c; T.npack += c;
+            T.pack.push_back(e.t);
+        }
+        for (XRecv& e : xr) {
+            const long long c = (long long)e.u.n[0] * e.u.n[1] * e.u.n[2];
+            e.u.start = T.nunpack; e.u.rsrc = rc[e.peer];
+            ids(T.recv_ids, e.u.rsrc, e.slev, e.sgb, e.u.lo, e.u.n);
+            rc[e.peer] += c; T.nunpack += c;
+            T.unpack.push_back(e.u);
         }
     }
     return fill_patch_.emplace(key, std::move(T)).first->second;

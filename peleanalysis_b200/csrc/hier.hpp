@@ -143,7 +143,18 @@ struct FillPatchTable {
     long long ncrse = 0;              // scratch cells (per component)
     long long ncopy = 0;              // coarse cells gathered
     long long nclamp = 0;             // cells of the grown boxes in `clamps`
-    std::string err;                  // non-empty: the coarse level does not cover a coarse patch (improper nesting)
+    std::string err;                  // non-empty: the coarse level does not cover a coarse patch (improper nesting); decided
+                                      // over every box of the level, so all ranks reach the same verdict
+    // Several ranks: the sources owned by another rank than the destination box's, moved as packed slabs ([cell][comp]).
+    // Every rank walks every box of the level in global id order (same-level sources, then coarse copies piece by piece);
+    // the stream from rank p to rank q is the subsequence with source owner p and destination owner q, so both sides agree
+    // on slab offsets without a handshake.  Empty on one rank.
+    std::vector<PaPackTag> pack;      // what this rank packs (slev = l: same-level source, l - 1: coarse source)
+    std::vector<PaFpUnpack> unpack;   // recv-slab cells -> ghost cells / coarse-patch cells of this rank
+    std::vector<long long> send_prefix, recv_prefix;   // nranks+1, in cells
+    long long npack = 0, nunpack = 0; // cells
+    // debug / parity: identity of the cell every send-slab slot carries / recv-slab slot expects (ExchangePlan's form)
+    std::vector<long long> send_ids, recv_ids;
 };
 
 // BoxList::maxSize: every box replaced, in place, by its chunks no longer than max_grid_size (AMReX_BoxList.cpp:765-815)
@@ -174,10 +185,11 @@ public:
     // coarse gather index resolved against the ng-ghost layout: element offset inside the coarse level's component slab,
     // -1 = never filled (NaN in the reference), <= -2: recv-slab slot -(v+2)
     std::vector<long long> crse_offsets(int ng);
-    // full FillBoundary table (all ng layers incl. edges/corners) -- debug / pa_fill_boundary(cross=0); local sources only
+    // full FillBoundary table (all ng layers incl. edges/corners) -- debug / pa_fill_boundary(cross=0); sources owned by
+    // this rank only (on several ranks the others arrive through fill_patch's exchange)
     const HaloTable& halo_full(int l, int ng);
     // FillPatchTwoLevels / FillPatchSingleLevel tables of level l for ng ghost layers; cgrow = coarse cells the
-    // interpolater reads around the coarsened piece.  Single-rank, non-periodic hierarchies only.
+    // interpolater reads around the coarsened piece, with the exchange plan of the cross-rank sources.  Non-periodic only.
     const FillPatchTable& fill_patch(int l, int ng, int cgrow);
 
     void periodic_shifts(const Box& dom, int ng, std::vector<std::array<int, 3>>& out) const;

@@ -169,6 +169,10 @@ cudaError_t launch_halo_blocks(const PaHaloTag* tags, int ntags, int slices, con
 cudaError_t launch_fp_gather(const PaFpCopy* copies, int ncopies, long long ncells, const PaFpPiece* pieces, const PaBoxDev* cboxes,
                              const PaLayDev* clay, const double* cbase, long long ccs, int ncomp, double* scratch, long long ncrse,
                              cudaStream_t st);
+// several ranks: recv slab ([cell][comp]) -> ghost cells of local boxes and coarse-patch cells of the pieces
+cudaError_t launch_fp_unpack(const PaFpUnpack* recs, int nrecs, long long ncells, const double* recv, const PaFpPiece* pieces,
+                             double* scratch, long long ncrse, const PaBoxDev* fboxes, const PaLayDev* flay, double* fbase, long long fcs,
+                             int ncomp, cudaStream_t st);
 cudaError_t launch_fp_interp(bool conservative, const PaFpPiece* pieces, int npieces, long long ncells, const double* scratch,
                              long long ncrse, const int cdom_lo[3], const int cdom_hi[3], int ratio, const PaBoxDev* fboxes,
                              const PaLayDev* flay, double* fbase, long long fcs, int ncomp, cudaStream_t st);

@@ -137,6 +137,15 @@ struct PaFpCopy {
     int lo[3], n[3];
     long long start;    // prefix over the cells of all copy tags
 };
+// several ranks: recv-slab cells [rsrc, rsrc + n) -> cells [lo, lo+n) of a ghost region of a local box (same-level source
+// owned by another rank, box >= 0) or of the coarse patch of piece -1 - box (coarse source owned by another rank)
+struct PaFpUnpack {
+    int box;            // >= 0: local fine box (fine index space); < 0: piece -1 - box (coarse index space)
+    int lo[3], n[3];
+    int pad;
+    long long rsrc;     // first cell of this record inside the recv slab (per component)
+    long long start;    // prefix over the cells of all unpack records (the kernel's enumeration)
+};
 // a local box whose grown region leaves the domain: its ghost cells outside take the value at the clamped index
 struct PaFpClamp {
     int box;

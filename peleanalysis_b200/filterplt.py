@@ -40,11 +40,15 @@ def rechop(P, pf: Plotfile, comps: Sequence[int], max_grid_size: int, nlev: int)
 
 
 class FilterRun:
-    """Device state of one filterPlt run: hierarchy on the re-chopped grids, input field with ghost cells, output field."""
+    """Device state of one filterPlt run: hierarchy on the re-chopped grids, input field with ghost cells, output field.
+
+    rank / nranks > 1: the re-chopped boxes of every level are spread over the ranks by pa_sfc_distribute, only this rank's
+    boxes are uploaded and returned, and every fill is preceded by its slab exchange (multigpu.FillPatchExchange over the
+    current torch.distributed group; `multigpu` / `wrap` let tests hand in another binding and host-memory slabs)."""
 
     def __init__(self, P, pf: Plotfile, filter_type: int = 1, base_fgr: int = 2, same_fgr_all_levels: bool = False,
                  max_grid_size: int = 32, interp_type: int = 1, variables: Optional[Sequence[str]] = None,
-                 max_filter_level: int = 1000, upload: bool = True):
+                 max_filter_level: int = 1000, upload: bool = True, rank: int = 0, nranks: int = 1, multigpu=None, wrap=None):
         self.P = P
         self.names = list(variables) if variables else list(pf.names)
         comps = [pf.comp(n) for n in self.names]
@@ -55,25 +59,34 @@ class FilterRun:
         self.fgr = [level_fgr(base_fgr, ratios, same_fgr_all_levels, l) for l in range(self.nlev)]
         self.ngrow = [P.filter_weights(filter_type, f)[0] for f in self.fgr]
         self.levels = rechop(P, pf, comps, max_grid_size, self.nlev)
-        self.hier = P.Hierarchy(self.levels, is_per=(0, 0, 0), sym_dir=(0, 0, 0), flags=P.FILTER_ONLY)
+        self.hier = P.Hierarchy(self.levels, is_per=(0, 0, 0), sym_dir=(0, 0, 0), rank=rank, nranks=nranks, flags=P.FILTER_ONLY)
         self.ncomp = len(comps)
         self.fin = P.Field(self.hier, self.ncomp, max(self.ngrow))
         self.fout = P.Field(self.hier, self.ncomp, 0)
+        self.exchanges = []
+        if nranks > 1:
+            if multigpu is None:
+                from . import multigpu
+            kw = {} if wrap is None else {"wrap": wrap}
+            self.exchanges = [multigpu.FillPatchExchange(self.fin, self.ncomp, l, self.ngrow[l], interp_type, **kw) for l in range(self.nlev)]
         if upload:
             for c in range(self.ncomp):
                 self.fin.upload_fabs(c, [[f[c] for f in lv.fabs] for lv in self.levels])
 
     def step(self) -> None:
-        """ghost fill + filter of every level (filterPlt.cpp:166-221), asynchronous on the library stream"""
+        """[exchange +] ghost fill + filter of every level (filterPlt.cpp:166-221), asynchronous on the library stream"""
         P = self.P
         for l in range(self.nlev):
+            if self.exchanges:
+                self.exchanges[l].run(0)
             P.fill_patch(self.fin, 0, self.ncomp, l, self.ngrow[l], self.interp_type)
             P.filter_level(self.fin, 0, self.fout, 0, self.ncomp, l, self.filter_type, self.fgr[l])
 
-    def result(self) -> List[List[np.ndarray]]:
-        """per level, per box: [ncomp][nz][ny][nx]"""
+    def result(self) -> List[List[Optional[np.ndarray]]]:
+        """per level, per box: [ncomp][nz][ny][nx] (None for boxes of other ranks)"""
         per_comp = [self.fout.download_fabs(c) for c in range(self.ncomp)]
-        return [[np.stack([per_comp[c][l][b] for c in range(self.ncomp)]) for b in range(len(lv.boxes))] for l, lv in enumerate(self.levels)]
+        return [[np.stack([per_comp[c][l][b] for c in range(self.ncomp)]) if per_comp[0][l][b] is not None else None
+                 for b in range(len(lv.boxes))] for l, lv in enumerate(self.levels)]
 
     def grown_input(self, lev: int, box: int, comp: int) -> np.ndarray:
         """the input FAB with the field's ghost width; only the level's own ngrow layers are filled"""

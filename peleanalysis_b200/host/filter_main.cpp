@@ -4,10 +4,12 @@
 //
 //   filterPlt3d.b200.ex infile=<plotfile> [variables=a b c] [max_filter_level=N] [filter_type=1] [base_fgr=2]
 //                       [same_fgr_all_levels=0] [max_grid_size=32] [interp_type=1]
+//                       [ngpus=N]  (one host thread per GPU, multi_gpu.hpp: the output boxes spread over the GPUs, the
+//                                   FillPatch sources of other GPUs moved as packed slabs, one Cell_D file per GPU)
 #include <chrono>
 #include <cstring>
 
-#include "tool_common.hpp"
+#include "multi_gpu.hpp"
 
 static void print_usage(char** argv) {
     std::cerr << "Utility to filter the fields of a pltfile\nusage:\n" << argv[0] << " infile=<s> [options] \n\tOptions:\n"
@@ -37,6 +39,9 @@ int main(int argc, char** argv) {
     pp.query("max_grid_size", max_grid_size);
     pp.query("interp_type", interp_type);
     pp.query("verbose", verbose);
+    int ngpus = 1;
+    pp.query("ngpus", ngpus);
+    if (ngpus < 1) pa_abort("ngpus must be >= 1");
 
     pltio::Header H;
     try { H = pltio::read_header(infile); } catch (std::exception& e) { pa_abort(std::string("cannot read plotfile: ") + e.what()); }
@@ -61,6 +66,7 @@ int main(int argc, char** argv) {
     std::vector<int> fgr(Nlev), ngrow(Nlev);
     pltio::Header meta = H;
     std::vector<std::vector<std::vector<pltio::BoxI>>> chunks(Nlev);           // [level][original box] -> its chunks
+    std::vector<std::vector<int>> parent(Nlev);                                 // [level][chunk] -> original box
     int fgr_lev = base_fgr, ngmax = 0;
     for (int l = 0; l < Nlev; ++l) {
         if (!same_fgr && l > 0) {
@@ -85,8 +91,17 @@ int main(int argc, char** argv) {
                 for (int d = 0; d < 3; ++d) { C.lo[d] = out[6 * c + d]; C.hi[d] = out[6 * c + 3 + d]; }
                 chunks[l][b].push_back(C);
                 meta.levels[l].boxes.push_back(C);
+                parent[l].push_back((int)b);
             }
         }
+    }
+    const std::string outfile = file_root(infile) + "_filtered";
+    if (ngpus > 1) {
+        FilterJob J;
+        J.infile = infile; J.outfile = outfile; J.H = &H; J.meta = &meta; J.parent = parent; J.Nlev = Nlev;
+        J.filter_type = filter_type; J.interp_type = interp_type; J.ngmax = ngmax; J.fgr = fgr; J.ngrow = ngrow; J.names = names;
+        run_filter_multi(ngpus, J);
+        return 0;
     }
     HierInput hi;
     make_level_descs(meta, Nlev, hi);
@@ -153,7 +168,6 @@ int main(int argc, char** argv) {
     auto t2 = std::chrono::steady_clock::now();
 
     std::cout << "Saving filtered data..." << std::endl;
-    const std::string outfile = file_root(infile) + "_filtered";
     std::vector<std::vector<const double*>> data(Nlev);
     for (int l = 0; l < Nlev; ++l) for (int c = 0; c < ncomp; ++c) data[l].push_back(buf[l].comp(c));
     std::vector<int> rr(std::max(Nlev - 1, 0), 2);            // write_plotfile hard-codes ref_ratio 2 (filterPlt.cpp:50)

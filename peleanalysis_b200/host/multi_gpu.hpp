@@ -302,3 +302,148 @@ inline void run_curv_multi(int ngpus, CurvJob& J) {
     meta.time = 0.0;
     try { pltio::write_metadata(J.outfile, meta, J.names, J.Nlev, M.records, rr); } catch (std::exception& e) { pa_abort(e.what()); }
 }
+
+// ---- filterPlt: boxes of every level spread over the threads, FillPatch sources of other ranks moved as packed slabs -----
+// The exchange in front of pa_fill_patch(lev): pack -> device-to-device copies of each peer's segment (pa_copy_async, as
+// exchange_slabs) -> mark.  Collective; the filterPlt hierarchy has no peer links, so nothing is read in place.
+inline void exchange_fill_patch(int r, MultiShared& M, pa_field* f, int ncomp, int lev, int nghost, int interp_type) {
+    const int n = M.n;
+    double *send = nullptr, *recv = nullptr;
+    std::vector<int64_t> so(n + 1), ro(n + 1);
+    check(pa_fill_patch_exchange_buffers(f, ncomp, lev, nghost, interp_type, &send, &recv, so.data(), ro.data()), "pa_fill_patch_exchange_buffers");
+    check(pa_fill_patch_pack(f, 0, ncomp, lev, nghost, interp_type), "pa_fill_patch_pack");
+    check(pa_sync(), "pa_sync");
+    M.send[r] = send;
+    M.soff[r] = so;
+    M.bar.wait();
+    for (int p = 0; p < n; ++p) {
+        if (p == r) continue;
+        const int64_t cnt = ro[p + 1] - ro[p];
+        if (cnt != M.soff[p][r + 1] - M.soff[p][r]) pa_abort("multi-GPU FillPatch plan: send / recv counts disagree");
+        if (cnt > 0) check(pa_copy_async(recv + ro[p], M.send[p] + M.soff[p][r], cnt), "pa_copy_async");
+    }
+    check(pa_fill_patch_mark_received(f, 0, ncomp, lev, nghost, interp_type), "pa_fill_patch_mark_received");
+    check(pa_sync(), "pa_sync");
+    M.bar.wait();                                      // the send slabs may be repacked from here on
+}
+
+struct FilterJob {
+    std::string infile, outfile;
+    const pltio::Header* H;                            // the plotfile
+    const pltio::Header* meta;                         // its grids re-chopped to max_grid_size (the output's boxes)
+    std::vector<std::vector<int>> parent;              // [level][output box] -> the plotfile box it was cut from
+    int Nlev, filter_type, interp_type, ngmax;
+    std::vector<int> fgr, ngrow;
+    std::vector<std::string> names;
+    std::vector<std::vector<int>> owner;               // [level][output box] -> rank
+};
+
+inline void filter_rank(int r, MultiShared& M, const FilterJob& J) {
+    const pltio::Header& H = *J.H;
+    const pltio::Header& meta = *J.meta;
+    const int n = M.n, Nlev = J.Nlev, ncomp = (int)J.names.size();
+    const bool talk = r == 0;                          // the tool's progress messages, once
+    check(pa_init(r), "pa_init");
+    for (int p = 0; p < n; ++p) if (p != r) check(pa_enable_peer_access(p), "pa_enable_peer_access");
+    HierInput hi;
+    make_level_descs(meta, Nlev, hi);
+    std::vector<std::vector<int>> own(Nlev), mine(Nlev);
+    for (int l = 0; l < Nlev; ++l) {
+        own[l] = J.owner[l];
+        hi.lv[l].owner = own[l].data();
+        for (int b = 0; b < (int)own[l].size(); ++b) if (own[l][b] == r) mine[l].push_back(b);
+    }
+    const int no_per[3] = {0, 0, 0}, bck[3] = {PA_BC_NEUMANN, PA_BC_NEUMANN, PA_BC_NEUMANN};
+    pa_hier* h = nullptr;
+    check(pa_hier_create2(&h, Nlev, hi.lv.data(), no_per, bck, r, n, PA_HIER_FILTER_ONLY), "pa_hier_create2");
+    pa_field *fin = nullptr, *fout = nullptr;
+    check(pa_field_alloc(h, ncomp, J.ngmax, &fin), "pa_field_alloc");
+    check(pa_field_alloc(h, ncomp, 0, &fout), "pa_field_alloc");
+
+    // this rank's output boxes, cut from the plotfile boxes that contain them (only those are read)
+    if (talk) std::cout << "Reading data..." << std::endl;
+    std::vector<PinnedLevel> buf(Nlev);
+    for (int l = 0; l < Nlev; ++l) {
+        if (talk) std::cout << "on level " << l << std::endl;
+        long long nc = 0;
+        for (int b : mine[l]) nc += meta.levels[l].boxes[b].npts();
+        buf[l].alloc(std::max<long long>(nc, 1), ncomp);
+        buf[l].ncells = nc;
+        if (mine[l].empty()) continue;
+        std::vector<double> tmp;
+        for (int v = 0; v < ncomp; ++v) {
+            double* dst = buf[l].comp(v);
+            for (size_t i = 0; i < mine[l].size();) {
+                const int pb = J.parent[l][mine[l][i]];
+                const pltio::BoxI& B = H.levels[l].boxes[pb];
+                tmp.resize((size_t)B.npts());
+                pltio::read_boxes_comp(J.infile, H, l, H.comp(J.names[v]), {pb}, tmp.data());
+                const long long nx = B.hi[0] - B.lo[0] + 1, ny = B.hi[1] - B.lo[1] + 1;
+                for (; i < mine[l].size() && J.parent[l][mine[l][i]] == pb; ++i) {      // chunk ids ascend with their parent's
+                    const pltio::BoxI& Cb = meta.levels[l].boxes[mine[l][i]];
+                    const int cx = Cb.hi[0] - Cb.lo[0] + 1;
+                    for (int k = Cb.lo[2]; k <= Cb.hi[2]; ++k)
+                        for (int j = Cb.lo[1]; j <= Cb.hi[1]; ++j) {
+                            std::memcpy(dst, tmp.data() + ((long long)(k - B.lo[2]) * ny + (j - B.lo[1])) * nx + (Cb.lo[0] - B.lo[0]), (size_t)cx * 8);
+                            dst += cx;
+                        }
+                }
+            }
+            check(pa_field_upload_level(fin, l, v, buf[l].comp(v)), "upload");
+        }
+    }
+    check(pa_sync(), "pa_sync");
+    M.bar.wait();
+    if (talk) std::cout << "Done!" << std::endl;
+
+    if (talk) std::cout << "FillPatching data..." << std::endl;
+    for (int l = 0; l < Nlev; ++l) {
+        if (talk) std::cout << "on level " << l << std::endl;
+        exchange_fill_patch(r, M, fin, ncomp, l, J.ngrow[l], J.interp_type);
+        check(pa_fill_patch(fin, 0, ncomp, l, J.ngrow[l], J.interp_type), "pa_fill_patch");
+    }
+    if (talk) std::cout << "Done!" << std::endl;
+    if (talk) std::cout << "Filtering data..." << std::endl;
+    for (int l = 0; l < Nlev; ++l) {
+        if (talk) std::cout << "on level " << l << std::endl;
+        check(pa_filter(fin, 0, fout, 0, ncomp, l, J.filter_type, J.fgr[l]), "pa_filter");
+    }
+    for (int l = 0; l < Nlev; ++l)
+        if (!mine[l].empty())
+            for (int c = 0; c < ncomp; ++c) check(pa_field_download_level(fout, l, c, buf[l].comp(c)), "download");
+    check(pa_sync(), "pa_sync");
+    M.bar.wait();
+    if (talk) std::cout << "Done!" << std::endl;
+
+    if (talk) std::cout << "Saving filtered data..." << std::endl;
+    char fn[32];
+    std::snprintf(fn, sizeof fn, "Cell_D_%05d", r);
+    std::vector<pltio::FabRecord> recs;
+    for (int l = 0; l < Nlev; ++l) {
+        std::vector<const double*> data;
+        for (int c = 0; c < ncomp; ++c) data.push_back(buf[l].comp(c));
+        auto w = pltio::write_fab_file(J.outfile, meta, l, fn, mine[l], data);
+        recs.insert(recs.end(), w.begin(), w.end());
+    }
+    {
+        std::lock_guard<std::mutex> lk(M.mu);
+        M.records.insert(M.records.end(), recs.begin(), recs.end());
+    }
+    pa_field_free(fin); pa_field_free(fout); pa_hier_destroy(h);
+    M.bar.wait();
+}
+
+// returns after the output plotfile is complete
+inline void run_filter_multi(int ngpus, FilterJob& J) {
+    J.owner = sfc_owners(*J.meta, J.Nlev, ngpus);
+    try { pltio::create_plotfile_dirs(J.outfile, J.Nlev); } catch (std::exception& e) { pa_abort(e.what()); }
+    MultiShared M(ngpus);
+    std::vector<std::thread> th;
+    for (int r = 0; r < ngpus; ++r) th.emplace_back([&, r] {
+        try { filter_rank(r, M, J); } catch (std::exception& e) { pa_abort(e.what()); }
+    });
+    for (auto& t : th) t.join();
+    std::vector<int> rr(std::max(J.Nlev - 1, 0), 2);              // write_plotfile hard-codes ref_ratio 2 (filterPlt.cpp:50)
+    try { pltio::write_metadata(J.outfile, *J.meta, J.names, J.Nlev, M.records, rr); } catch (std::exception& e) { pa_abort(e.what()); }
+    std::cout << "Done!" << std::endl;
+}

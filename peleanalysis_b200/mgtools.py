@@ -5,10 +5,13 @@
     python -m peleanalysis_b200.mgtools curvature infile=plt00100 [progressName=temp] [progMin=.. progMax=..] [useFileMinMax=1]
                                                   [threshold_prog=0 threshold_value=1e-4] [do_gaussCurv=0] [do_strain=0]
                                                   [getStrainTensor=0] [do_velnormal=0] [Aux_Variables=..] [is_per=..] [sym_dir=..]
+    python -m peleanalysis_b200.mgtools filter    infile=plt00100 [variables=a b] [max_filter_level=N] [filter_type=1] [base_fgr=2]
+                                                  [same_fgr_all_levels=0] [max_grid_size=32] [interp_type=1]
     python -m torch.distributed.run --nproc-per-node 8 -m peleanalysis_b200.mgtools grad infile=... [transport=peer|slab]
 
-Same keys, same output variable names and the same plotfile format as R/Src/grad.cpp / curvature.cpp (and as the C++ shells
-in host/).  What an MPI build of the reference does, rank by rank, is done here process by process: every rank reads the
+Same keys, same output variable names and the same plotfile format as R/Src/grad.cpp / curvature.cpp / filterPlt.cpp (and
+as the C++ shells in host/).  filter spreads the boxes re-chopped to max_grid_size over the ranks; the FillPatch sources of
+other ranks move as packed slabs (multigpu.FillPatchExchange).  What an MPI build of the reference does, rank by rank, is done here process by process: every rank reads the
 metadata, owns the boxes the SFC distribution gives it, reads only those from disk, runs the C-ABI calls on its GPU (cross-
 rank ghost cells through peer links over NVLink or NCCL slab exchange, multigpu.py), writes its own boxes to its own
 Level_l/Cell_D_<rank> file, and rank 0 writes Header and Cell_H from the gathered per-box (file, offset, min, max) records --
@@ -134,7 +137,7 @@ def run(tool: str, argv: Sequence[str], capi=None, multigpu=None, wrap=None, bac
         from . import capi as _capi
         capi = _capi
     pp = parse_args(argv)
-    if tool not in ("grad", "curvature") or "infile" not in pp:
+    if tool not in ("grad", "curvature", "filter") or "infile" not in pp:
         raise SystemExit(__doc__)
     dev = device if device is not None else int(os.environ.get("LOCAL_RANK", "0"))
     D = _Dist(backend, dev)
@@ -143,6 +146,8 @@ def run(tool: str, argv: Sequence[str], capi=None, multigpu=None, wrap=None, bac
         multigpu = _mg
     infile = pp["infile"][0]
     hd = plotfile.read_header(infile)
+    if tool == "filter":
+        return _filter(pp, infile, hd, capi, multigpu, wrap, backend, D, dev)
     nlev = min(_get(pp, "finestLevel", 1000, int), hd["finest"]) + 1
     is_per = _ints3(pp, "is_per", (1, 1, 1))
     sym_dir = _ints3(pp, "sym_dir", (0, 0, 0))
@@ -303,6 +308,84 @@ def run(tool: str, argv: Sequence[str], capi=None, multigpu=None, wrap=None, bac
     allrec = [r for part in D.gather_objects(records) for r in part]
     if D.rank == 0:
         _write_metadata(outfile, hd, levels, nlev, out_names, allrec, 0.0)
+    D.barrier()
+    D.close()
+    return outfile
+
+
+def _filter(pp, infile, hd, capi, multigpu, wrap, backend, D, dev) -> str:
+    """filterPlt (filterPlt.cpp:100-222) with this rank's share of the re-chopped boxes."""
+    from . import filterplt
+    variables = pp.get("variables") or None
+    for v in variables or []:
+        if v not in hd["names"]:
+            raise SystemExit("Variable '%s' not found in file" % v)
+    nfile = hd["finest"] + 1
+    metas = [plotfile.read_cell_h(infile, hd["paths"][l]) for l in range(nfile)]
+    levels = [plotfile.Level(hd["domains"][l][0], hd["domains"][l][1], hd["dx"][l], metas[l][1], []) for l in range(nfile)]
+    pf = plotfile.Plotfile(list(hd["names"]), hd["prob_lo"], hd["prob_hi"], hd["ref_ratio"], levels, hd["time"], hd["coord"])
+    mgs = _get(pp, "max_grid_size", 32, int)
+    capi.init(dev)
+    if D.world > 1 and backend == "nccl":
+        import torch
+        capi.set_stream(torch.cuda.current_stream().cuda_stream)
+    kw = {} if wrap is None else {"wrap": wrap}
+    R = filterplt.FilterRun(capi, pf, filter_type=_get(pp, "filter_type", 1, int), base_fgr=_get(pp, "base_fgr", 2, int),
+                            same_fgr_all_levels=bool(_get(pp, "same_fgr_all_levels", 0, int)), max_grid_size=mgs,
+                            interp_type=_get(pp, "interp_type", 1, int), variables=variables,
+                            max_filter_level=_get(pp, "max_filter_level", 1000, int), upload=False, rank=D.rank, nranks=D.world,
+                            multigpu=multigpu, **kw)
+    comps = [hd["names"].index(n) for n in R.names]
+    # this rank's output boxes, cut from the plotfile boxes that contain them (only those FABs are read)
+    for l in range(R.nlev):
+        parent = [b for b, bx in enumerate(levels[l].boxes) for _ in capi.boxes_max_size([bx], mgs)]
+        ids = R.hier.local_boxes[l]
+        if not ids:
+            continue
+        host = np.empty((len(comps), R.hier.local_cells[l]))
+        o, i = 0, 0
+        while i < len(ids):
+            pb = parent[ids[i]]
+            (lo, hi) = levels[l].boxes[pb]
+            data = read_boxes(infile, hd, l, metas[l], [pb], comps).reshape(len(comps), hi[2] - lo[2] + 1, hi[1] - lo[1] + 1, hi[0] - lo[0] + 1)
+            while i < len(ids) and parent[ids[i]] == pb:
+                clo, chi = R.levels[l].boxes[ids[i]]
+                blk = data[(slice(None),) + tuple(slice(clo[d] - lo[d], chi[d] - lo[d] + 1) for d in (2, 1, 0))].reshape(len(comps), -1)
+                host[:, o:o + blk.shape[1]] = blk
+                o += blk.shape[1]
+                i += 1
+        for c in range(len(comps)):
+            R.fin.upload_level(l, c, np.ascontiguousarray(host[c]))
+            capi.sync()
+    D.barrier()
+    R.step()
+    capi.sync()
+    D.barrier()
+    outfile = file_root(infile) + "_filtered"
+    if D.rank == 0:
+        if os.path.lexists(outfile):
+            os.rename(outfile, plotfile.unique_old_name(outfile))
+        os.makedirs(outfile)
+        for l in range(R.nlev):
+            os.makedirs(os.path.join(outfile, "Level_%d" % l))
+    D.barrier()
+    records = []
+    res = R.result()
+    fn = "Cell_D_%05d" % D.rank
+    for l in range(R.nlev):
+        if not R.hier.local_boxes[l]:
+            continue
+        with open(os.path.join(outfile, "Level_%d" % l, fn), "wb") as f:
+            for b in R.hier.local_boxes[l]:
+                lo, hi = R.levels[l].boxes[b]
+                blk = res[l][b].reshape(R.ncomp, -1)
+                off = f.tell()
+                f.write(("FAB ((8, (64 11 52 0 1 12 0 1023)),(8, (8 7 6 5 4 3 2 1)))%s %d\n" % (plotfile._box_str(lo, hi), R.ncomp)).encode())
+                f.write(np.ascontiguousarray(blk, dtype="<f8").tobytes())
+                records.append((l, b, fn, off, blk.min(axis=1).tolist(), blk.max(axis=1).tolist()))
+    allrec = [r for part in D.gather_objects(records) for r in part]
+    if D.rank == 0:
+        _write_metadata(outfile, hd, R.levels, R.nlev, R.names, allrec, hd["time"])    # ref_ratio 2 (filterPlt.cpp:50)
     D.barrier()
     D.close()
     return outfile

@@ -87,6 +87,41 @@ class SlabExchange:
         capi.check(capi.lib().pa_exchange_mark_received(f.f, comp, self.ncomp))
 
 
+class FillPatchExchange:
+    """NCCL send/recv of the packed slabs of one pa_fill_patch(lev, nghost, interp_type) on ncomp components of a field: the
+    same-level neighbours and coarse-patch cells owned by another rank than the box they fill.  pack -> send/recv -> mark;
+    then capi.fill_patch with the same arguments reads the recv slab.  The slabs are shared by every fill of the hierarchy and
+    grow to the largest plan, so their pointers are taken afresh at every run."""
+
+    def __init__(self, field: capi.Field, ncomp: int, lev: int, nghost: int, interp_type: int = 1, wrap=_wrap_device):
+        """wrap(ptr, n): raw slab pointer -> tensor for the process group's backend (CUDA tensors for NCCL)."""
+        H = field.hier
+        self.field, self.ncomp, self.lev, self.nghost, self.interp_type = field, ncomp, lev, nghost, interp_type
+        self.rank, self.world, self.wrap = H.rank, H.nranks, wrap
+        # the plan (and the nesting verdict, the same on every rank) is built here, before any communication
+        _, _, self.soff, self.roff = capi.fill_patch_exchange_buffers(field, ncomp, lev, nghost, interp_type)
+        self.bytes_sent = 8 * self.soff[-1]
+
+    def run(self, comp: int = 0) -> None:
+        if self.world == 1:
+            return
+        f, a = self.field, (self.lev, self.nghost, self.interp_type)
+        sp, rp, so, ro = capi.fill_patch_exchange_buffers(f, self.ncomp, *a)
+        capi.fill_patch_pack(f, comp, self.ncomp, *a)
+        ops = []
+        for p in range(self.world):
+            if p == self.rank:
+                continue
+            if ro[p + 1] > ro[p]:
+                ops.append(dist.P2POp(dist.irecv, self.wrap(rp + 8 * ro[p], ro[p + 1] - ro[p]), p))
+            if so[p + 1] > so[p]:
+                ops.append(dist.P2POp(dist.isend, self.wrap(sp + 8 * so[p], so[p + 1] - so[p]), p))
+        if ops:
+            for w in dist.batch_isend_irecv(ops):
+                w.wait()
+        capi.fill_patch_mark_received(f, comp, self.ncomp, *a)
+
+
 class Curvature:
     """The curvature tool on a multi-rank hierarchy: its steps (pa_curvature_steps) with the cross-rank step each one needs
     in front of it.
