@@ -755,6 +755,13 @@ static void poly_interp_coeff(double xInt, const double* x, int N, double* c) {
 }
 
 std::string Hier::build_faces() {
+    // level 0 must cover the domain.  Decided over every box of the level, not only this rank's, so that on several ranks
+    // every rank rejects the same hierarchy before any communication (the same first box, hence the same message, as the
+    // per-record check below finds on one rank).
+    for (int gb = 0; gb < (int)lev[0].boxes.size(); ++gb)
+        for (int face = 0; face < 6; ++face)
+            if (!face_is_physical(*this, 0, gb, face) && face_has_uncovered(*this, 0, gb, face))
+                return "level 0 does not cover the domain (box " + std::to_string(gb) + " has an interior face with no neighbour)";
     faces = FaceTable();
     faces.level_rec_begin.assign(nlev + 1, 0);
     std::vector<uint8_t> m;

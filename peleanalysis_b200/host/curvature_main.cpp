@@ -2,7 +2,7 @@
 // in/out and output names; progress variable, flame normal, mean curvature and the optional Gaussian curvature /
 // strain rate / normal velocity branches run through the C ABI.  do_smooth is the one key not served (it needs a
 // multigrid solve): the shell aborts if it is set.  Extension: ngpus=N runs on N GPUs from this one process, one host thread
-// per GPU (multi_gpu.hpp).
+// per GPU (multi_gpu.hpp); transport=peer|slab picks peer links + packed slabs (default) or packed slabs only.
 #include <algorithm>
 
 #include "multi_gpu.hpp"
@@ -113,8 +113,13 @@ int main(int argc, char** argv) {
 
     int ngpus = 1;
     pp.query("ngpus", ngpus);
+    std::string transport = "peer";
+    pp.query("transport", transport);
+    if (transport != "peer" && transport != "slab") pa_abort("transport must be peer or slab (got " + transport + ")");
     if (ngpus > 1) {
         CurvJob J;
+        J.peer = transport == "peer";
+        J.verbose = verbose != 0;
         J.infile = plotFileName; J.outfile = outfile; J.H = &H; J.Nlev = Nlev;
         J.inNames = inNames; J.velNames = velNames; J.names = names; J.need_vel = need_vel; J.o = o;
         J.slot = slot; J.zero_slots = zero_slots; J.nCompOut = nCompOut; J.is_per = is_per;

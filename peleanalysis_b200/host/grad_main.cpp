@@ -4,6 +4,8 @@
 //   grad3d.b200.ex infile=<plotfile> [gradVar=temp] [finestLevel=N] [Aux_Variables=a b ...] [is_per=1 1 1]
 //                  [sym_dir=0 0 0] [outfile=<name>]          extensions: gradVars=a b c  (several variables, one pass)
 //                                                                        ngpus=N  (one host thread per GPU, multi_gpu.hpp)
+//                                                                        transport=peer|slab  (with ngpus=N: peer links +
+//                                                                        packed slabs, or packed slabs only)
 #include <chrono>
 
 #include "multi_gpu.hpp"
@@ -51,9 +53,14 @@ int main(int argc, char** argv) {
 
     int ngpus = 1;
     pp.query("ngpus", ngpus);
+    std::string transport = "peer";
+    pp.query("transport", transport);
+    if (transport != "peer" && transport != "slab") pa_abort("transport must be peer or slab (got " + transport + ")");
     if (ngpus > 1) {
         GradJob J;
         J.infile = infile; J.H = &H; J.Nlev = Nlev; J.gvars = gvars; J.aux = aux; J.is_per = is_per;
+        J.peer = transport == "peer";
+        J.verbose = verbose != 0;
         for (int d = 0; d < 3; ++d) J.bck[d] = sym_dir[d] ? PA_BC_REFLECT_ODD : PA_BC_NEUMANN;
         for (auto& v : gvars) J.names.push_back(v);
         for (auto& a : aux) J.names.push_back(a);

@@ -1,12 +1,18 @@
-// multi_gpu.hpp -- the grad tool on several GPUs of one node from ONE process: one host thread per GPU, no MPI, no NCCL.
+// multi_gpu.hpp -- the grad, curvature and filterPlt tools on several GPUs of one node from ONE process: one host thread per
+// GPU, no MPI, no NCCL.
 //
 // What an MPI build of the reference does rank by rank (boxes distributed by DistributionMapping, ghost cells through
 // FillBoundary / ParallelCopy, one Cell_D file per rank) is done here thread by thread: thread r owns GPU r and the boxes the
-// SFC distribution gives rank r, reads only those from disk, maps the other threads' level slabs as peers
-// (pa_field_map_peer_ptr: the stencil kernels then read cross-GPU neighbour faces in place over NVLink), moves whatever the
-// neighbour links do not cover as packed slabs with device-to-device copies (pa_copy_async), runs pa_grad, and writes its
-// own boxes to Level_l/Cell_D_<r>; thread 0 writes Header and Cell_H.  Barriers between threads stand where the reference
-// has MPI synchronisation: before anyone reads a peer's slab, and before anyone frees a slab a peer may still read.
+// SFC distribution gives rank r, reads only those from disk, moves the ghost sources owned by other threads as packed slabs
+// with device-to-device copies (pa_copy_async), runs the tool's C-ABI calls, and writes its own boxes to Level_l/Cell_D_<r>;
+// thread 0 writes Header and Cell_H.  Barriers between threads stand where the reference has MPI synchronisation: before
+// anyone reads a peer's slab, and before anyone frees a slab a peer may still read.
+// grad and curvature have two transports (key transport=peer|slab): with peer links (the default) every thread also maps the
+// other threads' level slabs (pa_field_map_peer_ptr) and the stencil kernels read cross-GPU neighbour faces and coarse cells in
+// place over NVLink, so only the ragged remainder travels in the slabs; with transport=slab no field slab is mapped and every
+// ghost source of another thread travels in the slabs (the width-1 exchange plan of hier.cpp: build_exchange), as filterPlt's
+// FillPatch sources always do.  Every transport enables peer access between the GPUs: it lets the copy engines move the
+// pa_copy_async copies GPU to GPU directly instead of through host memory.
 #pragma once
 #include <condition_variable>
 #include <cstdio>
@@ -30,7 +36,7 @@ private:
 };
 
 struct MultiShared {
-    explicit MultiShared(int n) : n(n), bar(n), slab(n), send(n, nullptr), soff(n) {}
+    explicit MultiShared(int n) : n(n), bar(n), slab(n), send(n, nullptr), soff(n), mapped(n, 0), received(n, 0) {}
     int n;
     ThreadBarrier bar;
     std::mutex mu;
@@ -39,7 +45,18 @@ struct MultiShared {
     std::vector<std::vector<int64_t>> soff;            // [rank][peer .. ]: offsets into it
     std::vector<pltio::FabRecord> records;             // what every thread wrote
     long long launches = 0;
+    std::vector<long long> mapped;                     // [rank]: peer level slabs mapped (pa_field_map_peer_ptr calls)
+    std::vector<long long> received;                   // [rank]: doubles received through the slabs over the whole run
 };
+
+// verbose=1: what crossed between the GPUs, one line (the transport is visible in it: no slab is mapped with transport=slab)
+inline void print_transport_report(const MultiShared& M, bool peer) {
+    std::cout << "[b200] transport=" << (peer ? "peer" : "slab") << ": peer slabs mapped per GPU";
+    for (long long v : M.mapped) std::cout << " " << v;
+    std::cout << "; doubles received through slabs per GPU";
+    for (long long v : M.received) std::cout << " " << v;
+    std::cout << std::endl;
+}
 
 // every thread publishes the level slabs of its fields, then maps everyone else's (collective: all threads call it with the
 // same number of fields in the same order)
@@ -51,7 +68,10 @@ inline void map_all_peers(int r, MultiShared& M, int nlev, const std::vector<pa_
     for (int p = 0; p < M.n; ++p)
         if (p != r)
             for (size_t f = 0; f < fields.size(); ++f)
-                for (int l = 0; l < nlev; ++l) check(pa_field_map_peer_ptr(fields[f], l, p, M.slab[p][f * nlev + l]), "pa_field_map_peer_ptr");
+                for (int l = 0; l < nlev; ++l) {
+                    check(pa_field_map_peer_ptr(fields[f], l, p, M.slab[p][f * nlev + l]), "pa_field_map_peer_ptr");
+                    ++M.mapped[r];
+                }
     M.bar.wait();
 }
 
@@ -74,6 +94,7 @@ inline void exchange_slabs(int r, MultiShared& M, pa_field* f, int comp, int nco
         if (cnt != M.soff[p][r + 1] - M.soff[p][r]) pa_abort("multi-GPU exchange plan: send / recv counts disagree");
         if (cnt > 0) check(pa_copy_async(recv + ro[p], M.send[p] + M.soff[p][r], cnt), "pa_copy_async");
     }
+    M.received[r] += ro[n];
     check(pa_exchange_mark_received(f, comp, ncomp), "pa_exchange_mark_received");
     check(pa_sync(), "pa_sync");
     M.bar.wait();                                      // the send slabs may be repacked from here on
@@ -86,8 +107,13 @@ struct GradJob {
     std::vector<std::string> gvars, aux, names;
     std::vector<int> is_per;
     int bck[3];
+    bool peer = true;                                  // transport=peer (peer links + slabs) or slab (packed slabs only)
+    bool verbose = false;                              // print_transport_report after the run
     std::vector<std::vector<int>> owner;               // [level][box] -> rank
 };
+
+// the hierarchy flags of a grad / curvature rank for its transport
+inline unsigned transport_flags(bool peer) { return peer ? PA_HIER_PEER_LINKS : 0u; }
 
 inline void grad_rank(int r, MultiShared& M, const GradJob& J) {
     const pltio::Header& H = *J.H;
@@ -104,7 +130,7 @@ inline void grad_rank(int r, MultiShared& M, const GradJob& J) {
         for (int b = 0; b < (int)own[l].size(); ++b) if (own[l][b] == r) mine[l].push_back(b);
     }
     pa_hier* h = nullptr;
-    check(pa_hier_create2(&h, Nlev, hi.lv.data(), J.is_per.data(), J.bck, r, n, PA_HIER_PEER_LINKS), "pa_hier_create2");
+    check(pa_hier_create2(&h, Nlev, hi.lv.data(), J.is_per.data(), J.bck, r, n, transport_flags(J.peer)), "pa_hier_create2");
     pa_field *fin = nullptr, *fout = nullptr;
     check(pa_field_alloc(h, nv, 1, &fin), "pa_field_alloc");
     check(pa_field_alloc(h, 4 * nv, 0, &fout), "pa_field_alloc");
@@ -124,7 +150,7 @@ inline void grad_rank(int r, MultiShared& M, const GradJob& J) {
     }
     check(pa_sync(), "pa_sync");
 
-    map_all_peers(r, M, Nlev, {fin});
+    if (J.peer) map_all_peers(r, M, Nlev, {fin});
     exchange_slabs(r, M, fin, 0, nv);
 
     check(pa_grad(fin, 0, nv, fout, 0), "pa_grad");
@@ -174,6 +200,7 @@ inline void run_grad_multi(int ngpus, GradJob& J) {
         try { grad_rank(r, M, J); } catch (std::exception& e) { pa_abort(e.what()); }
     });
     for (auto& t : th) t.join();
+    if (J.verbose) print_transport_report(M, J.peer);
     std::vector<int> rr(std::max(J.Nlev - 1, 0), 2);              // the reference hard-codes refRatios = 2 (grad.cpp:255)
     pltio::Header meta = H;
     meta.time = 0.0;                                               // WriteMultiLevelPlotfile(..., 0.0, ...) (grad.cpp:256)
@@ -193,6 +220,8 @@ struct CurvJob {
     int nCompOut;
     std::vector<int> is_per;
     int bck[3];
+    bool peer = true;                                    // as GradJob::peer
+    bool verbose = false;
     std::vector<std::vector<int>> owner;
 };
 
@@ -210,7 +239,7 @@ inline void curv_rank(int r, MultiShared& M, const CurvJob& J) {
         for (int b = 0; b < (int)own[l].size(); ++b) if (own[l][b] == r) mine[l].push_back(b);
     }
     pa_hier* h = nullptr;
-    check(pa_hier_create2(&h, Nlev, hi.lv.data(), J.is_per.data(), J.bck, r, n, PA_HIER_PEER_LINKS), "pa_hier_create2");
+    check(pa_hier_create2(&h, Nlev, hi.lv.data(), J.is_per.data(), J.bck, r, n, transport_flags(J.peer)), "pa_hier_create2");
     const int nres = pa_curvature_num_outputs(&J.o);
     pa_field *st = nullptr, *res = nullptr, *scratch = nullptr;
     check(pa_field_alloc(h, J.need_vel ? 4 : 1, 1, &st), "pa_field_alloc");
@@ -237,7 +266,7 @@ inline void curv_rank(int r, MultiShared& M, const CurvJob& J) {
     check(pa_sync(), "pa_sync");
     std::vector<pa_field*> fields{st, res};
     if (scratch) fields.push_back(scratch);
-    map_all_peers(r, M, Nlev, fields);
+    if (J.peer) map_all_peers(r, M, Nlev, fields);
 
     auto step = [&](int steps, int lo, int hi) { check(pa_curvature_steps(st, 0, 1, &J.o, res, 0, steps, lo, hi), "pa_curvature_steps"); };
     exchange_slabs(r, M, st, 0, 1);
@@ -246,10 +275,13 @@ inline void curv_rank(int r, MultiShared& M, const CurvJob& J) {
         for (int l = 0; l < Nlev; ++l) {
             exchange_slabs(r, M, res, 2, 3);
             step(PA_CURV_DIV, l, l);
-            // the clip zeroes n(l) in place; every rank's DIV(l) reads its peers' UNCLIPPED n(l) over the links first
-            // (curvature.cpp:487-567: FillBoundary of n precedes the clip)
-            check(pa_sync(), "pa_sync");
-            M.bar.wait();
+            // the clip zeroes n(l) in place; with peer links every rank's DIV(l) reads its peers' UNCLIPPED n(l) over the links
+            // first (curvature.cpp:487-567: FillBoundary of n precedes the clip).  With transport=slab the peers' cells of n(l)
+            // were copied inside exchange_slabs, which ends in a barrier: nothing reads n(l) in place.
+            if (J.peer) {
+                check(pa_sync(), "pa_sync");
+                M.bar.wait();
+            }
             step(PA_CURV_CLIP, l, l);
         }
     } else {
@@ -297,6 +329,7 @@ inline void run_curv_multi(int ngpus, CurvJob& J) {
         try { curv_rank(r, M, J); } catch (std::exception& e) { pa_abort(e.what()); }
     });
     for (auto& t : th) t.join();
+    if (J.verbose) print_transport_report(M, J.peer);
     std::vector<int> rr(std::max(J.Nlev - 1, 0), 2);              // curvature.cpp:842
     pltio::Header meta = H;
     meta.time = 0.0;
