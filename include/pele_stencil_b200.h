@@ -31,7 +31,8 @@ typedef enum {
     PA_ERR_CUDA = -2,       /* CUDA runtime error or no usable device */
     PA_ERR_NOMEM = -3,
     PA_ERR_UNSUPPORTED = -4,
-    PA_ERR_STATE = -5       /* call order (e.g. remote halo data not exchanged yet) */
+    PA_ERR_STATE = -5,      /* call order (e.g. remote halo data not exchanged yet) */
+    PA_ERR_NOCONV = -6      /* an iterative solve did not converge (pa_last_error gives the residual reached) */
 } pa_status;
 
 /* Domain-boundary kinds for NON-periodic directions: LinOpBCType::Neumann / reflect_odd as chosen by the
@@ -61,6 +62,14 @@ typedef struct {
     int do_velnormal;                 /* do_velnormal */
     int reserved[8];
 } pa_curv_opts;
+
+/* Options of curvature's do_smooth (ParmParse smoothing_time of Src/curvature.cpp:72-106; the solve of :328-406). */
+typedef struct {
+    double smoothing_time;            /* smoothing_time: beta of phi - beta * div(grad phi) = c (>= 0) */
+    double tol_rel;                   /* stop when max|c - A phi| <= tol_rel * max|c| over uncovered cells; 0 = 1e-10 */
+    int max_iter;                     /* iterations before PA_ERR_NOCONV; 0 = 1000 */
+    int reserved[8];
+} pa_smooth_opts;
 
 /* ---- runtime ------------------------------------------------------------------------------------- */
 /* Select the CUDA device of this process (one process per GPU).  amrex::Initialize's device part. */
@@ -198,6 +207,21 @@ int pa_curvature_steps(pa_field *state, int comp_S, int comp_vel, const pa_curv_
 /* Internal field a multi-rank caller must exchange / peer-map: which = 0, the un-normalised gradient of the progress
  * variable (3 components, nghost 1).  Owned by the hierarchy; do not free. */
 int pa_curvature_scratch(pa_hier *h, int which, pa_field **f);
+
+/* ---- do_smooth: one backward-Euler diffusion step of the progress variable (Src/curvature.cpp:328-406) ----------------------
+ * The reference builds MLABecLaplacian(alpha = 1, a = 1, beta = smoothing_time, b = 1) on all levels and MLMG-solves
+ *     phi - beta * div(grad phi) = c,   c = (S - prog_min) / (prog_max - prog_min),
+ * as one composite AMR system: the 7-point operator on every valid cell with the ghost cells of pa_fill_ghosts (same-level /
+ * periodic copies, Neumann / reflect_odd walls, the coarse-fine polynomial through the o3-interpolated coarse value, here of
+ * maxorder 3), the coarse side of every coarse-fine face taking the average of the fine face fluxes, covered coarse cells holding
+ * the average of their fine cells.  Writes c into out[comp_c] -- bit-identical to pa_curvature's Progress -- and phi into
+ * out[comp_phi]; the curvature of the smoothed field is then pa_curvature on phi with prog_min = 0, prog_max = 1.
+ * Solver: right-preconditioned BiCGStab on the composite residual, deterministic (fixed reduction order); the stop test is on
+ * the TRUE residual.  *iters = iterations, *resid = max|c - A phi| / max|c| over uncovered cells (both may be NULL).
+ * smoothing_time = 0 copies c into phi bit for bit.  One rank and refinement ratio 2 only (PA_ERR_UNSUPPORTED otherwise);
+ * negative smoothing_time: PA_ERR_ARG; not converged within max_iter: PA_ERR_NOCONV, phi not written. */
+int pa_smooth(pa_field *state, int comp_S, double prog_min, double prog_max, const pa_smooth_opts *o, pa_field *out, int comp_c,
+              int comp_phi, int *iters, double *resid);
 
 /* ---- filterPlt: the neighbouring stencil tool (Src/filterPlt.cpp:100-222; SURVEY 8(f) rank 4) -------------------------
  * PP/ = Submodules/PelePhysics/Source.  The tool re-chops the plotfile's grids to max_grid_size, fills nGrow = fgr/2 ghost

@@ -32,6 +32,14 @@ class CurvOpts(C.Structure):
                 ("get_strain_tensor", C.c_int), ("do_velnormal", C.c_int), ("reserved", C.c_int * 8)]
 
 
+class SmoothOpts(C.Structure):
+    """pa_smooth_opts: smoothing_time (>= 0), tol_rel (0 = 1e-10), max_iter (0 = 1000)."""
+    _fields_ = [("smoothing_time", C.c_double), ("tol_rel", C.c_double), ("max_iter", C.c_int), ("reserved", C.c_int * 8)]
+
+
+PA_ERR_UNSUPPORTED, PA_ERR_NOCONV = -4, -6
+
+
 # every symbol include/pele_stencil_b200.h declares: (restype, argtypes)
 _vp, _i, _i64, _d = C.c_void_p, C.c_int, C.c_int64, C.c_double
 SYMBOLS = {
@@ -84,6 +92,7 @@ SYMBOLS = {
     "pa_fill_patch_pack": (_i, [_vp, _i, _i, _i, _i, _i]), "pa_fill_patch_mark_received": (_i, [_vp, _i, _i, _i, _i, _i]),
     "pa_debug_fill_patch_exchange_ids": (_i64, [_vp, _i, _i, _i, _i, _vp, _i64]),
     "pa_filter": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _i]),
+    "pa_smooth": (_i, [_vp, _i, _d, _d, C.POINTER(SmoothOpts), _vp, _i, _i, C.POINTER(_i), C.POINTER(_d)]),
 }
 
 _lib = None
@@ -488,6 +497,15 @@ def fill_patch_mark_received(f: Field, comp: int, ncomp: int, lev: int, nghost: 
 
 def filter_level(inp: Field, comp_in: int, out: Field, comp_out: int, ncomp: int, lev: int, filter_type: int, fgr: int) -> None:
     check(lib().pa_filter(inp.f, comp_in, out.f, comp_out, ncomp, lev, filter_type, fgr))
+
+
+def smooth(state: Field, comp_S: int, prog_min: float, prog_max: float, opts: SmoothOpts, out: Field, comp_c: int, comp_phi: int):
+    """curvature's do_smooth (curvature.cpp:328-406): c = (S - prog_min) / (prog_max - prog_min) into out[comp_c], the solution
+    phi of phi - smoothing_time * div(grad phi) = c on the composite hierarchy into out[comp_phi].  Returns (iterations,
+    relative residual); raises PaError (code PA_ERR_NOCONV) if the solve does not converge."""
+    it, res = C.c_int(0), C.c_double(0.0)
+    check(lib().pa_smooth(state.f, comp_S, prog_min, prog_max, C.byref(opts), out.f, comp_c, comp_phi, C.byref(it), C.byref(res)))
+    return it.value, res.value
 
 
 def curvature_num_outputs(opts: CurvOpts) -> int:

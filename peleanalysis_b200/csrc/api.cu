@@ -77,6 +77,15 @@ struct TileTable {
     bool ok = true;
 };
 
+// pa_smooth: the composite operator's tables on the device and the solver's work fields (allocated on the first call)
+struct SmoothDev {
+    DevBuf<PaFaceRec> recs;                            // face records with the smoothing operator's coarse-fine polynomial
+    DevBuf<PaAvgDown> avg;
+    DevBuf<PaReflux> reflux;
+    DevBuf<double> partial, scal;                      // reduction partials and the reduced scalar
+    pa_field* w[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+};
+
 }  // namespace
 
 struct pa_hier {
@@ -132,6 +141,7 @@ struct pa_hier {
     pa_field* tmpG = nullptr;
     pa_field* tmpH = nullptr;
     pa_field* tmpW = nullptr;
+    std::unique_ptr<SmoothDev> sm;
 };
 
 struct pa_field {
@@ -560,7 +570,9 @@ int check_field(const pa_field* f, int comp, int ncomp, const char* who) {
 // ghost fill of comps [comp, comp+ncomp) on levels [l0, l1]: halo gather per level + one BC-fill launch.
 // linked_too = false (the product path): faces with a neighbour link are skipped -- the stencil kernels read the
 // neighbour in place; true: every ghost cell of the width-1 face layers is materialised (pa_fill_ghosts).
-int fill_ghosts_impl(pa_field* f, int comp, int ncomp, int l0, int l1, bool linked_too, GhostXform xf = GhostXform{0, 0.0, 1.0}) {
+// recs: face records to use instead of the hierarchy's (pa_smooth's coarse-fine polynomial order); same order and extents.
+int fill_ghosts_impl(pa_field* f, int comp, int ncomp, int l0, int l1, bool linked_too, GhostXform xf = GhostXform{0, 0.0, 1.0},
+                     const PaFaceRec* recs = nullptr) {
     pa_hier* h = f->h;
     Hier& H = h->H;
     CHK(ensure_device(h));
@@ -597,7 +609,7 @@ int fill_ghosts_impl(pa_field* f, int comp, int ncomp, int l0, int l1, bool link
             CU(cudaStreamSynchronize(t_stream));           // v dies at the end of this scope
             it = h->face_coff.emplace(f->ng, std::move(buf)).first;
         }
-        CU(launch_bcfill(h->face_recs.p, h->face_level.p, h->face_blocks.p, b0, b1, h->face_flags.p, it->second->p, ga, ncomp, recv, xf, t_stream));
+        CU(launch_bcfill(recs ? recs : h->face_recs.p, h->face_level.p, h->face_blocks.p, b0, b1, h->face_flags.p, it->second->p, ga, ncomp, recv, xf, t_stream));
     }
     return PA_OK;
 }
@@ -702,6 +714,7 @@ int pa_hier_destroy(pa_hier* h) {
     if (h->tmpG) pa_field_free(h->tmpG);
     if (h->tmpH) pa_field_free(h->tmpH);
     if (h->tmpW) pa_field_free(h->tmpW);
+    if (h->sm) for (pa_field* f : h->sm->w) if (f) pa_field_free(f);
     if (h->ev_fork) cudaEventDestroy(h->ev_fork);
     if (h->ev_join) cudaEventDestroy(h->ev_join);
     if (h->side) cudaStreamDestroy(h->side);
@@ -1501,6 +1514,246 @@ int pa_curvature_scratch(pa_hier* h, int which, pa_field** f) {
     CHK(ensure_device(h));
     CHK(tmp_field(h, &h->tmpG, 3));
     *f = h->tmpG;
+    return PA_OK;
+}
+
+// ---- do_smooth: one backward-Euler diffusion step of the progress variable (curvature.cpp:328-406) --------------------------
+}  // extern "C"
+namespace {
+
+// Order of the coarse-fine ghost polynomial of the smoothing operator.  AMReX's MLLinOp default maxorder is 3
+// (AMReX_MLLinOp.H, LPInfo / maxorder); the gradient passes of the tools call setMaxOrder(4) (grad.cpp:179,
+// curvature.cpp:426-441).  Whether curvature.cpp:328-406 calls setMaxOrder on its MLABecLaplacian is not verified here
+// (DESIGN.md section 10, point 1): 3 holds unless it does.
+constexpr int SMOOTH_MAXORDER = 3;
+constexpr double SMOOTH_TOL_REL = 1e-10;
+constexpr int SMOOTH_MAX_ITER = 1000;
+
+struct SmCtx {
+    pa_hier* h;
+    SmoothDev* S;
+    const SmoothTables* T;
+    double beta;
+    int nlev;
+    std::vector<const PaLayDev*> lay;   // nghost-1 layout per level (every work field)
+};
+
+// y = A x on every valid cell: covered cells of x <- fine averages, ghost fill, 7-point operator, reflux; y's covered cells <- 0
+int sm_matvec(SmCtx& c, pa_field* x, pa_field* y) {
+    pa_hier* h = c.h;
+    Hier& H = h->H;
+    const SmoothTables& T = *c.T;
+    for (int l = c.nlev - 2; l >= 0; --l)
+        CU(launch_sm_avgdown(c.S->avg.p + T.avg_begin[l], (int)(T.avg_begin[l + 1] - T.avg_begin[l]), T.avg_cells[l], h->lev[l]->boxes.p,
+                             c.lay[l], h->lev[l + 1]->boxes.p, c.lay[l + 1], x->slab[l], x->slab[l + 1], false, t_stream));
+    CHK(fill_ghosts_impl(x, 0, 1, 0, c.nlev - 1, true, GhostXform{0, 0.0, 1.0}, c.S->recs.p));
+    for (int l = 0; l < c.nlev; ++l) {
+        const LevelDev& D = *h->lev[l];
+        CU(launch_sm_apply(D.boxes.p, c.lay[l], D.host_off.p, (int)H.lev[l].local.size(), D.host_off_h.back(), x->slab[l], y->slab[l],
+                           c.beta, H.lev[l].dxinv, t_stream));
+    }
+    for (int l = 0; l + 1 < c.nlev; ++l)
+        for (int g = 0; g < 6; ++g) {
+            const long long a = T.reflux_begin[(size_t)l * 6 + g], b = T.reflux_begin[(size_t)l * 6 + g + 1];
+            const int d = g / 2;
+            CU(launch_sm_reflux(c.S->reflux.p + a, b - a, c.lay[l], c.lay[l + 1], x->slab[l], x->slab[l + 1], y->slab[l], c.beta,
+                                H.lev[l].dxinv[d], H.lev[l + 1].dxinv[d], t_stream));
+        }
+    for (int l = 0; l + 1 < c.nlev; ++l)
+        CU(launch_sm_avgdown(c.S->avg.p + T.avg_begin[l], (int)(T.avg_begin[l + 1] - T.avg_begin[l]), T.avg_cells[l], h->lev[l]->boxes.p,
+                             c.lay[l], h->lev[l + 1]->boxes.p, c.lay[l + 1], y->slab[l], nullptr, true, t_stream));
+    return PA_OK;
+}
+
+// out = a_l*x + b*y + cz*z on every level (whole slabs); a_l per level
+int sm_lin(SmCtx& c, const std::vector<double>& a, pa_field* x, double b, pa_field* y, double cz, pa_field* z, pa_field* out) {
+    for (int l = 0; l < c.nlev; ++l)
+        CU(launch_sm_lin3(out->cs[l], a[l], x->slab[l], b, y ? y->slab[l] : nullptr, cz, z ? z->slab[l] : nullptr, out->slab[l], t_stream));
+    return PA_OK;
+}
+
+// mode 0: sum over valid cells of x*y; mode 1: max |x| (NaN if any cell is NaN).  Fixed reduction order; synchronises.
+int sm_reduce(SmCtx& c, pa_field* x, pa_field* y, int mode, double* out) {
+    int off = 0;
+    for (int l = 0; l < c.nlev; ++l) {
+        const LevelDev& D = *c.h->lev[l];
+        int nb = 0;
+        CU(launch_sm_reduce(D.boxes.p, c.lay[l], D.host_off.p, (int)c.h->H.lev[l].local.size(), D.host_off_h.back(), x->slab[l],
+                            y ? y->slab[l] : nullptr, mode, c.S->partial.p + off, &nb, t_stream));
+        off += nb;
+    }
+    CU(launch_sm_final(c.S->partial.p, off, mode, c.S->scal.p, t_stream));
+    CU(cudaMemcpyAsync(out, c.S->scal.p, sizeof(double), cudaMemcpyDeviceToHost, t_stream));
+    CU(cudaStreamSynchronize(t_stream));
+    return PA_OK;
+}
+
+int ensure_smooth(pa_hier* h, const SmoothTables& T) {
+    if (h->sm) return PA_OK;
+    auto S = std::make_unique<SmoothDev>();
+    CU(S->recs.upload(T.recs, t_stream));
+    CU(S->avg.upload(T.avg, t_stream));
+    CU(S->reflux.upload(T.reflux, t_stream));
+    CU(S->partial.reserve((size_t)std::max(1, h->H.nlev) * smooth_max_partials()));
+    CU(S->scal.reserve(1));
+    CU(cudaStreamSynchronize(t_stream));
+    for (auto& f : S->w) {
+        int rc = pa_field_alloc(h, 1, 1, &f);
+        if (rc != PA_OK) { for (pa_field* g : S->w) if (g) pa_field_free(g); return rc; }
+    }
+    h->sm = std::move(S);
+    return PA_OK;
+}
+
+}  // namespace
+extern "C" {
+
+int pa_smooth(pa_field* state, int comp_S, double prog_min, double prog_max, const pa_smooth_opts* o, pa_field* out, int comp_c,
+              int comp_phi, int* iters, double* resid) {
+    if (iters) *iters = 0;
+    if (resid) *resid = 0.0;
+    if (!o) return fail(PA_ERR_ARG, "pa_smooth: null options");
+    CHK(check_field(state, comp_S, 1, "pa_smooth(state)"));
+    CHK(check_field(out, comp_c, 1, "pa_smooth(out, comp_c)"));
+    CHK(check_field(out, comp_phi, 1, "pa_smooth(out, comp_phi)"));
+    if (state->h != out->h) return fail(PA_ERR_ARG, "pa_smooth: fields belong to different hierarchies");
+    if (comp_c == comp_phi) return fail(PA_ERR_ARG, "pa_smooth: comp_c and comp_phi must differ");
+    if (out == state && (comp_c == comp_S || comp_phi == comp_S)) return fail(PA_ERR_ARG, "pa_smooth: the outputs would overwrite S");
+    if (!(prog_min < prog_max)) return fail(PA_ERR_ARG, "progMin must be less than progMax");   // curvature.cpp:157-159
+    const double t = o->smoothing_time;
+    if (!(t >= 0.0) || !std::isfinite(t)) return fail(PA_ERR_ARG, "pa_smooth: smoothing_time must be finite and >= 0");
+    if (!(o->tol_rel >= 0.0) || o->max_iter < 0) return fail(PA_ERR_ARG, "pa_smooth: tol_rel and max_iter must be >= 0 (0 = default)");
+    const double tol_rel = o->tol_rel > 0.0 ? o->tol_rel : SMOOTH_TOL_REL;
+    const int max_iter = o->max_iter > 0 ? o->max_iter : SMOOTH_MAX_ITER;
+    pa_hier* h = state->h;
+    Hier& H = h->H;
+    if (H.nranks > 1) return fail(PA_ERR_UNSUPPORTED, "pa_smooth supports one rank only (do_smooth is not available on several GPUs)");
+    if (H.filter_only) return fail(PA_ERR_UNSUPPORTED, "pa_smooth needs a hierarchy created without PA_HIER_FILTER_ONLY");
+    for (int l = 1; l < H.nlev; ++l)
+        if (H.lev[l].ratio != 2)
+            return fail(PA_ERR_UNSUPPORTED, "pa_smooth supports refinement ratio 2 only (curvature.cpp:445,518,842 hard-code it); level " +
+                                                std::to_string(l) + " has ratio " + std::to_string(H.lev[l].ratio));
+    CHK(ensure_device(h));
+    const SmoothTables& T = H.smooth_tables(SMOOTH_MAXORDER);
+    if (!T.err.empty()) return fail(PA_ERR_ARG, T.err);
+    CHK(ensure_smooth(h, T));
+    SmCtx c;
+    c.h = h; c.S = h->sm.get(); c.T = &T; c.beta = t; c.nlev = H.nlev;
+    for (int l = 0; l < H.nlev; ++l) {
+        int err = PA_OK;
+        const PaLayDev* ly = dev_layout(h, l, 1, &err);
+        if (!ly && !H.lev[l].local.empty()) return err;
+        c.lay.push_back(ly);
+    }
+    pa_field **w = c.S->w, *x = w[0], *b = w[1], *r = w[2], *r0 = w[3], *p = w[4], *v = w[5], *tt = w[6], *z = w[7];
+    // c = (S - progMin) * invdenom: pa_curvature's Progress arithmetic (curvature.cpp:310-321), into out and into b
+    const double invdenom = 1.0 / (prog_max - prog_min);
+    for (int l = 0; l < H.nlev; ++l) {
+        const LevelDev& D = *h->lev[l];
+        const int nb = (int)H.lev[l].local.size();
+        int err = PA_OK;
+        const PaLayDev* ls = dev_layout(h, l, state->ng, &err);
+        const PaLayDev* lo = dev_layout(h, l, out->ng, &err);
+        if (nb && (!ls || !lo)) return err;
+        const double* S = state->slab[l] + (long long)comp_S * state->cs[l];
+        CU(launch_progress(D.boxes.p, ls, lo, nb, S, out->slab[l] + (long long)comp_c * out->cs[l], prog_min, invdenom, t_stream));
+        if (t == 0.0)      // phi - 0 * Laplacian(phi) = c: phi is c, bit for bit
+            CU(launch_progress(D.boxes.p, ls, lo, nb, S, out->slab[l] + (long long)comp_phi * out->cs[l], prog_min, invdenom, t_stream));
+        else
+            CU(launch_progress(D.boxes.p, ls, c.lay[l], nb, S, b->slab[l], prog_min, invdenom, t_stream));
+    }
+    if (t == 0.0) return PA_OK;
+    const std::vector<double> one(H.nlev, 1.0), zero(H.nlev, 0.0);
+    std::vector<double> jac(H.nlev);         // right preconditioner: the inverse diagonal of each level's operator
+    for (int l = 0; l < H.nlev; ++l) {
+        const double* q = H.lev[l].dxinv;
+        jac[l] = 1.0 / (1.0 + 2.0 * t * (q[0] * q[0] + q[1] * q[1] + q[2] * q[2]));
+    }
+    CHK(sm_lin(c, one, b, 0.0, nullptr, 0.0, nullptr, x));                  // initial guess: c
+    for (int l = 0; l + 1 < H.nlev; ++l)                                    // the right-hand side lives on the uncovered cells
+        CU(launch_sm_avgdown(c.S->avg.p + T.avg_begin[l], (int)(T.avg_begin[l + 1] - T.avg_begin[l]), T.avg_cells[l], h->lev[l]->boxes.p,
+                             c.lay[l], h->lev[l + 1]->boxes.p, c.lay[l + 1], b->slab[l], nullptr, true, t_stream));
+    double bmax = 0.0;
+    CHK(sm_reduce(c, b, nullptr, 1, &bmax));
+    if (!std::isfinite(bmax)) return fail(PA_ERR_ARG, "pa_smooth: the progress variable has non-finite values");
+    const double tol = tol_rel * bmax;
+    // true residual r = b - A x
+    auto true_residual = [&](double* rn) -> int {
+        CHK(sm_matvec(c, x, tt));
+        CHK(sm_lin(c, one, b, -1.0, tt, 0.0, nullptr, r));
+        return sm_reduce(c, r, nullptr, 1, rn);
+    };
+    double rnorm = 0.0;
+    CHK(true_residual(&rnorm));
+    // Right-preconditioned BiCGStab on the composite operator, restarted from the true residual whenever the recurrence
+    // residual meets the tolerance but the true one does not, or on a breakdown.
+    int it = 0;
+    bool restart = true;
+    double rho_old = 1.0, alpha = 1.0, omega = 1.0;
+    while (!(rnorm <= tol)) {
+        if (it >= max_iter || !std::isfinite(rnorm)) {
+            if (iters) *iters = it;
+            if (resid) *resid = bmax > 0.0 ? rnorm / bmax : rnorm;
+            char msg[256];
+            std::snprintf(msg, sizeof msg, "pa_smooth: not converged after %d iterations: max|c - A phi| / max|c| = %.3e (tol_rel %.3e)", it,
+                          bmax > 0.0 ? rnorm / bmax : rnorm, tol_rel);
+            return fail(PA_ERR_NOCONV, msg);
+        }
+        if (restart) {
+            CHK(sm_lin(c, one, r, 0.0, nullptr, 0.0, nullptr, r0));
+            CHK(sm_lin(c, zero, r, 0.0, nullptr, 0.0, nullptr, p));
+            CHK(sm_lin(c, zero, r, 0.0, nullptr, 0.0, nullptr, v));
+            rho_old = alpha = omega = 1.0;
+            restart = false;
+        }
+        ++it;
+        double rho = 0.0;
+        CHK(sm_reduce(c, r0, r, 0, &rho));
+        if (rho == 0.0 || !std::isfinite(rho)) { restart = true; CHK(true_residual(&rnorm)); continue; }
+        const double bk = (rho / rho_old) * (alpha / omega);
+        CHK(sm_lin(c, one, r, bk, p, -bk * omega, v, p));                   // p = r + bk (p - omega v)
+        CHK(sm_lin(c, jac, p, 0.0, nullptr, 0.0, nullptr, z));               // z = M^-1 p
+        CHK(sm_matvec(c, z, v));                                             // v = A z
+        double den = 0.0;
+        CHK(sm_reduce(c, r0, v, 0, &den));
+        if (den == 0.0 || !std::isfinite(den)) { restart = true; CHK(true_residual(&rnorm)); continue; }
+        alpha = rho / den;
+        CHK(sm_lin(c, one, r, -alpha, v, 0.0, nullptr, r));                  // s = r - alpha v (in r)
+        CHK(sm_lin(c, one, x, alpha, z, 0.0, nullptr, x));                   // x += alpha z
+        double snorm = 0.0;
+        CHK(sm_reduce(c, r, nullptr, 1, &snorm));
+        rho_old = rho;
+        if (!(snorm <= tol)) {
+            CHK(sm_lin(c, jac, r, 0.0, nullptr, 0.0, nullptr, z));           // z = M^-1 s
+            CHK(sm_matvec(c, z, tt));                                        // t = A z
+            double ts = 0.0, t2 = 0.0;
+            CHK(sm_reduce(c, tt, r, 0, &ts));
+            CHK(sm_reduce(c, tt, tt, 0, &t2));
+            if (t2 == 0.0 || !std::isfinite(t2) || ts == 0.0) { restart = true; CHK(true_residual(&rnorm)); continue; }
+            omega = ts / t2;
+            CHK(sm_lin(c, one, x, omega, z, 0.0, nullptr, x));               // x += omega z
+            CHK(sm_lin(c, one, r, -omega, tt, 0.0, nullptr, r));             // r = s - omega t
+            CHK(sm_reduce(c, r, nullptr, 1, &snorm));
+        }
+        rnorm = snorm;
+        if (rnorm <= tol) {                                                  // converged by the recurrence: confirm on the true residual
+            CHK(true_residual(&rnorm));
+            if (!(rnorm <= tol)) restart = true;
+        }
+    }
+    // covered cells of phi <- fine averages, then phi -> out
+    for (int l = H.nlev - 2; l >= 0; --l)
+        CU(launch_sm_avgdown(c.S->avg.p + T.avg_begin[l], (int)(T.avg_begin[l + 1] - T.avg_begin[l]), T.avg_cells[l], h->lev[l]->boxes.p,
+                             c.lay[l], h->lev[l + 1]->boxes.p, c.lay[l + 1], x->slab[l], x->slab[l + 1], false, t_stream));
+    for (int l = 0; l < H.nlev; ++l) {
+        const LevelDev& D = *h->lev[l];
+        int err = PA_OK;
+        const PaLayDev* lo = dev_layout(h, l, out->ng, &err);
+        CU(launch_sm_copy(D.boxes.p, c.lay[l], lo, D.host_off.p, (int)H.lev[l].local.size(), D.host_off_h.back(), x->slab[l],
+                          out->slab[l] + (long long)comp_phi * out->cs[l], t_stream));
+    }
+    if (iters) *iters = it;
+    if (resid) *resid = bmax > 0.0 ? rnorm / bmax : 0.0;
     return PA_OK;
 }
 

@@ -956,4 +956,117 @@ void sfc_distribute(int nboxes, const int* boxes, int nranks, int* owner_out) {
     }
 }
 
+// Tables of pa_smooth's composite operator (see DESIGN.md section 10):
+//  * the box-face records with the coarse-fine polynomial of order `maxorder` (the halo tables, masks and coarse gather
+//    indices of faces are shared with every other ghost fill; only NX and the coefficients differ);
+//  * the covered coarse cells of every level, per (coarse box, fine box) intersection (average_down);
+//  * the coarse side of every coarse-fine face (reflux), one record per coarse face, found from the fine level's
+//    coarse-fine ghost cells (mask not_covered on a coarse-fine face record), periodic images included.
+const SmoothTables& Hier::smooth_tables(int maxorder) {
+    auto it = smooth_.find(maxorder);
+    if (it != smooth_.end()) return it->second;
+    SmoothTables T;
+    auto done = [&]() -> const SmoothTables& { return smooth_.emplace(maxorder, std::move(T)).first->second; };
+    if (nranks > 1) { T.err = "pa_smooth supports one rank only"; return done(); }
+    if (filter_only) { T.err = "pa_smooth needs a hierarchy created without PA_HIER_FILTER_ONLY"; return done(); }
+    for (int l = 1; l < nlev; ++l)
+        if (lev[l].ratio != 2) {
+            T.err = "pa_smooth supports refinement ratio 2 only (level " + std::to_string(l) + " has ratio " + std::to_string(lev[l].ratio) +
+                    "; curvature.cpp hard-codes 2)";
+            return done();
+        }
+    T.recs = faces.recs;
+    for (size_t q = 0; q < T.recs.size(); ++q) {
+        PaFaceRec& R = T.recs[q];
+        if (R.kind != PA_FACE_CF) continue;
+        const Level& V = lev[faces.rec_level[q]];
+        const int d = R.face % 3;
+        const Box& B = V.boxes[V.local[R.box]];
+        R.nx = std::min(B.len(d) + 1, maxorder);
+        double bcl = 0.5 * (double)R.ratio * V.dx[d];
+        double x[4] = {-bcl * V.dxinv[d], 0.5, 1.5, 2.5};
+        for (int m = 0; m < 4; ++m) R.coef[m] = 0.0;
+        poly_interp_coeff(-0.5, x, R.nx, R.coef);
+    }
+    T.avg_begin.assign(nlev + 1, 0);
+    T.avg_cells.assign(nlev, 0);
+    for (int lc = 0; lc < nlev; ++lc) {
+        T.avg_begin[lc] = (long long)T.avg.size();
+        if (lc + 1 >= nlev) continue;
+        const Level& C = lev[lc];
+        const Level& F = lev[lc + 1];
+        long long start = 0;
+        for (int fg : F.local) {
+            Box cb = F.boxes[fg];
+            for (int d = 0; d < 3; ++d) { cb.lo[d] = coarsen(cb.lo[d], 2); cb.hi[d] = coarsen(cb.hi[d], 2); }
+            std::vector<std::pair<int, Box>> is;
+            C.hash.query(cb, [&](int k, const Box& ib) { is.emplace_back(k, ib); });
+            std::sort(is.begin(), is.end(), [](const std::pair<int, Box>& a, const std::pair<int, Box>& b) { return a.first < b.first; });
+            for (auto& e : is) {
+                PaAvgDown A;
+                A.cbox = C.g2l[e.first]; A.fbox = F.g2l[fg];
+                for (int d = 0; d < 3; ++d) { A.lo[d] = e.second.lo[d]; A.n[d] = e.second.len(d); }
+                A.start = start;
+                start += e.second.npts();
+                T.avg.push_back(A);
+            }
+        }
+        T.avg_cells[lc] = start;
+    }
+    T.avg_begin[nlev] = (long long)T.avg.size();
+    std::map<std::array<int, 7>, PaReflux> rf;            // (coarse level, dir, side, coarse box, c[2], c[1], c[0])
+    for (int lf = 1; lf < nlev; ++lf) {
+        const Level& F = lev[lf];
+        const Level& C = lev[lf - 1];
+        for (long long q = faces.level_rec_begin[lf]; q < faces.level_rec_begin[lf + 1]; ++q) {
+            const PaFaceRec& R = faces.recs[q];
+            if (R.kind != PA_FACE_CF) continue;
+            const int gb = F.local[R.box];
+            const Box& B = F.boxes[gb];
+            const int d = R.face % 3;
+            const int t1 = (d == 0) ? 1 : 0, t2 = (d == 2) ? 1 : 2;
+            const bool lo_face = R.face < 3;
+            for (int a2 = 0; a2 < R.n2; ++a2)
+                for (int a1 = 0; a1 < R.n1; ++a1) {
+                    if (PA_FLAG_MASK(faces.flags[R.start + (long long)a2 * R.n1 + a1]) != 1) continue;
+                    int g[3];
+                    g[d] = lo_face ? B.lo[d] - 1 : B.hi[d] + 1;
+                    g[t1] = B.lo[t1] + a1; g[t2] = B.lo[t2] + a2;
+                    int w[3] = {g[0], g[1], g[2]};
+                    const int nd = F.dom.len(d);
+                    if (w[d] < F.dom.lo[d]) { if (!is_per[d]) continue; w[d] += nd; }
+                    if (w[d] > F.dom.hi[d]) { if (!is_per[d]) continue; w[d] -= nd; }
+                    int cc[3];
+                    for (int e = 0; e < 3; ++e) cc[e] = coarsen(w[e], 2);
+                    int cg = -1;
+                    Box one{{cc[0], cc[1], cc[2]}, {cc[0], cc[1], cc[2]}};
+                    C.hash.query(one, [&](int k, const Box&) { cg = k; });
+                    if (cg < 0) {
+                        T.err = "pa_smooth: level " + std::to_string(lf) + " is not properly nested in level " + std::to_string(lf - 1) +
+                                " (a coarse-fine face of box " + std::to_string(gb) + " has no coarse cell)";
+                        return done();
+                    }
+                    const Box& CB = C.boxes[cg];
+                    const int side = lo_face ? 1 : 0;
+                    std::array<int, 7> key{lf - 1, d, side, C.g2l[cg], cc[2] - CB.lo[2], cc[1] - CB.lo[1], cc[0] - CB.lo[0]};
+                    if (rf.count(key)) continue;
+                    PaReflux X;
+                    X.cbox = C.g2l[cg]; X.fbox = R.box; X.dir = d; X.side = side;
+                    for (int e = 0; e < 3; ++e) X.c[e] = cc[e] - CB.lo[e];
+                    X.f[d] = (lo_face ? B.lo[d] : B.hi[d]) - B.lo[d];
+                    X.f[t1] = 2 * coarsen(g[t1], 2) - B.lo[t1];
+                    X.f[t2] = 2 * coarsen(g[t2], 2) - B.lo[t2];
+                    rf.emplace(key, X);
+                }
+        }
+    }
+    T.reflux_begin.assign((size_t)nlev * 6 + 1, 0);
+    for (auto& kv : rf) {
+        T.reflux.push_back(kv.second);
+        ++T.reflux_begin[(size_t)kv.first[0] * 6 + 2 * kv.first[1] + kv.first[2] + 1];
+    }
+    for (size_t i = 1; i < T.reflux_begin.size(); ++i) T.reflux_begin[i] += T.reflux_begin[i - 1];
+    return done();
+}
+
 }  // namespace pa

@@ -157,6 +157,17 @@ struct FillPatchTable {
     std::vector<long long> send_ids, recv_ids;
 };
 
+// Tables of the composite implicit-diffusion solve (pa_smooth), built on its first call on a hierarchy.
+struct SmoothTables {
+    std::string err;                          // non-empty: the hierarchy is not supported (message says why)
+    std::vector<PaFaceRec> recs;              // faces.recs with the smoothing operator's coarse-fine polynomial order
+    std::vector<PaAvgDown> avg;               // level-major by COARSE level
+    std::vector<long long> avg_begin;         // nlev+1: first record of each coarse level
+    std::vector<long long> avg_cells;         // nlev: covered cells of each coarse level
+    std::vector<PaReflux> reflux;             // sorted by (coarse level, dir, side)
+    std::vector<long long> reflux_begin;      // nlev*6+1: first record of each (coarse level, 2*dir+side)
+};
+
 // BoxList::maxSize: every box replaced, in place, by its chunks no longer than max_grid_size (AMReX_BoxList.cpp:765-815)
 void box_max_size(int nboxes, const int* boxes, int max_grid_size, std::vector<Box>& out);
 
@@ -191,6 +202,8 @@ public:
     // FillPatchTwoLevels / FillPatchSingleLevel tables of level l for ng ghost layers; cgrow = coarse cells the
     // interpolater reads around the coarsened piece, with the exchange plan of the cross-rank sources.  Non-periodic only.
     const FillPatchTable& fill_patch(int l, int ng, int cgrow);
+    // covered-cell, reflux and coarse-fine coefficient tables of pa_smooth (lazily built, cached; one rank, ratio 2)
+    const SmoothTables& smooth_tables(int maxorder);
 
     void periodic_shifts(const Box& dom, int ng, std::vector<std::array<int, 3>>& out) const;
 
@@ -198,6 +211,7 @@ private:
     std::map<std::pair<int, int>, Layout> layouts_;
     std::map<std::pair<int, int>, HaloTable> halo_full_;
     std::map<std::array<int, 3>, FillPatchTable> fill_patch_;
+    std::map<int, SmoothTables> smooth_;
     void build_links();
     void build_halo(int l, int ng, bool cross, HaloTable& out, bool allow_remote);
     std::string build_faces();

@@ -720,3 +720,7 @@ cudaError_t launch_velnormal(const PaBoxDev* boxes, const PaLayDev* lay_u, const
 }
 
 }  // namespace pa
+
+// The kernels of the composite implicit-diffusion solve (pa_smooth) live in smooth.cu and are compiled in this translation
+// unit: they use the layout addressing above, and the library is built from a fixed list of translation units.
+#include "smooth.cu"

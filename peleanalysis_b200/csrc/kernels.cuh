@@ -182,6 +182,28 @@ cudaError_t launch_fp_clamp(const PaFpClamp* clamps, int nclamps, long long ncel
 cudaError_t launch_filter(int g, const PaBoxDev* boxes, const PaLayDev* lin, const PaLayDev* lout, int nboxes, const long long* work_prefix,
                           long long nwork_per_comp, const double* in, long long cs_in, double* out, long long cs_out, int ncomp,
                           const double* w3_dev, cudaStream_t st);
+// ---- composite implicit-diffusion solve (smooth.cu) --------------------------------------------------------------------
+// out = in - beta * Laplacian(in) on the valid cells of one level (`in` ghost-filled, one ghost layer)
+cudaError_t launch_sm_apply(const PaBoxDev* boxes, const PaLayDev* lay, const long long* host_off, int nboxes, long long ncells,
+                            const double* in, double* out, double beta, const double dxi[3], cudaStream_t st);
+// coarse-fine faces of one (coarse level, dir, side) group: cout += the flux difference (average fine flux - coarse flux)
+cudaError_t launch_sm_reflux(const PaReflux* recs, long long nrec, const PaLayDev* clay, const PaLayDev* flay, const double* cin,
+                             const double* fin, double* cout, double beta, double dxic, double dxif, cudaStream_t st);
+// covered cells of one coarse level <- average of their fine cells (or 0 when zero)
+cudaError_t launch_sm_avgdown(const PaAvgDown* recs, int nrec, long long ncells, const PaBoxDev* cboxes, const PaLayDev* clay,
+                              const PaBoxDev* fboxes, const PaLayDev* flay, double* crse, const double* fine, bool zero, cudaStream_t st);
+// out = a*x + b*y + c*z elementwise over n doubles (y, z may be null)
+cudaError_t launch_sm_lin3(long long n, double a, const double* x, double b, const double* y, double c, const double* z, double* out,
+                           cudaStream_t st);
+// partials of sum x*y (mode 0) or max |x| (mode 1) over the valid cells of one level -> partial[0 .. *nblocks)
+cudaError_t launch_sm_reduce(const PaBoxDev* boxes, const PaLayDev* lay, const long long* host_off, int nboxes, long long ncells,
+                             const double* x, const double* y, int mode, double* partial, int* nblocks, cudaStream_t st);
+cudaError_t launch_sm_final(const double* partial, int n, int mode, double* out, cudaStream_t st);
+int smooth_max_partials();            // most partials one launch_sm_reduce writes
+// valid cells of one level, layout -> layout
+cudaError_t launch_sm_copy(const PaBoxDev* boxes, const PaLayDev* lay_in, const PaLayDev* lay_out, const long long* host_off, int nboxes,
+                           long long ncells, const double* in, double* out, cudaStream_t st);
+
 // microbenchmark: blocks x threads threads each doing iters x 8 (multiply, add) pairs; out has blocks * threads doubles
 cudaError_t launch_fp64_rate(double* out, int blocks, int threads, int iters, cudaStream_t st);
 

@@ -153,6 +153,24 @@ struct PaFpClamp {
     long long start;    // prefix over the cells of the grown boxes in this list
 };
 
+// ---- composite implicit-diffusion solve (pa_smooth, smooth.cu) ----------------------------------------------------------
+// coarse cells [lo, lo+n) (coarse index space) of local coarse box cbox are covered by local fine box fbox: they hold the
+// average of their 8 fine cells (average_down)
+struct PaAvgDown {
+    int cbox, fbox;
+    int lo[3], n[3];
+    long long start;    // prefix over the cells of all records of the coarse level (the kernel's enumeration)
+};
+// one coarse-fine face seen from the coarse side: the face `side` (0 low, 1 high) along `dir` of the uncovered coarse cell c
+// (box-relative in local coarse box cbox) borders the fine region; its flux is replaced by the average of the 4 fine face
+// fluxes between the fine cells f + (0 | 1 along the two tangential directions) (box-relative in local fine box fbox, the
+// first fine cells inside the fine region) and their coarse-fine ghost cells
+struct PaReflux {
+    int cbox, fbox;
+    int c[3], f[3];
+    int dir, side;
+};
+
 // face flags (uint16 per face-plane cell)
 #define PA_FLAG_MASK(f)   ((f) & 3)
 #define PA_FLAG_NC(f, b)  (((f) >> (2 + (b))) & 1)   // b: 0 (-r,0) 1 (+r,0) 2 (0,-r) 3 (0,+r) 4 (-,-) 5 (+,-) 6 (-,+) 7 (+,+)

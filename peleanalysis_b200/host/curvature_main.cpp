@@ -1,8 +1,9 @@
 // curvature3d.b200.ex -- drop-in for PeleAnalysis' curvature tool (R/Src/curvature.cpp): same ParmParse keys, plotfile
 // in/out and output names; progress variable, flame normal, mean curvature and the optional Gaussian curvature /
-// strain rate / normal velocity branches run through the C ABI.  do_smooth is the one key not served (it needs a
-// multigrid solve): the shell aborts if it is set.  Extension: ngpus=N runs on N GPUs from this one process, one host thread
-// per GPU (multi_gpu.hpp); transport=peer|slab picks peer links + packed slabs (default) or packed slabs only.
+// strain rate / normal velocity branches run through the C ABI.  do_smooth=1 (curvature.cpp:328-406) solves the implicit
+// diffusion step with pa_smooth and runs the curvature on the smoothed field (one GPU only).  Extension: ngpus=N runs on N GPUs
+// from this one process, one host thread per GPU (multi_gpu.hpp); transport=peer|slab picks peer links + packed slabs (default)
+// or packed slabs only.
 #include <algorithm>
 
 #include "multi_gpu.hpp"
@@ -35,7 +36,6 @@ int main(int argc, char** argv) {
     int nAux = pp.countval("Aux_Variables");
     std::vector<std::string> aux(nAux);
     for (int i = 0; i < nAux; ++i) pp.get("Aux_Variables", aux[i], i);
-    if (do_smooth) pa_abort("do_smooth=1 needs the MLMG solve of the reference build; not available in the B200 path");
 
     std::cout << "infile = " << plotFileName << "\n" << "reading plt file = " << plotFileName << "\n";
     pltio::Header H;
@@ -107,7 +107,8 @@ int main(int argc, char** argv) {
     if (do_velnormal) names[idVelNormal] = "VelFlameNormal";
     // SmoothedProgress (do_smooth off) and GaussianCurvature (do_gaussCurv off) are never written by the reference
     // (uninitialised memory there); they are written as zeros here.
-    std::vector<int> zero_slots{idSmProg};
+    std::vector<int> zero_slots;
+    if (!do_smooth) zero_slots.push_back(idSmProg);
     if (!do_gaussCurv) zero_slots.push_back(idKg);
     if (getStrainTensor && !do_strain) for (int i = 0; i < 9; ++i) zero_slots.push_back(idROST + i);
 
@@ -116,6 +117,8 @@ int main(int argc, char** argv) {
     std::string transport = "peer";
     pp.query("transport", transport);
     if (transport != "peer" && transport != "slab") pa_abort("transport must be peer or slab (got " + transport + ")");
+    if (ngpus > 1 && do_smooth)
+        pa_abort("do_smooth=1 runs on one GPU only: the smoothing solve has no multi-GPU path (use ngpus=1)");
     if (ngpus > 1) {
         CurvJob J;
         J.peer = transport == "peer";
@@ -135,7 +138,9 @@ int main(int argc, char** argv) {
     pa_hier* h = nullptr;
     check(pa_hier_create(&h, Nlev, hi.lv.data(), is_per.data(), bck, 0, 1), "pa_hier_create");
     pa_field *st = nullptr, *res = nullptr;
-    check(pa_field_alloc(h, need_vel ? 4 : 1, 1, &st), "pa_field_alloc");
+    // do_smooth: two more state components, c and the smoothed phi, which the curvature then reads as its scalar
+    const int nst = need_vel ? 4 : 1, comp_c = nst, comp_phi = nst + 1;
+    check(pa_field_alloc(h, do_smooth ? nst + 2 : nst, 1, &st), "pa_field_alloc");
     check(pa_field_alloc(h, nres, 1, &res), "pa_field_alloc");
 
     std::vector<PinnedLevel> buf(Nlev);
@@ -153,7 +158,23 @@ int main(int argc, char** argv) {
             }
         }
     }
-    check(pa_curvature(st, 0, 1, &o, res, 0), "pa_curvature");
+    if (do_smooth) {
+        pa_smooth_opts so{};
+        so.smoothing_time = smooth_time;
+        int iters = 0;
+        double resid = 0.0;
+        check(pa_smooth(st, 0, progMin, progMax, &so, st, comp_c, comp_phi, &iters, &resid), "pa_smooth");
+        if (verbose) std::cout << "do_smooth: smoothing_time = " << smooth_time << ", " << iters << " iterations, max|c - A phi| / max|c| = "
+                               << resid << "\n";
+        // the curvature of phi with the identity normalisation (curvature.cpp:328-406 hands the solution on as the progress
+        // variable); its Progress output is phi itself and goes to SmoothedProgress, Progress is c
+        pa_curv_opts os = o;
+        os.prog_min = 0.0; os.prog_max = 1.0;
+        slot[0] = idSmProg;
+        check(pa_curvature(st, comp_phi, 1, &os, res, 0), "pa_curvature");
+    } else {
+        check(pa_curvature(st, 0, 1, &o, res, 0), "pa_curvature");
+    }
     {
         long long mx = 0;
         for (int l = 0; l < Nlev; ++l) mx = std::max(mx, buf[l].ncells);
@@ -161,6 +182,7 @@ int main(int argc, char** argv) {
         for (int l = 0; l < Nlev; ++l) {
             for (int z : zero_slots) std::fill(buf[l].comp(z), buf[l].comp(z) + buf[l].ncells, 0.0);
             for (int c = 0; c < nres; ++c) dl.download(res, l, c, buf[l].comp(slot[c]), buf[l].ncells);
+            if (do_smooth) dl.download(st, l, comp_c, buf[l].comp(idProg), buf[l].ncells);
         }
         dl.flush();
     }

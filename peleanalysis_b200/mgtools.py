@@ -175,6 +175,7 @@ def run(tool: str, argv: Sequence[str], capi=None, multigpu=None, wrap=None, bac
     H = capi.Hierarchy(levels, is_per, sym_dir, D.rank, D.world, flags=flags)
     kw = {} if wrap is None else {"wrap": wrap}
 
+    do_smooth = False
     if tool == "grad":
         gvars = pp.get("gradVars") or [_get(pp, "gradVar", "temp")]
         dev_in = [comp(v) for v in gvars]
@@ -191,8 +192,11 @@ def run(tool: str, argv: Sequence[str], capi=None, multigpu=None, wrap=None, bac
         o.threshold = _get(pp, "threshold_value", 1.0e-4, float)
         o.do_gauss, o.do_strain = _get(pp, "do_gaussCurv", 0, int), _get(pp, "do_strain", 0, int)
         o.get_strain_tensor, o.do_velnormal = _get(pp, "getStrainTensor", 0, int), _get(pp, "do_velnormal", 0, int)
-        if _get(pp, "do_smooth", 0, int):
-            raise SystemExit("amrex::Abort::0::do_smooth=1 needs the MLMG solve of the reference build; not available in the B200 path !!!")
+        do_smooth = bool(_get(pp, "do_smooth", 0, int))
+        if do_smooth and D.world > 1:
+            raise SystemExit("amrex::Abort::0::do_smooth=1 runs on one GPU only: the smoothing solve has no multi-GPU path (run at world size 1) !!!")
+        so = capi.SmoothOpts()
+        so.smoothing_time = _get(pp, "smoothing_time", 1.0e-7, float)
         if _get(pp, "useFileMinMax", 1, int):
             o.prog_min, o.prog_max = plotfile.file_min_max(infile, prog, nlev)
         else:
@@ -213,7 +217,7 @@ def run(tool: str, argv: Sequence[str], capi=None, multigpu=None, wrap=None, bac
         if o.do_velnormal:
             out_names.append("VelFlameNormal")
         outfile = _get(pp, "outfile", file_root(infile) + "_K")
-        fin = capi.Field(H, len(dev_in), 1)
+        fin = capi.Field(H, len(dev_in) + (2 if do_smooth else 0), 1)     # do_smooth: + c and phi
         nres = capi.curvature_num_outputs(o)
         fout = capi.Field(H, nres, 1)
 
@@ -244,6 +248,14 @@ def run(tool: str, argv: Sequence[str], capi=None, multigpu=None, wrap=None, bac
         op = multigpu.Curvature(fin, 0, o, fout, 0, comp_vel=1, **kw)
         D.barrier()
         op.run()
+    elif do_smooth:                                            # curvature.cpp:328-406: curvature of phi, identity normalisation
+        cc, cphi = len(dev_in), len(dev_in) + 1
+        iters, resid = capi.smooth(fin, 0, o.prog_min, o.prog_max, so, fin, cc, cphi)
+        if _get(pp, "verbose", 0, int):
+            print("do_smooth: smoothing_time = %g, %d iterations, max|c - A phi| / max|c| = %g" % (so.smoothing_time, iters, resid))
+        o_phi = capi.CurvOpts.from_buffer_copy(o)
+        o_phi.prog_min, o_phi.prog_max = 0.0, 1.0
+        capi.curvature(fin, cphi, 1, o_phi, fout, 0)
     else:
         capi.curvature(fin, 0, 1, o, fout, 0)
     capi.sync()
@@ -268,6 +280,8 @@ def run(tool: str, argv: Sequence[str], capi=None, multigpu=None, wrap=None, bac
                         nxt += 1
         if o.do_velnormal:
             res_index["VelFlameNormal"] = nxt
+        if do_smooth:                                         # the curvature's Progress is phi; the file's Progress is c (in fin)
+            res_index["SmoothedProgress"] = res_index.pop("Progress")
     else:
         res_index = {n: k for k, n in enumerate(out_names[len(keep):])}
 
@@ -291,6 +305,10 @@ def run(tool: str, argv: Sequence[str], capi=None, multigpu=None, wrap=None, bac
         for k, n in enumerate(out_names[len(keep):]):
             if n in res_index:
                 fout.download_level(l, res_index[n], buf)
+                capi.sync()
+                res[len(keep) + k] = buf
+            elif do_smooth and n == "Progress":
+                fin.download_level(l, len(dev_in), buf)
                 capi.sync()
                 res[len(keep) + k] = buf
         fn = "Cell_D_%05d" % D.rank

@@ -71,16 +71,31 @@ class GradRun(_Run):
 
 class CurvatureRun(_Run):
     """curvature.cpp on the progress variable `progress` (and the velocities, when the options need them): state field
-    [S, (u, v, w)] with one ghost layer, output in the library's order (Progress, K, n, [Kg], [SR], [ROST], [VN])."""
+    [S, (u, v, w)] with one ghost layer, output in the library's order (Progress, K, n, [Kg], [SR], [ROST], [VN]).
+
+    do_smooth (one rank only, curvature.cpp:328-406): the progress variable c is first smoothed by one implicit diffusion
+    step of `smoothing_time` (capi.smooth) and the curvature runs on the smoothed phi with prog_min = 0, prog_max = 1.
+    Progress stays c; smoothed_progress() returns phi; `iterations` / `residual` report the last solve."""
 
     VEL = ("x_velocity", "y_velocity", "z_velocity")
 
     def __init__(self, P, pf: Plotfile, opts, progress: str = "temp", is_per=(1, 1, 1), sym_dir=(0, 0, 0), upload: bool = True,
-                 rank: int = 0, nranks: int = 1, multigpu=None, wrap=None):
+                 rank: int = 0, nranks: int = 1, multigpu=None, wrap=None, do_smooth: bool = False, smoothing_time: float = 1.0e-7):
+        if do_smooth and nranks > 1:
+            raise ValueError("do_smooth runs on one rank only: the smoothing solve has no multi-rank path")
         super().__init__(P, pf, is_per, sym_dir, rank, nranks, multigpu, wrap)
         self.opts = opts
         self.names = [progress] + (list(self.VEL) if (opts.do_strain or opts.do_velnormal) else [])
-        self.state = P.Field(self.hier, len(self.names), 1)
+        self.do_smooth = bool(do_smooth)
+        self.iterations, self.residual = 0, 0.0
+        nst = len(self.names)
+        self.comp_c, self.comp_phi = nst, nst + 1
+        if self.do_smooth:
+            self.sopts = P.SmoothOpts()
+            self.sopts.smoothing_time = smoothing_time
+            self.opts_phi = P.CurvOpts.from_buffer_copy(opts)
+            self.opts_phi.prog_min, self.opts_phi.prog_max = 0.0, 1.0
+        self.state = P.Field(self.hier, nst + 2 if self.do_smooth else nst, 1)
         self.nout = P.curvature_num_outputs(opts)
         self.fout = P.Field(self.hier, self.nout, 1)
         comp_vel = 1 if len(self.names) > 1 else 0
@@ -90,10 +105,28 @@ class CurvatureRun(_Run):
 
     def step(self) -> None:
         """every step of the tool with the exchange each one needs in front of it, asynchronous on the library stream"""
+        comp_vel = 1 if len(self.names) > 1 else 0
         if self.op is not None:
             self.op.run()
+        elif self.do_smooth:
+            self.iterations, self.residual = self.P.smooth(self.state, 0, self.opts.prog_min, self.opts.prog_max, self.sopts,
+                                                           self.state, self.comp_c, self.comp_phi)
+            self.P.curvature(self.state, self.comp_phi, comp_vel, self.opts_phi, self.fout, 0)
         else:
-            self.P.curvature(self.state, 0, 1 if len(self.names) > 1 else 0, self.opts, self.fout, 0)
+            self.P.curvature(self.state, 0, comp_vel, self.opts, self.fout, 0)
 
     def result(self):
-        return self._result(self.fout, self.nout)
+        res = self._result(self.fout, self.nout)
+        if self.do_smooth:                       # the curvature's Progress is phi; the tool's Progress is c
+            c = self.state.download_fabs(self.comp_c)
+            for l, lv in enumerate(res):
+                for b, a in enumerate(lv):
+                    if a is not None:
+                        a[0] = c[l][b]
+        return res
+
+    def smoothed_progress(self):
+        """per level, per box: phi [nz][ny][nx] (do_smooth only)"""
+        if not self.do_smooth:
+            raise ValueError("smoothed_progress() needs do_smooth=True")
+        return self.fout.download_fabs(0)
