@@ -68,8 +68,13 @@ typedef struct {
     double smoothing_time;            /* smoothing_time: beta of phi - beta * div(grad phi) = c (>= 0) */
     double tol_rel;                   /* stop when max|c - A phi| <= tol_rel * max|c| over uncovered cells; 0 = 1e-10 */
     int max_iter;                     /* iterations before PA_ERR_NOCONV; 0 = 1000 */
-    int reserved[8];
+    int precond;                      /* preconditioner of the solve: PA_SMOOTH_PRECOND_* (0 = Jacobi) */
+    int reserved[7];
 } pa_smooth_opts;
+enum {
+    PA_SMOOTH_PRECOND_JACOBI = 0,     /* per-level inverse diagonal */
+    PA_SMOOTH_PRECOND_MG = 1          /* one multigrid V-cycle (red-black Gauss-Seidel, composite restriction; see pa_smooth) */
+};
 
 /* ---- runtime ------------------------------------------------------------------------------------- */
 /* Select the CUDA device of this process (one process per GPU).  amrex::Initialize's device part. */
@@ -218,6 +223,12 @@ int pa_curvature_scratch(pa_hier *h, int which, pa_field **f);
  * out[comp_phi]; the curvature of the smoothed field is then pa_curvature on phi with prog_min = 0, prog_max = 1.
  * Solver: right-preconditioned BiCGStab on the composite residual, deterministic (fixed reduction order); the stop test is on
  * the TRUE residual.  *iters = iterations, *resid = max|c - A phi| / max|c| over uncovered cells (both may be NULL).
+ * Preconditioner (o->precond): PA_SMOOTH_PRECOND_JACOBI, the inverse diagonal of each level's operator, whose iteration count
+ * grows with smoothing_time / dx_finest^2; or PA_SMOOTH_PRECOND_MG, one V-cycle per application: red-black Gauss-Seidel on the
+ * AMR levels from the finest down, the composite residual restricted level by level, a geometric V-cycle over level 0's own
+ * coarsenings by 2 (as far as every box of level 0 coarsens), then back up with piecewise-constant prolongation.  The
+ * V-cycle is a fixed linear map (fixed sweep counts), so runs stay bit-identical; the discrete system, the stop test, the
+ * restarts and every error code are the same in both modes.  Another precond value: PA_ERR_ARG.
  * smoothing_time = 0 copies c into phi bit for bit.  One rank and refinement ratio 2 only (PA_ERR_UNSUPPORTED otherwise);
  * negative smoothing_time: PA_ERR_ARG; not converged within max_iter: PA_ERR_NOCONV, phi not written. */
 int pa_smooth(pa_field *state, int comp_S, double prog_min, double prog_max, const pa_smooth_opts *o, pa_field *out, int comp_c,
@@ -331,6 +342,13 @@ int pa_debug_normal_math(void);
 /* Measured FP64 rate of the device for separate multiplies and adds (no FMA: the instruction mix bit parity with the
  * reference's CPU build imposes on pa_filter), in Gop/s: the roofline denominator of the filter for ghost widths >= 2. */
 int pa_debug_fp64_rate(double *gops);
+/* The multigrid preconditioner of pa_smooth on its own: with pa_smooth's inputs (o->smoothing_time > 0; o->precond, tol_rel
+ * and max_iter are not used), runs ncycles steps of phi <- phi + B (c - A phi) from phi = c, B one V-cycle, and writes
+ * max|c - A phi| / max|c| into resid[0 .. ncycles]: resid[0] before the first step, resid[n] after step n.  c goes into
+ * out[comp_c], the last phi into out[comp_phi].
+ * *nmg = the number of multigrid levels of level 0, level 0 itself included (1: level 0 does not coarsen). */
+int pa_debug_smooth_vcycle(pa_field *state, int comp_S, double prog_min, double prog_max, const pa_smooth_opts *o, pa_field *out,
+                           int comp_c, int comp_phi, int ncycles, double *resid, int *nmg);
 /* 1 if curvature on this hierarchy runs through the fused kernel (every local box eligible: >= 3 cells in every direction,
  * <= 128 wide), 0 if it takes the separate flame-normal / divergence kernels, < 0 on error. */
 int pa_debug_curv_fused(pa_hier *h);

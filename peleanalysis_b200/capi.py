@@ -33,11 +33,14 @@ class CurvOpts(C.Structure):
 
 
 class SmoothOpts(C.Structure):
-    """pa_smooth_opts: smoothing_time (>= 0), tol_rel (0 = 1e-10), max_iter (0 = 1000)."""
-    _fields_ = [("smoothing_time", C.c_double), ("tol_rel", C.c_double), ("max_iter", C.c_int), ("reserved", C.c_int * 8)]
+    """pa_smooth_opts: smoothing_time (>= 0), tol_rel (0 = 1e-10), max_iter (0 = 1000), precond (PA_SMOOTH_PRECOND_*, 0 = Jacobi)."""
+    _fields_ = [("smoothing_time", C.c_double), ("tol_rel", C.c_double), ("max_iter", C.c_int), ("precond", C.c_int),
+                ("reserved", C.c_int * 7)]
 
 
 PA_ERR_UNSUPPORTED, PA_ERR_NOCONV = -4, -6
+PA_SMOOTH_PRECOND_JACOBI, PA_SMOOTH_PRECOND_MG = 0, 1
+SMOOTH_PRECONDS = {"jacobi": PA_SMOOTH_PRECOND_JACOBI, "mg": PA_SMOOTH_PRECOND_MG}
 
 
 # every symbol include/pele_stencil_b200.h declares: (restype, argtypes)
@@ -93,6 +96,7 @@ SYMBOLS = {
     "pa_debug_fill_patch_exchange_ids": (_i64, [_vp, _i, _i, _i, _i, _vp, _i64]),
     "pa_filter": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _i]),
     "pa_smooth": (_i, [_vp, _i, _d, _d, C.POINTER(SmoothOpts), _vp, _i, _i, C.POINTER(_i), C.POINTER(_d)]),
+    "pa_debug_smooth_vcycle": (_i, [_vp, _i, _d, _d, C.POINTER(SmoothOpts), _vp, _i, _i, _i, C.POINTER(_d), C.POINTER(_i)]),
 }
 
 _lib = None
@@ -506,6 +510,24 @@ def smooth(state: Field, comp_S: int, prog_min: float, prog_max: float, opts: Sm
     it, res = C.c_int(0), C.c_double(0.0)
     check(lib().pa_smooth(state.f, comp_S, prog_min, prog_max, C.byref(opts), out.f, comp_c, comp_phi, C.byref(it), C.byref(res)))
     return it.value, res.value
+
+
+def smooth_precond(name: str) -> int:
+    """PA_SMOOTH_PRECOND_* of a preconditioner name ("jacobi" or "mg"); ValueError for any other name"""
+    if name not in SMOOTH_PRECONDS:
+        raise ValueError("smooth_precond must be one of %s (got %r)" % ("|".join(SMOOTH_PRECONDS), name))
+    return SMOOTH_PRECONDS[name]
+
+
+def debug_smooth_vcycle(state: Field, comp_S: int, prog_min: float, prog_max: float, opts: SmoothOpts, out: Field, comp_c: int,
+                        comp_phi: int, ncycles: int):
+    """pa_debug_smooth_vcycle: ncycles steps of phi <- phi + B (c - A phi) from phi = c, B one V-cycle of pa_smooth's multigrid
+    preconditioner.  Returns (relative residuals: [0] before the first step, [n] after step n; number of MG levels of level 0)."""
+    res = np.zeros(max(ncycles, 0) + 1, dtype=np.float64)
+    nmg = C.c_int(0)
+    check(lib().pa_debug_smooth_vcycle(state.f, comp_S, prog_min, prog_max, C.byref(opts), out.f, comp_c, comp_phi, ncycles,
+                                       res.ctypes.data_as(C.POINTER(C.c_double)), C.byref(nmg)))
+    return res, nmg.value
 
 
 def curvature_num_outputs(opts: CurvOpts) -> int:

@@ -84,6 +84,15 @@ struct SmoothDev {
     DevBuf<PaReflux> reflux;
     DevBuf<double> partial, scal;                      // reduction partials and the reduced scalar
     pa_field* w[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    // multigrid preconditioner (built on the first PA_SMOOTH_PRECOND_MG call): the V-cycle's right-hand side and residual on
+    // the hierarchy, and the coarsenings of level 0 (MG levels 1, 2, ...) as single-level one-rank hierarchies with their
+    // correction, right-hand side and residual fields
+    pa_field* mg_rhs = nullptr;
+    pa_field* mg_res = nullptr;
+    std::vector<pa_hier*> mg_h;
+    std::vector<std::array<pa_field*, 3>> mg_f;
+    DevBuf<PaAvgDown> mg_avg;
+    bool mg_ready = false;
 };
 
 }  // namespace
@@ -655,6 +664,18 @@ int join_side(pa_hier* h) {
     return PA_OK;
 }
 
+// the multigrid preconditioner's fields and level-0 coarsenings (fields before the hierarchies they live on)
+void free_smooth_mg(SmoothDev& S) {
+    for (auto& f : S.mg_f) for (pa_field* g : f) if (g) pa_field_free(g);
+    for (pa_hier* m : S.mg_h) pa_hier_destroy(m);
+    if (S.mg_rhs) pa_field_free(S.mg_rhs);
+    if (S.mg_res) pa_field_free(S.mg_res);
+    S.mg_f.clear();
+    S.mg_h.clear();
+    S.mg_rhs = S.mg_res = nullptr;
+    S.mg_ready = false;
+}
+
 }  // namespace
 
 // =============================================================================================================
@@ -714,7 +735,10 @@ int pa_hier_destroy(pa_hier* h) {
     if (h->tmpG) pa_field_free(h->tmpG);
     if (h->tmpH) pa_field_free(h->tmpH);
     if (h->tmpW) pa_field_free(h->tmpW);
-    if (h->sm) for (pa_field* f : h->sm->w) if (f) pa_field_free(f);
+    if (h->sm) {
+        for (pa_field* f : h->sm->w) if (f) pa_field_free(f);
+        free_smooth_mg(*h->sm);
+    }
     if (h->ev_fork) cudaEventDestroy(h->ev_fork);
     if (h->ev_join) cudaEventDestroy(h->ev_join);
     if (h->side) cudaStreamDestroy(h->side);
@@ -1528,6 +1552,21 @@ namespace {
 constexpr int SMOOTH_MAXORDER = 3;
 constexpr double SMOOTH_TOL_REL = 1e-10;
 constexpr int SMOOTH_MAX_ITER = 1000;
+// The multigrid preconditioner's V-cycle: red-black Gauss-Seidel sweeps before (NU1) and after (NU2) the coarse correction on
+// every level, and a fixed number of sweeps on the coarsest coarsening of level 0 in place of a coarse solve.  Fixed counts and
+// no tolerance: the V-cycle is the same linear map on every call, as right-preconditioned BiCGStab needs.
+constexpr int SMOOTH_MG_NU1 = 2;
+constexpr int SMOOTH_MG_NU2 = 2;
+constexpr int SMOOTH_MG_BOTTOM_SWEEPS = 16;
+
+// one level the V-cycle smooths: an AMR level of the hierarchy, or a coarsening of level 0 (level 0 of its own hierarchy)
+struct SmLev {
+    pa_hier* h;
+    int l;
+    const PaFaceRec* recs;              // face records of the ghost fill (nullptr: the hierarchy's own)
+    const PaLayDev* lay;                // nghost-1 layout
+    pa_field *e, *rhs, *res;            // correction, right-hand side, residual
+};
 
 struct SmCtx {
     pa_hier* h;
@@ -1536,6 +1575,9 @@ struct SmCtx {
     double beta;
     int nlev;
     std::vector<const PaLayDev*> lay;   // nghost-1 layout per level (every work field)
+    bool mg = false;                    // preconditioner: the V-cycle (else Jacobi)
+    std::vector<SmLev> amr;             // per AMR level (mg only; e is the V-cycle's output field)
+    std::vector<SmLev> coarse;          // MG levels 1, 2, ... of level 0 (mg only)
 };
 
 // y = A x on every valid cell: covered cells of x <- fine averages, ghost fill, 7-point operator, reflux; y's covered cells <- 0
@@ -1588,6 +1630,100 @@ int sm_reduce(SmCtx& c, pa_field* x, pa_field* y, int mode, double* out) {
     return PA_OK;
 }
 
+// ---- the multigrid preconditioner -----------------------------------------------------------------------------------------
+int sm_fill(const SmLev& v) { return fill_ghosts_impl(v.e, 0, 1, v.l, v.l, true, GhostXform{0, 0.0, 1.0}, v.recs); }
+
+// n red-black Gauss-Seidel sweeps of A_l e = rhs on one level; the ghost cells are refilled before each colour
+int sm_gsrb(const SmLev& v, double beta, int n) {
+    const LevelDev& D = *v.h->lev[v.l];
+    const Level& V = v.h->H.lev[v.l];
+    const double* q = V.dxinv;
+    const double diag = 1.0 + 2.0 * beta * (q[0] * q[0] + q[1] * q[1] + q[2] * q[2]);
+    for (int s = 0; s < n; ++s)
+        for (int colour = 0; colour < 2; ++colour) {
+            CHK(sm_fill(v));
+            CU(launch_sm_gsrb(D.boxes.p, v.lay, D.host_off.p, (int)V.local.size(), D.host_off_h.back(), v.rhs->slab[v.l], v.e->slab[v.l],
+                              beta, q, diag, colour, t_stream));
+        }
+    return PA_OK;
+}
+
+// res = rhs - A_l e on one level (ghost cells refilled first)
+int sm_resid(const SmLev& v, double beta) {
+    const LevelDev& D = *v.h->lev[v.l];
+    const Level& V = v.h->H.lev[v.l];
+    CHK(sm_fill(v));
+    CU(launch_sm_resid(D.boxes.p, v.lay, D.host_off.p, (int)V.local.size(), D.host_off_h.back(), v.rhs->slab[v.l], v.e->slab[v.l],
+                       v.res->slab[v.l], beta, V.dxinv, t_stream));
+    return PA_OK;
+}
+
+int sm_zero(pa_field* f, int l) {
+    if (f->cs[l] > 0) CU(cudaMemsetAsync(f->slab[l], 0, (size_t)f->cs[l] * sizeof(double), t_stream));
+    return PA_OK;
+}
+
+// z = B r, one V-cycle from a zero initial guess (DESIGN.md section 10):
+//  1. AMR levels L .. 1: NU1 sweeps, the residual, restricted into level l-1 -- the 8-cell average on covered cells, and on the
+//     uncovered coarse cells of coarse-fine faces minus the fine-flux term of the composite operator (the reflux of z_l
+//     against a zero z_{l-1}, i.e. with beta negated);
+//  2. level 0: a geometric V-cycle over its coarsenings (8-cell average down, piecewise-constant up, NU1 / NU2 sweeps, the
+//     coarsest level SMOOTH_MG_BOTTOM_SWEEPS sweeps);
+//  3. AMR levels 1 .. L: z_l += the piecewise-constant prolongation of z_{l-1}, NU2 sweeps with ghost cells from z_{l-1};
+//  4. covered cells of z <- 0 (the Krylov vectors are zero there).
+int sm_vcycle(SmCtx& c, pa_field* r, pa_field* z) {
+    pa_hier* h = c.h;
+    const Hier& H = h->H;
+    const SmoothTables& T = *c.T;
+    SmoothDev& S = *c.S;
+    const int L = c.nlev - 1;
+    for (int l = 0; l <= L; ++l) {
+        c.amr[l].e = z;
+        CHK(sm_zero(z, l));
+        CU(launch_sm_lin3(r->cs[l], 1.0, r->slab[l], 0.0, nullptr, 0.0, nullptr, S.mg_rhs->slab[l], t_stream));
+    }
+    for (int l = L; l >= 1; --l) {
+        const SmLev& v = c.amr[l];
+        CHK(sm_gsrb(v, c.beta, SMOOTH_MG_NU1));
+        CHK(sm_resid(v, c.beta));
+        CU(launch_sm_avgdown(S.avg.p + T.avg_begin[l - 1], (int)(T.avg_begin[l] - T.avg_begin[l - 1]), T.avg_cells[l - 1],
+                             h->lev[l - 1]->boxes.p, c.lay[l - 1], h->lev[l]->boxes.p, c.lay[l], S.mg_rhs->slab[l - 1], S.mg_res->slab[l],
+                             false, t_stream));
+        for (int g = 0; g < 6; ++g) {
+            const long long a = T.reflux_begin[(size_t)(l - 1) * 6 + g], b = T.reflux_begin[(size_t)(l - 1) * 6 + g + 1];
+            const int d = g / 2;
+            CU(launch_sm_reflux(S.reflux.p + a, b - a, c.lay[l - 1], c.lay[l], z->slab[l - 1], z->slab[l], S.mg_rhs->slab[l - 1], -c.beta,
+                                H.lev[l - 1].dxinv[d], H.lev[l].dxinv[d], t_stream));
+        }
+    }
+    const int K = 1 + (int)c.coarse.size();
+    auto mg = [&](int k) -> const SmLev& { return k == 0 ? c.amr[0] : c.coarse[k - 1]; };
+    for (int k = 0; k + 1 < K; ++k) {
+        const SmLev &f = mg(k), &q = mg(k + 1);
+        CHK(sm_gsrb(f, c.beta, SMOOTH_MG_NU1));
+        CHK(sm_resid(f, c.beta));
+        CHK(sm_zero(q.e, 0));
+        CU(launch_sm_avgdown(S.mg_avg.p + T.mg_avg_begin[k], (int)(T.mg_avg_begin[k + 1] - T.mg_avg_begin[k]), T.mg_avg_cells[k],
+                             q.h->lev[0]->boxes.p, q.lay, f.h->lev[f.l]->boxes.p, f.lay, q.rhs->slab[0], f.res->slab[f.l], false, t_stream));
+    }
+    CHK(sm_gsrb(mg(K - 1), c.beta, SMOOTH_MG_BOTTOM_SWEEPS));
+    for (int k = K - 2; k >= 0; --k) {
+        const SmLev &f = mg(k), &q = mg(k + 1);
+        CU(launch_sm_prolong(S.mg_avg.p + T.mg_avg_begin[k], (int)(T.mg_avg_begin[k + 1] - T.mg_avg_begin[k]), T.mg_avg_cells[k],
+                             q.h->lev[0]->boxes.p, q.lay, f.h->lev[f.l]->boxes.p, f.lay, q.e->slab[0], f.e->slab[f.l], t_stream));
+        CHK(sm_gsrb(f, c.beta, SMOOTH_MG_NU2));
+    }
+    for (int l = 1; l <= L; ++l) {
+        CU(launch_sm_prolong(S.avg.p + T.avg_begin[l - 1], (int)(T.avg_begin[l] - T.avg_begin[l - 1]), T.avg_cells[l - 1],
+                             h->lev[l - 1]->boxes.p, c.lay[l - 1], h->lev[l]->boxes.p, c.lay[l], z->slab[l - 1], z->slab[l], t_stream));
+        CHK(sm_gsrb(c.amr[l], c.beta, SMOOTH_MG_NU2));
+    }
+    for (int l = 0; l < L; ++l)
+        CU(launch_sm_avgdown(S.avg.p + T.avg_begin[l], (int)(T.avg_begin[l + 1] - T.avg_begin[l]), T.avg_cells[l], h->lev[l]->boxes.p,
+                             c.lay[l], h->lev[l + 1]->boxes.p, c.lay[l + 1], z->slab[l], nullptr, true, t_stream));
+    return PA_OK;
+}
+
 int ensure_smooth(pa_hier* h, const SmoothTables& T) {
     if (h->sm) return PA_OK;
     auto S = std::make_unique<SmoothDev>();
@@ -1605,13 +1741,46 @@ int ensure_smooth(pa_hier* h, const SmoothTables& T) {
     return PA_OK;
 }
 
-}  // namespace
-extern "C" {
+// the multigrid preconditioner's work fields and level-0 coarsenings: one single-level, one-rank hierarchy per coarsening
+// (boxes and domain of T.mg_boxes / T.mg_dom, dx * 2^k, the hierarchy's periodicity and wall kinds), which brings its layouts,
+// halo and wall tables and ghost fill
+int ensure_smooth_mg(pa_hier* h, const SmoothTables& T) {
+    SmoothDev& S = *h->sm;
+    if (S.mg_ready) return PA_OK;
+    free_smooth_mg(S);                  // what an earlier, failed attempt left
+    const Hier& H = h->H;
+    CHK(pa_field_alloc(h, 1, 1, &S.mg_rhs));
+    CHK(pa_field_alloc(h, 1, 1, &S.mg_res));
+    for (size_t k = 1; k < T.mg_boxes.size(); ++k) {
+        const std::vector<Box>& B = T.mg_boxes[k];
+        std::vector<int> bx;
+        for (const Box& b : B) bx.insert(bx.end(), {b.lo[0], b.lo[1], b.lo[2], b.hi[0], b.hi[1], b.hi[2]});
+        pa_level_desc L{};
+        for (int d = 0; d < 3; ++d) {
+            L.domain_lo[d] = T.mg_dom[k].lo[d];
+            L.domain_hi[d] = T.mg_dom[k].hi[d];
+            L.dx[d] = H.lev[0].dx[d] * (double)(1 << k);
+        }
+        L.nboxes = (int)B.size();
+        L.boxes = bx.data();
+        L.owner = nullptr;
+        pa_hier* m = nullptr;
+        CHK(pa_hier_create2(&m, 1, &L, H.is_per, H.bc_kind, 0, 1, 0u));
+        S.mg_h.push_back(m);
+        S.mg_f.push_back({nullptr, nullptr, nullptr});
+        for (pa_field*& f : S.mg_f.back()) CHK(pa_field_alloc(m, 1, 1, &f));
+    }
+    CU(S.mg_avg.upload(T.mg_avg, t_stream));
+    CU(cudaStreamSynchronize(t_stream));
+    S.mg_ready = true;
+    return PA_OK;
+}
 
-int pa_smooth(pa_field* state, int comp_S, double prog_min, double prog_max, const pa_smooth_opts* o, pa_field* out, int comp_c,
-              int comp_phi, int* iters, double* resid) {
-    if (iters) *iters = 0;
-    if (resid) *resid = 0.0;
+// What pa_smooth and pa_debug_smooth_vcycle share: argument checks, tables, work fields (and, with mg, the multigrid
+// preconditioner's), and c = (S - progMin) * invdenom -- pa_curvature's Progress arithmetic (curvature.cpp:310-321) -- into
+// out[comp_c] and, for t > 0, into the right-hand side w[1]; for t = 0 into out[comp_phi] as well.
+int smooth_prepare(pa_field* state, int comp_S, double prog_min, double prog_max, const pa_smooth_opts* o, pa_field* out, int comp_c,
+                   int comp_phi, SmCtx& c) {
     if (!o) return fail(PA_ERR_ARG, "pa_smooth: null options");
     CHK(check_field(state, comp_S, 1, "pa_smooth(state)"));
     CHK(check_field(out, comp_c, 1, "pa_smooth(out, comp_c)"));
@@ -1623,8 +1792,8 @@ int pa_smooth(pa_field* state, int comp_S, double prog_min, double prog_max, con
     const double t = o->smoothing_time;
     if (!(t >= 0.0) || !std::isfinite(t)) return fail(PA_ERR_ARG, "pa_smooth: smoothing_time must be finite and >= 0");
     if (!(o->tol_rel >= 0.0) || o->max_iter < 0) return fail(PA_ERR_ARG, "pa_smooth: tol_rel and max_iter must be >= 0 (0 = default)");
-    const double tol_rel = o->tol_rel > 0.0 ? o->tol_rel : SMOOTH_TOL_REL;
-    const int max_iter = o->max_iter > 0 ? o->max_iter : SMOOTH_MAX_ITER;
+    if (o->precond != PA_SMOOTH_PRECOND_JACOBI && o->precond != PA_SMOOTH_PRECOND_MG)
+        return fail(PA_ERR_ARG, "pa_smooth: unknown precond " + std::to_string(o->precond) + " (PA_SMOOTH_PRECOND_JACOBI = 0, PA_SMOOTH_PRECOND_MG = 1)");
     pa_hier* h = state->h;
     Hier& H = h->H;
     if (H.nranks > 1) return fail(PA_ERR_UNSUPPORTED, "pa_smooth supports one rank only (do_smooth is not available on several GPUs)");
@@ -1637,7 +1806,6 @@ int pa_smooth(pa_field* state, int comp_S, double prog_min, double prog_max, con
     const SmoothTables& T = H.smooth_tables(SMOOTH_MAXORDER);
     if (!T.err.empty()) return fail(PA_ERR_ARG, T.err);
     CHK(ensure_smooth(h, T));
-    SmCtx c;
     c.h = h; c.S = h->sm.get(); c.T = &T; c.beta = t; c.nlev = H.nlev;
     for (int l = 0; l < H.nlev; ++l) {
         int err = PA_OK;
@@ -1645,8 +1813,19 @@ int pa_smooth(pa_field* state, int comp_S, double prog_min, double prog_max, con
         if (!ly && !H.lev[l].local.empty()) return err;
         c.lay.push_back(ly);
     }
-    pa_field **w = c.S->w, *x = w[0], *b = w[1], *r = w[2], *r0 = w[3], *p = w[4], *v = w[5], *tt = w[6], *z = w[7];
-    // c = (S - progMin) * invdenom: pa_curvature's Progress arithmetic (curvature.cpp:310-321), into out and into b
+    c.mg = o->precond == PA_SMOOTH_PRECOND_MG;
+    if (c.mg && t > 0.0) {
+        CHK(ensure_smooth_mg(h, T));
+        SmoothDev& S = *c.S;
+        for (int l = 0; l < H.nlev; ++l) c.amr.push_back(SmLev{h, l, S.recs.p, c.lay[l], nullptr, S.mg_rhs, S.mg_res});
+        for (size_t k = 0; k < S.mg_h.size(); ++k) {
+            int err = PA_OK;
+            const PaLayDev* ly = dev_layout(S.mg_h[k], 0, 1, &err);
+            if (!ly) return err;
+            c.coarse.push_back(SmLev{S.mg_h[k], 0, nullptr, ly, S.mg_f[k][0], S.mg_f[k][1], S.mg_f[k][2]});
+        }
+    }
+    pa_field* b = c.S->w[1];
     const double invdenom = 1.0 / (prog_max - prog_min);
     for (int l = 0; l < H.nlev; ++l) {
         const LevelDev& D = *h->lev[l];
@@ -1662,20 +1841,66 @@ int pa_smooth(pa_field* state, int comp_S, double prog_min, double prog_max, con
         else
             CU(launch_progress(D.boxes.p, ls, c.lay[l], nb, S, b->slab[l], prog_min, invdenom, t_stream));
     }
-    if (t == 0.0) return PA_OK;
-    const std::vector<double> one(H.nlev, 1.0), zero(H.nlev, 0.0);
-    std::vector<double> jac(H.nlev);         // right preconditioner: the inverse diagonal of each level's operator
+    return PA_OK;
+}
+
+// x = c (initial guess), then b's covered cells <- 0 (the right-hand side lives on the uncovered cells); *bmax = max|b|
+int smooth_start(SmCtx& c, pa_field* x, pa_field* b, double* bmax) {
+    const SmoothTables& T = *c.T;
+    const std::vector<double> one(c.nlev, 1.0);
+    CHK(sm_lin(c, one, b, 0.0, nullptr, 0.0, nullptr, x));
+    for (int l = 0; l + 1 < c.nlev; ++l)
+        CU(launch_sm_avgdown(c.S->avg.p + T.avg_begin[l], (int)(T.avg_begin[l + 1] - T.avg_begin[l]), T.avg_cells[l], c.h->lev[l]->boxes.p,
+                             c.lay[l], c.h->lev[l + 1]->boxes.p, c.lay[l + 1], b->slab[l], nullptr, true, t_stream));
+    CHK(sm_reduce(c, b, nullptr, 1, bmax));
+    if (!std::isfinite(*bmax)) return fail(PA_ERR_ARG, "pa_smooth: the progress variable has non-finite values");
+    return PA_OK;
+}
+
+// covered cells of phi <- fine averages, then phi -> out[comp_phi]
+int smooth_finish(SmCtx& c, pa_field* x, pa_field* out, int comp_phi) {
+    pa_hier* h = c.h;
+    const Hier& H = h->H;
+    const SmoothTables& T = *c.T;
+    for (int l = H.nlev - 2; l >= 0; --l)
+        CU(launch_sm_avgdown(c.S->avg.p + T.avg_begin[l], (int)(T.avg_begin[l + 1] - T.avg_begin[l]), T.avg_cells[l], h->lev[l]->boxes.p,
+                             c.lay[l], h->lev[l + 1]->boxes.p, c.lay[l + 1], x->slab[l], x->slab[l + 1], false, t_stream));
     for (int l = 0; l < H.nlev; ++l) {
+        const LevelDev& D = *h->lev[l];
+        int err = PA_OK;
+        const PaLayDev* lo = dev_layout(h, l, out->ng, &err);
+        CU(launch_sm_copy(D.boxes.p, c.lay[l], lo, D.host_off.p, (int)H.lev[l].local.size(), D.host_off_h.back(), x->slab[l],
+                          out->slab[l] + (long long)comp_phi * out->cs[l], t_stream));
+    }
+    return PA_OK;
+}
+
+}  // namespace
+extern "C" {
+
+int pa_smooth(pa_field* state, int comp_S, double prog_min, double prog_max, const pa_smooth_opts* o, pa_field* out, int comp_c,
+              int comp_phi, int* iters, double* resid) {
+    if (iters) *iters = 0;
+    if (resid) *resid = 0.0;
+    SmCtx c;
+    CHK(smooth_prepare(state, comp_S, prog_min, prog_max, o, out, comp_c, comp_phi, c));
+    const double t = c.beta;
+    if (t == 0.0) return PA_OK;
+    const double tol_rel = o->tol_rel > 0.0 ? o->tol_rel : SMOOTH_TOL_REL;
+    const int max_iter = o->max_iter > 0 ? o->max_iter : SMOOTH_MAX_ITER;
+    const int nlev = c.nlev;
+    const Hier& H = c.h->H;
+    pa_field **w = c.S->w, *x = w[0], *b = w[1], *r = w[2], *r0 = w[3], *p = w[4], *v = w[5], *tt = w[6], *z = w[7];
+    const std::vector<double> one(nlev, 1.0), zero(nlev, 0.0);
+    std::vector<double> jac(nlev);           // Jacobi preconditioner: the inverse diagonal of each level's operator
+    for (int l = 0; l < nlev; ++l) {
         const double* q = H.lev[l].dxinv;
         jac[l] = 1.0 / (1.0 + 2.0 * t * (q[0] * q[0] + q[1] * q[1] + q[2] * q[2]));
     }
-    CHK(sm_lin(c, one, b, 0.0, nullptr, 0.0, nullptr, x));                  // initial guess: c
-    for (int l = 0; l + 1 < H.nlev; ++l)                                    // the right-hand side lives on the uncovered cells
-        CU(launch_sm_avgdown(c.S->avg.p + T.avg_begin[l], (int)(T.avg_begin[l + 1] - T.avg_begin[l]), T.avg_cells[l], h->lev[l]->boxes.p,
-                             c.lay[l], h->lev[l + 1]->boxes.p, c.lay[l + 1], b->slab[l], nullptr, true, t_stream));
+    // z = M^-1 y: the Jacobi scaling or one V-cycle
+    auto precondition = [&](pa_field* y) -> int { return c.mg ? sm_vcycle(c, y, z) : sm_lin(c, jac, y, 0.0, nullptr, 0.0, nullptr, z); };
     double bmax = 0.0;
-    CHK(sm_reduce(c, b, nullptr, 1, &bmax));
-    if (!std::isfinite(bmax)) return fail(PA_ERR_ARG, "pa_smooth: the progress variable has non-finite values");
+    CHK(smooth_start(c, x, b, &bmax));
     const double tol = tol_rel * bmax;
     // true residual r = b - A x
     auto true_residual = [&](double* rn) -> int {
@@ -1712,7 +1937,7 @@ int pa_smooth(pa_field* state, int comp_S, double prog_min, double prog_max, con
         if (rho == 0.0 || !std::isfinite(rho)) { restart = true; CHK(true_residual(&rnorm)); continue; }
         const double bk = (rho / rho_old) * (alpha / omega);
         CHK(sm_lin(c, one, r, bk, p, -bk * omega, v, p));                   // p = r + bk (p - omega v)
-        CHK(sm_lin(c, jac, p, 0.0, nullptr, 0.0, nullptr, z));               // z = M^-1 p
+        CHK(precondition(p));                                                // z = M^-1 p
         CHK(sm_matvec(c, z, v));                                             // v = A z
         double den = 0.0;
         CHK(sm_reduce(c, r0, v, 0, &den));
@@ -1724,7 +1949,7 @@ int pa_smooth(pa_field* state, int comp_S, double prog_min, double prog_max, con
         CHK(sm_reduce(c, r, nullptr, 1, &snorm));
         rho_old = rho;
         if (!(snorm <= tol)) {
-            CHK(sm_lin(c, jac, r, 0.0, nullptr, 0.0, nullptr, z));           // z = M^-1 s
+            CHK(precondition(r));                                            // z = M^-1 s
             CHK(sm_matvec(c, z, tt));                                        // t = A z
             double ts = 0.0, t2 = 0.0;
             CHK(sm_reduce(c, tt, r, 0, &ts));
@@ -1741,20 +1966,38 @@ int pa_smooth(pa_field* state, int comp_S, double prog_min, double prog_max, con
             if (!(rnorm <= tol)) restart = true;
         }
     }
-    // covered cells of phi <- fine averages, then phi -> out
-    for (int l = H.nlev - 2; l >= 0; --l)
-        CU(launch_sm_avgdown(c.S->avg.p + T.avg_begin[l], (int)(T.avg_begin[l + 1] - T.avg_begin[l]), T.avg_cells[l], h->lev[l]->boxes.p,
-                             c.lay[l], h->lev[l + 1]->boxes.p, c.lay[l + 1], x->slab[l], x->slab[l + 1], false, t_stream));
-    for (int l = 0; l < H.nlev; ++l) {
-        const LevelDev& D = *h->lev[l];
-        int err = PA_OK;
-        const PaLayDev* lo = dev_layout(h, l, out->ng, &err);
-        CU(launch_sm_copy(D.boxes.p, c.lay[l], lo, D.host_off.p, (int)H.lev[l].local.size(), D.host_off_h.back(), x->slab[l],
-                          out->slab[l] + (long long)comp_phi * out->cs[l], t_stream));
-    }
+    CHK(smooth_finish(c, x, out, comp_phi));
     if (iters) *iters = it;
     if (resid) *resid = bmax > 0.0 ? rnorm / bmax : 0.0;
     return PA_OK;
+}
+
+int pa_debug_smooth_vcycle(pa_field* state, int comp_S, double prog_min, double prog_max, const pa_smooth_opts* o, pa_field* out,
+                           int comp_c, int comp_phi, int ncycles, double* resid, int* nmg) {
+    if (nmg) *nmg = 0;
+    if (!o || !(o->smoothing_time > 0.0)) return fail(PA_ERR_ARG, "pa_debug_smooth_vcycle: needs options with smoothing_time > 0");
+    if (ncycles < 0 || !resid) return fail(PA_ERR_ARG, "pa_debug_smooth_vcycle: ncycles must be >= 0 and resid non-null");
+    pa_smooth_opts om = *o;
+    om.precond = PA_SMOOTH_PRECOND_MG;
+    SmCtx c;
+    CHK(smooth_prepare(state, comp_S, prog_min, prog_max, &om, out, comp_c, comp_phi, c));
+    if (nmg) *nmg = (int)c.T->mg_boxes.size();
+    pa_field **w = c.S->w, *x = w[0], *b = w[1], *r = w[2], *tt = w[6], *z = w[7];
+    const std::vector<double> one(c.nlev, 1.0);
+    double bmax = 0.0;
+    CHK(smooth_start(c, x, b, &bmax));
+    for (int n = 0; n <= ncycles; ++n) {
+        if (n > 0) {
+            CHK(sm_vcycle(c, r, z));
+            CHK(sm_lin(c, one, x, 1.0, z, 0.0, nullptr, x));               // phi += B r
+        }
+        CHK(sm_matvec(c, x, tt));
+        CHK(sm_lin(c, one, b, -1.0, tt, 0.0, nullptr, r));                 // r = c - A phi
+        double rn = 0.0;
+        CHK(sm_reduce(c, r, nullptr, 1, &rn));
+        resid[n] = bmax > 0.0 ? rn / bmax : rn;
+    }
+    return smooth_finish(c, x, out, comp_phi);
 }
 
 // ---------------------------------------------------------------------------------------------- debug

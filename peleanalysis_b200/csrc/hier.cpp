@@ -1066,6 +1066,39 @@ const SmoothTables& Hier::smooth_tables(int maxorder) {
         ++T.reflux_begin[(size_t)kv.first[0] * 6 + 2 * kv.first[1] + kv.first[2] + 1];
     }
     for (size_t i = 1; i < T.reflux_begin.size(); ++i) T.reflux_begin[i] += T.reflux_begin[i - 1];
+    // coarsenings of level 0 for the multigrid preconditioner (one rank: local index = global id)
+    T.mg_boxes.push_back(lev[0].boxes);
+    T.mg_dom.push_back(lev[0].dom);
+    T.mg_avg_begin.push_back(0);
+    auto coarsenable = [](const Box& B) {
+        for (int d = 0; d < 3; ++d)
+            if ((B.lo[d] & 1) || (B.len(d) & 1) || B.len(d) < 4) return false;
+        return true;
+    };
+    auto half = [](const Box& B) {
+        Box c;
+        for (int d = 0; d < 3; ++d) { c.lo[d] = B.lo[d] / 2; c.hi[d] = (B.hi[d] + 1) / 2 - 1; }
+        return c;
+    };
+    for (;;) {
+        const std::vector<Box>& F = T.mg_boxes.back();
+        if (!coarsenable(T.mg_dom.back()) || !std::all_of(F.begin(), F.end(), coarsenable)) break;
+        std::vector<Box> C(F.size());
+        long long start = 0;
+        for (size_t b = 0; b < F.size(); ++b) {
+            C[b] = half(F[b]);
+            PaAvgDown A;
+            A.cbox = A.fbox = (int)b;
+            for (int d = 0; d < 3; ++d) { A.lo[d] = C[b].lo[d]; A.n[d] = C[b].len(d); }
+            A.start = start;
+            start += C[b].npts();
+            T.mg_avg.push_back(A);
+        }
+        T.mg_avg_cells.push_back(start);
+        T.mg_avg_begin.push_back((long long)T.mg_avg.size());
+        T.mg_dom.push_back(half(T.mg_dom.back()));
+        T.mg_boxes.push_back(std::move(C));
+    }
     return done();
 }
 

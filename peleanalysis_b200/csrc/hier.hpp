@@ -166,6 +166,14 @@ struct SmoothTables {
     std::vector<long long> avg_cells;         // nlev: covered cells of each coarse level
     std::vector<PaReflux> reflux;             // sorted by (coarse level, dir, side)
     std::vector<long long> reflux_begin;      // nlev*6+1: first record of each (coarse level, 2*dir+side)
+    // multigrid preconditioner: level 0 and its coarsenings by 2 (MG level k+1 = MG level k with every box and the domain
+    // coarsened; it exists while every box of level k is coarsenable -- even low corner and length -- and the coarsened length is
+    // at least 2).  mg_boxes[0] / mg_dom[0] are level 0 itself; box b of MG level k+1 is box b of level k coarsened.
+    std::vector<std::vector<Box>> mg_boxes;
+    std::vector<Box> mg_dom;
+    std::vector<PaAvgDown> mg_avg;            // restriction / prolongation between MG levels k and k+1: one record per box
+    std::vector<long long> mg_avg_begin;      // nmg: first record of each (k, k+1) pair; [nmg-1] = end
+    std::vector<long long> mg_avg_cells;      // nmg-1: cells of MG level k+1
 };
 
 // BoxList::maxSize: every box replaced, in place, by its chunks no longer than max_grid_size (AMReX_BoxList.cpp:765-815)

@@ -186,6 +186,16 @@ cudaError_t launch_filter(int g, const PaBoxDev* boxes, const PaLayDev* lin, con
 // out = in - beta * Laplacian(in) on the valid cells of one level (`in` ghost-filled, one ghost layer)
 cudaError_t launch_sm_apply(const PaBoxDev* boxes, const PaLayDev* lay, const long long* host_off, int nboxes, long long ncells,
                             const double* in, double* out, double beta, const double dxi[3], cudaStream_t st);
+// out = rhs - A x on the valid cells of one level (`x` ghost-filled)
+cudaError_t launch_sm_resid(const PaBoxDev* boxes, const PaLayDev* lay, const long long* host_off, int nboxes, long long ncells,
+                            const double* rhs, const double* x, double* out, double beta, const double dxi[3], cudaStream_t st);
+// one colour pass of red-black Gauss-Seidel on A x = rhs over one level (`x` ghost-filled): x += (rhs - A x) / diag on the valid
+// cells with (i + j + k) mod 2 = colour
+cudaError_t launch_sm_gsrb(const PaBoxDev* boxes, const PaLayDev* lay, const long long* host_off, int nboxes, long long ncells,
+                           const double* rhs, double* x, double beta, const double dxi[3], double diag, int colour, cudaStream_t st);
+// fine cells under the records' coarse cells += the coarse value (piecewise-constant prolongation)
+cudaError_t launch_sm_prolong(const PaAvgDown* recs, int nrec, long long ncells, const PaBoxDev* cboxes, const PaLayDev* clay,
+                              const PaBoxDev* fboxes, const PaLayDev* flay, const double* crse, double* fine, cudaStream_t st);
 // coarse-fine faces of one (coarse level, dir, side) group: cout += the flux difference (average fine flux - coarse flux)
 cudaError_t launch_sm_reflux(const PaReflux* recs, long long nrec, const PaLayDev* clay, const PaLayDev* flay, const double* cin,
                              const double* fin, double* cout, double beta, double dxic, double dxif, cudaStream_t st);

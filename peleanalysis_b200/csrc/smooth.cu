@@ -37,7 +37,18 @@ int sm_grid(long long n) {
     return (int)g;
 }
 
-// out = in - beta * sum_d ((in(+e_d) - in) * dxi_d - (in - in(-e_d)) * dxi_d) * dxi_d on every valid cell
+// (A in)(a) = in - beta * sum_d ((in(+e_d) - in) * dxi_d - (in - in(-e_d)) * dxi_d) * dxi_d: the one expression of the operator,
+// shared by its application, the residual and the Gauss-Seidel sweep
+__device__ __forceinline__ double sm_op(const double* in, long long a, const PaLayDev& y, double beta, double dxi0, double dxi1,
+                                        double dxi2) {
+    const double v = in[a];
+    const double lx = ((in[a + 1] - v) * dxi0 - (v - in[a - 1]) * dxi0) * dxi0;
+    const double ly = ((in[a + y.P] - v) * dxi1 - (v - in[a - y.P]) * dxi1) * dxi1;
+    const double lz = ((in[a + y.PS] - v) * dxi2 - (v - in[a - y.PS]) * dxi2) * dxi2;
+    return v - beta * ((lx + ly) + lz);
+}
+
+// out = A in on every valid cell
 __global__ void __launch_bounds__(SM_BLOCK) k_sm_apply(const PaBoxDev* __restrict__ boxes, const PaLayDev* __restrict__ lay,
                                                      const long long* __restrict__ host_off, int nboxes, long long ncells,
                                                      const double* __restrict__ in, double* __restrict__ out, double beta,
@@ -47,11 +58,39 @@ __global__ void __launch_bounds__(SM_BLOCK) k_sm_apply(const PaBoxDev* __restric
         const int b = sm_locate(host_off, nboxes, boxes, c, i, j, k);
         const PaLayDev y = lay[b];
         const long long a = cell_addr(y, i, j, k);
-        const double v = in[a];
-        const double lx = ((in[a + 1] - v) * dxi0 - (v - in[a - 1]) * dxi0) * dxi0;
-        const double ly = ((in[a + y.P] - v) * dxi1 - (v - in[a - y.P]) * dxi1) * dxi1;
-        const double lz = ((in[a + y.PS] - v) * dxi2 - (v - in[a - y.PS]) * dxi2) * dxi2;
-        out[a] = v - beta * ((lx + ly) + lz);
+        out[a] = sm_op(in, a, y, beta, dxi0, dxi1, dxi2);
+    }
+}
+
+// out = rhs - A x on every valid cell
+__global__ void __launch_bounds__(SM_BLOCK) k_sm_resid(const PaBoxDev* __restrict__ boxes, const PaLayDev* __restrict__ lay,
+                                                     const long long* __restrict__ host_off, int nboxes, long long ncells,
+                                                     const double* __restrict__ rhs, const double* __restrict__ x,
+                                                     double* __restrict__ out, double beta, double dxi0, double dxi1, double dxi2) {
+    for (long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x; c < ncells; c += (long long)gridDim.x * blockDim.x) {
+        int i, j, k;
+        const int b = sm_locate(host_off, nboxes, boxes, c, i, j, k);
+        const PaLayDev y = lay[b];
+        const long long a = cell_addr(y, i, j, k);
+        out[a] = rhs[a] - sm_op(x, a, y, beta, dxi0, dxi1, dxi2);
+    }
+}
+
+// one colour of a red-black Gauss-Seidel sweep of A x = rhs: x += (rhs - A x) / diag on the valid cells with
+// (i + j + k) mod 2 = colour in global level indices.  Such a cell reads only cells of the other colour inside its box, and
+// ghost cells filled before the launch, so no cell is read and written in the same launch.
+__global__ void __launch_bounds__(SM_BLOCK) k_sm_gsrb(const PaBoxDev* __restrict__ boxes, const PaLayDev* __restrict__ lay,
+                                                    const long long* __restrict__ host_off, int nboxes, long long ncells,
+                                                    const double* __restrict__ rhs, double* x, double beta, double dxi0,
+                                                    double dxi1, double dxi2, double diag, int colour) {
+    for (long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x; c < ncells; c += (long long)gridDim.x * blockDim.x) {
+        int i, j, k;
+        const int b = sm_locate(host_off, nboxes, boxes, c, i, j, k);
+        const PaBoxDev B = boxes[b];
+        if (((B.lo[0] + i + B.lo[1] + j + B.lo[2] + k) & 1) != colour) continue;
+        const PaLayDev y = lay[b];
+        const long long a = cell_addr(y, i, j, k);
+        x[a] += (rhs[a] - sm_op(x, a, y, beta, dxi0, dxi1, dxi2)) / diag;
     }
 }
 
@@ -108,6 +147,31 @@ __global__ void __launch_bounds__(SM_BLOCK) k_sm_avgdown(const PaAvgDown* __rest
                 for (int ii = 0; ii < 2; ++ii)
                     s += fine[cell_addr(yf, 2 * ci + ii - fb.lo[0], 2 * cj + jj - fb.lo[1], 2 * ck + kk - fb.lo[2])];
         *p = 0.125 * s;
+    }
+}
+
+// piecewise-constant prolongation over average-down records: each of the 8 fine cells of a record's coarse cell += the coarse value
+__global__ void __launch_bounds__(SM_BLOCK) k_sm_prolong(const PaAvgDown* __restrict__ recs, int nrec, long long ncells,
+                                                       const PaBoxDev* __restrict__ cboxes, const PaLayDev* __restrict__ clay,
+                                                       const PaBoxDev* __restrict__ fboxes, const PaLayDev* __restrict__ flay,
+                                                       const double* __restrict__ crse, double* __restrict__ fine) {
+    for (long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x; c < ncells; c += (long long)gridDim.x * blockDim.x) {
+        long long lo = 0, hi = nrec;
+        while (hi - lo > 1) { long long mid = (lo + hi) >> 1; if (recs[mid].start <= c) lo = mid; else hi = mid; }
+        const PaAvgDown R = recs[lo];
+        const long long q = c - R.start;
+        const int ci = R.lo[0] + (int)(q % R.n[0]);
+        const long long r = q / R.n[0];
+        const int cj = R.lo[1] + (int)(r % R.n[1]);
+        const int ck = R.lo[2] + (int)(r / R.n[1]);
+        const PaBoxDev cb = cboxes[R.cbox];
+        const double v = crse[cell_addr(clay[R.cbox], ci - cb.lo[0], cj - cb.lo[1], ck - cb.lo[2])];
+        const PaBoxDev fb = fboxes[R.fbox];
+        const PaLayDev yf = flay[R.fbox];
+        for (int kk = 0; kk < 2; ++kk)
+            for (int jj = 0; jj < 2; ++jj)
+                for (int ii = 0; ii < 2; ++ii)
+                    fine[cell_addr(yf, 2 * ci + ii - fb.lo[0], 2 * cj + jj - fb.lo[1], 2 * ck + kk - fb.lo[2])] += v;
     }
 }
 
@@ -181,6 +245,31 @@ cudaError_t launch_sm_apply(const PaBoxDev* boxes, const PaLayDev* lay, const lo
                             const double* in, double* out, double beta, const double dxi[3], cudaStream_t st) {
     if (ncells <= 0) return cudaSuccess;
     PA_LAUNCH(sm_grid(ncells), SM_BLOCK, 0, st, k_sm_apply)(boxes, lay, host_off, nboxes, ncells, in, out, beta, dxi[0], dxi[1], dxi[2]);
+    ++g_launches;
+    return cudaGetLastError();
+}
+
+cudaError_t launch_sm_resid(const PaBoxDev* boxes, const PaLayDev* lay, const long long* host_off, int nboxes, long long ncells,
+                            const double* rhs, const double* x, double* out, double beta, const double dxi[3], cudaStream_t st) {
+    if (ncells <= 0) return cudaSuccess;
+    PA_LAUNCH(sm_grid(ncells), SM_BLOCK, 0, st, k_sm_resid)(boxes, lay, host_off, nboxes, ncells, rhs, x, out, beta, dxi[0], dxi[1], dxi[2]);
+    ++g_launches;
+    return cudaGetLastError();
+}
+
+cudaError_t launch_sm_gsrb(const PaBoxDev* boxes, const PaLayDev* lay, const long long* host_off, int nboxes, long long ncells,
+                           const double* rhs, double* x, double beta, const double dxi[3], double diag, int colour, cudaStream_t st) {
+    if (ncells <= 0) return cudaSuccess;
+    PA_LAUNCH(sm_grid(ncells), SM_BLOCK, 0, st, k_sm_gsrb)(boxes, lay, host_off, nboxes, ncells, rhs, x, beta, dxi[0], dxi[1], dxi[2], diag,
+                                                           colour);
+    ++g_launches;
+    return cudaGetLastError();
+}
+
+cudaError_t launch_sm_prolong(const PaAvgDown* recs, int nrec, long long ncells, const PaBoxDev* cboxes, const PaLayDev* clay,
+                              const PaBoxDev* fboxes, const PaLayDev* flay, const double* crse, double* fine, cudaStream_t st) {
+    if (ncells <= 0 || nrec <= 0) return cudaSuccess;
+    PA_LAUNCH(sm_grid(ncells), SM_BLOCK, 0, st, k_sm_prolong)(recs, nrec, ncells, cboxes, clay, fboxes, flay, crse, fine);
     ++g_launches;
     return cudaGetLastError();
 }

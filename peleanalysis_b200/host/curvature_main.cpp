@@ -3,7 +3,7 @@
 // strain rate / normal velocity branches run through the C ABI.  do_smooth=1 (curvature.cpp:328-406) solves the implicit
 // diffusion step with pa_smooth and runs the curvature on the smoothed field (one GPU only).  Extension: ngpus=N runs on N GPUs
 // from this one process, one host thread per GPU (multi_gpu.hpp); transport=peer|slab picks peer links + packed slabs (default)
-// or packed slabs only.
+// or packed slabs only; smooth_precond=jacobi|mg picks do_smooth's preconditioner (default jacobi).
 #include <algorithm>
 
 #include "multi_gpu.hpp"
@@ -30,6 +30,9 @@ int main(int argc, char** argv) {
     pp.query("threshold_value", threshold);
     pp.query("do_smooth", do_smooth);
     pp.query("smoothing_time", smooth_time);
+    std::string smooth_precond = "jacobi";
+    pp.query("smooth_precond", smooth_precond);
+    if (smooth_precond != "jacobi" && smooth_precond != "mg") pa_abort("smooth_precond must be jacobi or mg (got " + smooth_precond + ")");
     pp.query("do_strain", do_strain);
     if (do_strain) pp.query("getStrainTensor", getStrainTensor);
     pp.query("do_velnormal", do_velnormal);
@@ -161,11 +164,12 @@ int main(int argc, char** argv) {
     if (do_smooth) {
         pa_smooth_opts so{};
         so.smoothing_time = smooth_time;
+        so.precond = smooth_precond == "mg" ? PA_SMOOTH_PRECOND_MG : PA_SMOOTH_PRECOND_JACOBI;
         int iters = 0;
         double resid = 0.0;
         check(pa_smooth(st, 0, progMin, progMax, &so, st, comp_c, comp_phi, &iters, &resid), "pa_smooth");
-        if (verbose) std::cout << "do_smooth: smoothing_time = " << smooth_time << ", " << iters << " iterations, max|c - A phi| / max|c| = "
-                               << resid << "\n";
+        if (verbose) std::cout << "do_smooth: smoothing_time = " << smooth_time << ", precond " << smooth_precond << ", " << iters
+                               << " iterations, max|c - A phi| / max|c| = " << resid << "\n";
         // the curvature of phi with the identity normalisation (curvature.cpp:328-406 hands the solution on as the progress
         // variable); its Progress output is phi itself and goes to SmoothedProgress, Progress is c
         pa_curv_opts os = o;

@@ -197,6 +197,10 @@ def run(tool: str, argv: Sequence[str], capi=None, multigpu=None, wrap=None, bac
             raise SystemExit("amrex::Abort::0::do_smooth=1 runs on one GPU only: the smoothing solve has no multi-GPU path (run at world size 1) !!!")
         so = capi.SmoothOpts()
         so.smoothing_time = _get(pp, "smoothing_time", 1.0e-7, float)
+        precond = _get(pp, "smooth_precond", "jacobi")
+        if precond not in capi.SMOOTH_PRECONDS:
+            raise SystemExit("amrex::Abort::0::smooth_precond must be jacobi or mg (got %s) !!!" % precond)
+        so.precond = capi.SMOOTH_PRECONDS[precond]
         if _get(pp, "useFileMinMax", 1, int):
             o.prog_min, o.prog_max = plotfile.file_min_max(infile, prog, nlev)
         else:
@@ -252,7 +256,8 @@ def run(tool: str, argv: Sequence[str], capi=None, multigpu=None, wrap=None, bac
         cc, cphi = len(dev_in), len(dev_in) + 1
         iters, resid = capi.smooth(fin, 0, o.prog_min, o.prog_max, so, fin, cc, cphi)
         if _get(pp, "verbose", 0, int):
-            print("do_smooth: smoothing_time = %g, %d iterations, max|c - A phi| / max|c| = %g" % (so.smoothing_time, iters, resid))
+            print("do_smooth: smoothing_time = %g, precond %s, %d iterations, max|c - A phi| / max|c| = %g" % (so.smoothing_time, precond, iters,
+                                                                                                              resid))
         o_phi = capi.CurvOpts.from_buffer_copy(o)
         o_phi.prog_min, o_phi.prog_max = 0.0, 1.0
         capi.curvature(fin, cphi, 1, o_phi, fout, 0)

@@ -75,12 +75,15 @@ class CurvatureRun(_Run):
 
     do_smooth (one rank only, curvature.cpp:328-406): the progress variable c is first smoothed by one implicit diffusion
     step of `smoothing_time` (capi.smooth) and the curvature runs on the smoothed phi with prog_min = 0, prog_max = 1.
+    smooth_precond picks the solve's preconditioner: "jacobi" (default) or "mg" (a multigrid V-cycle).
     Progress stays c; smoothed_progress() returns phi; `iterations` / `residual` report the last solve."""
 
     VEL = ("x_velocity", "y_velocity", "z_velocity")
 
     def __init__(self, P, pf: Plotfile, opts, progress: str = "temp", is_per=(1, 1, 1), sym_dir=(0, 0, 0), upload: bool = True,
-                 rank: int = 0, nranks: int = 1, multigpu=None, wrap=None, do_smooth: bool = False, smoothing_time: float = 1.0e-7):
+                 rank: int = 0, nranks: int = 1, multigpu=None, wrap=None, do_smooth: bool = False, smoothing_time: float = 1.0e-7,
+                 smooth_precond: str = "jacobi"):
+        precond = P.smooth_precond(smooth_precond)
         if do_smooth and nranks > 1:
             raise ValueError("do_smooth runs on one rank only: the smoothing solve has no multi-rank path")
         super().__init__(P, pf, is_per, sym_dir, rank, nranks, multigpu, wrap)
@@ -93,6 +96,7 @@ class CurvatureRun(_Run):
         if self.do_smooth:
             self.sopts = P.SmoothOpts()
             self.sopts.smoothing_time = smoothing_time
+            self.sopts.precond = precond
             self.opts_phi = P.CurvOpts.from_buffer_copy(opts)
             self.opts_phi.prog_min, self.opts_phi.prog_max = 0.0, 1.0
         self.state = P.Field(self.hier, nst + 2 if self.do_smooth else nst, 1)
