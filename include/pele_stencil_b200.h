@@ -299,6 +299,10 @@ int pa_exchange_mark_received(pa_field *f, int comp, int ncomp);   /* recv slab 
 
 /* ---- instrumentation --------------------------------------------------------------------------------- */
 int64_t pa_kernel_launches(void);              /* number of kernels this library launched so far (this process) */
+/* Bytes of device memory the library holds on the calling thread's current device: every live allocation of hierarchies,
+ * fields and the library's internal counters.  After a hierarchy and its fields are freed, only the per-stream counters
+ * the first kernels created remain, so the value returns to the same number after every file of a series. */
+int pa_debug_device_bytes(int64_t *out);
 int pa_hier_build_seconds(const pa_hier *h, double *seconds);
 /* Algorithmic bytes of SURVEY 8(d): sum over local boxes of 8*V_in + 8*nout*V, V_in = V + 2(nx*ny+ny*nz+nx*nz). */
 int64_t pa_algorithmic_bytes(const pa_hier *h, int nout_per_cell);

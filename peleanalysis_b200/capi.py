@@ -80,6 +80,7 @@ SYMBOLS = {
     "pa_exchange_buffers": (_i, [_vp, _i, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_i64), C.POINTER(_i64)]),
     "pa_exchange_pack": (_i, [_vp, _i, _i]), "pa_exchange_mark_received": (_i, [_vp, _i, _i]),
     "pa_kernel_launches": (_i64, []), "pa_hier_build_seconds": (_i, [_vp, C.POINTER(_d)]),
+    "pa_debug_device_bytes": (_i, [C.POINTER(_i64)]),
     "pa_algorithmic_bytes": (_i64, [_vp, _i]),
     "pa_debug_download_grown": (_i, [_vp, _i, _i, _i, _vp]),
     "pa_debug_fb_source_map": (_i, [_vp, _i, _i, _i, _vp, _i64]),
@@ -139,6 +140,13 @@ def sync() -> None:
 
 def kernel_launches() -> int:
     return int(lib().pa_kernel_launches())
+
+
+def device_bytes() -> int:
+    """Device memory the library holds on the current device (pa_debug_device_bytes)."""
+    v = _i64()
+    check(lib().pa_debug_device_bytes(C.byref(v)))
+    return int(v.value)
 
 
 def curv_fused_launches() -> int:

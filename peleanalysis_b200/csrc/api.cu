@@ -9,7 +9,9 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <map>
 #include <memory>
+#include <mutex>
 #include <string>
 #include <vector>
 
@@ -18,6 +20,37 @@
 #include "kernels.cuh"
 
 using namespace pa;
+
+namespace pa {
+namespace {
+std::mutex g_alloc_mu;
+std::map<void*, std::pair<int, size_t>> g_alloc;       // live allocation -> (device, bytes)
+std::map<int, int64_t> g_alloc_bytes;                  // device -> live bytes
+}  // namespace
+
+cudaError_t dev_alloc(void** p, size_t bytes) {
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaMalloc(p, bytes);
+    if (e != cudaSuccess) return e;
+    std::lock_guard<std::mutex> lk(g_alloc_mu);
+    g_alloc[*p] = {dev, bytes};
+    g_alloc_bytes[dev] += (int64_t)bytes;
+    return cudaSuccess;
+}
+void dev_free(void* p) {
+    if (!p) return;
+    {
+        std::lock_guard<std::mutex> lk(g_alloc_mu);
+        auto it = g_alloc.find(p);
+        if (it != g_alloc.end()) {
+            g_alloc_bytes[it->second.first] -= (int64_t)it->second.second;
+            g_alloc.erase(it);
+        }
+    }
+    cudaFree(p);
+}
+}  // namespace pa
 
 namespace {
 
@@ -36,19 +69,19 @@ template <class T>
 struct DevBuf {
     T* p = nullptr;
     size_t n = 0;
-    ~DevBuf() { if (p) cudaFree(p); }
+    ~DevBuf() { if (p) dev_free(p); }
     cudaError_t upload(const std::vector<T>& v, cudaStream_t st) {
-        if (p) { cudaFree(p); p = nullptr; }
+        if (p) { dev_free(p); p = nullptr; }
         n = v.size();
         if (!n) return cudaSuccess;
-        cudaError_t e = cudaMalloc(&p, n * sizeof(T));
+        cudaError_t e = dev_alloc((void**)&p, n * sizeof(T));
         if (e != cudaSuccess) return e;
         return cudaMemcpyAsync(p, v.data(), n * sizeof(T), cudaMemcpyHostToDevice, st);
     }
     cudaError_t reserve(size_t m) {
         if (m <= n) return cudaSuccess;
-        if (p) { cudaFree(p); p = nullptr; n = 0; }
-        cudaError_t e = cudaMalloc(&p, m * sizeof(T));
+        if (p) { dev_free(p); p = nullptr; n = 0; }
+        cudaError_t e = dev_alloc((void**)&p, m * sizeof(T));
         if (e == cudaSuccess) n = m;
         return e;
     }
@@ -704,6 +737,15 @@ int pa_host_free(void* p) { CU(cudaFreeHost(p)); return PA_OK; }
 int pa_host_register(void* p, size_t bytes) { CU(cudaHostRegister(p, bytes, cudaHostRegisterDefault)); return PA_OK; }
 int pa_host_unregister(void* p) { CU(cudaHostUnregister(p)); return PA_OK; }
 int64_t pa_kernel_launches(void) { return g_launches; }
+int pa_debug_device_bytes(int64_t* out) {
+    if (!out) return fail(PA_ERR_ARG, "pa_debug_device_bytes: null output");
+    int dev = 0;
+    CU(cudaGetDevice(&dev));
+    std::lock_guard<std::mutex> lk(g_alloc_mu);
+    auto it = g_alloc_bytes.find(dev);
+    *out = it == g_alloc_bytes.end() ? 0 : it->second;
+    return PA_OK;
+}
 
 int pa_hier_create(pa_hier** out, int nlev, const pa_level_desc* levels, const int is_per[3], const int bc_kind[3],
                    int rank, int nranks) {
@@ -805,9 +847,9 @@ int pa_field_alloc(pa_hier* h, int ncomp, int nghost, pa_field** out) {
         }
         size_t n = (size_t)Y.comp_stride * ncomp + 16;          // 16 doubles of slack: pair loads may touch one element past a row
         if (Y.comp_stride == 0) continue;
-        cudaError_t e = cudaMalloc(&f->slab[l], n * sizeof(double));
+        cudaError_t e = dev_alloc((void**)&f->slab[l], n * sizeof(double));
         if (e != cudaSuccess) {
-            for (double* p : f->slab) if (p) cudaFree(p);
+            for (double* p : f->slab) if (p) dev_free(p);
             return e == cudaErrorMemoryAllocation ? fail(PA_ERR_NOMEM, "pa_field_alloc: out of device memory") : cuda_fail(e, "cudaMalloc");
         }
         // ghost cells and pads start as zeros (never NaN garbage)
@@ -828,7 +870,7 @@ int pa_field_free(pa_field* f) {
     if (f->h && f->h->recv_owner == f) f->h->recv_owner = nullptr;
     if (f->h && f->h->fp_mark.f == f) f->h->fp_mark = pa_hier::FpMark();
     for (void* p : f->ipc_mapped) cudaIpcCloseMemHandle(p);
-    for (double* p : f->slab) if (p) cudaFree(p);
+    for (double* p : f->slab) if (p) dev_free(p);
     delete f;
     return PA_OK;
 }
@@ -1030,20 +1072,20 @@ int pa_field_hash(const pa_field* f, int comp, int ncomp, uint64_t* out) {
     pa_hier* h = f->h;
     CHK(ensure_device(h));
     unsigned long long* d = nullptr;
-    CU(cudaMalloc(&d, sizeof(unsigned long long)));
+    CU(dev_alloc((void**)&d, sizeof(unsigned long long)));
     cudaError_t e = cudaMemsetAsync(d, 0, sizeof(unsigned long long), t_stream);
     for (int l = 0; l < h->H.nlev && e == cudaSuccess; ++l) {
         const int nb = (int)h->H.lev[l].local.size();
         if (!nb) continue;
         int err = PA_OK;
         const PaLayDev* ly = dev_layout(h, l, f->ng, &err);
-        if (!ly) { cudaFree(d); return err; }
+        if (!ly) { dev_free(d); return err; }
         e = launch_field_hash(h->lev[l]->boxes.p, ly, h->lev[l]->gid.p, nb, f->slab[l] + (long long)comp * f->cs[l], f->cs[l], comp, ncomp, l, d, t_stream);
     }
     unsigned long long v = 0;
     if (e == cudaSuccess) e = cudaMemcpyAsync(&v, d, sizeof(v), cudaMemcpyDeviceToHost, t_stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(t_stream);
-    cudaFree(d);
+    dev_free(d);
     if (e != cudaSuccess) return cuda_fail(e, "pa_field_hash");
     *out = (uint64_t)v;
     return PA_OK;
@@ -2426,7 +2468,7 @@ int pa_debug_fp64_rate(double* gops) {
     if (esm != cudaSuccess) return cuda_fail(esm, "device query");
     const int blocks = nsm * 8, threads = 256, iters = 4096;
     double* buf = nullptr;
-    CU(cudaMalloc(&buf, (size_t)blocks * threads * sizeof(double)));
+    CU(dev_alloc((void**)&buf, (size_t)blocks * threads * sizeof(double)));
     cudaEvent_t e0, e1;
     cudaEventCreate(&e0); cudaEventCreate(&e1);
     cudaError_t e = launch_fp64_rate(buf, blocks, threads, 64, t_stream);        // warm-up
@@ -2440,7 +2482,7 @@ int pa_debug_fp64_rate(double* gops) {
         if (e == cudaSuccess) { cudaEventElapsedTime(&ms, e0, e1); best = std::min(best, ms); }
     }
     cudaEventDestroy(e0); cudaEventDestroy(e1);
-    cudaFree(buf);
+    dev_free(buf);
     if (e != cudaSuccess) return cuda_fail(e, "pa_debug_fp64_rate");
     *gops = (double)blocks * threads * iters * 16.0 / (best * 1e-3) / 1e9;
     return PA_OK;

@@ -72,6 +72,11 @@ struct StencilExtra {
 
 extern std::atomic<long long> g_launches;     // kernels launched by this library (host threads may launch concurrently)
 
+// Every device allocation of the library goes through these two (api.cu), which keep the live bytes per device for
+// pa_debug_device_bytes: a long series of plotfiles must not grow the device footprint.
+cudaError_t dev_alloc(void** p, size_t bytes);
+void dev_free(void* p);
+
 cudaError_t launch_unpack_valid(const PaBoxDev* boxes, const PaLayDev* lay, const long long* host_off, int nboxes,
                                 long long ncells, const double* staging, double* comp_base, cudaStream_t st);
 cudaError_t launch_pack_valid(const PaBoxDev* boxes, const PaLayDev* lay, const long long* host_off, int nboxes,

@@ -479,7 +479,7 @@ cudaError_t launch_mode(const PaTile* tiles, int ntiles, int stage_doubles, cons
     const int grid = (int)std::min<long long>(nwork, (long long)num_sms * per_sm);
     Ticket& T = g_tickets[std::make_pair(dev, st)];
     if (!T.dev) {
-        cudaError_t e = cudaMalloc(&T.dev, sizeof(unsigned long long));
+        cudaError_t e = dev_alloc((void**)&T.dev, sizeof(unsigned long long));
         if (e == cudaSuccess) e = cudaMemset(T.dev, 0, sizeof(unsigned long long));
         if (e != cudaSuccess) return e;
     }
@@ -624,7 +624,7 @@ __global__ void k_selftest_math(long long n, unsigned long long seed, unsigned l
 
 cudaError_t selftest_math(long long n, unsigned long long seed, unsigned long long* bad_host, cudaStream_t st) {
     unsigned long long* d = nullptr;
-    cudaError_t e = cudaMalloc(&d, sizeof(unsigned long long));
+    cudaError_t e = dev_alloc((void**)&d, sizeof(unsigned long long));
     if (e != cudaSuccess) return e;
     e = cudaMemsetAsync(d, 0, sizeof(unsigned long long), st);
     int nsm = 0;
@@ -632,7 +632,7 @@ cudaError_t selftest_math(long long n, unsigned long long seed, unsigned long lo
     if (e == cudaSuccess) { PA_LAUNCH(nsm * 8, 256, 0, st, k_selftest_math)(n, seed, d); ++g_launches; e = cudaGetLastError(); }
     if (e == cudaSuccess) e = cudaMemcpyAsync(bad_host, d, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    cudaFree(d);
+    dev_free(d);
     return e;
 }
 
@@ -663,7 +663,7 @@ cudaError_t stencil_ticket(cudaStream_t st, unsigned long long nwork, int grid, 
     if (e != cudaSuccess) return e;
     Ticket& T = g_tickets[std::make_pair(dev, st)];
     if (!T.dev) {
-        e = cudaMalloc(&T.dev, sizeof(unsigned long long));
+        e = dev_alloc((void**)&T.dev, sizeof(unsigned long long));
         if (e == cudaSuccess) e = cudaMemset(T.dev, 0, sizeof(unsigned long long));
         if (e != cudaSuccess) return e;
     }
@@ -673,7 +673,7 @@ cudaError_t stencil_ticket(cudaStream_t st, unsigned long long nwork, int grid, 
 }
 void stencil_tma_release() {                          // pa_finalize: the per-stream ticket counters
     std::lock_guard<std::mutex> lock(g_launch_mutex);
-    for (auto& kv : g_tickets) if (kv.second.dev) cudaFree(kv.second.dev);
+    for (auto& kv : g_tickets) if (kv.second.dev) dev_free(kv.second.dev);
     g_tickets.clear();
 }
 int stencil_tma_tile_rows() { return MAX_TILE_ROWS; }

@@ -6,136 +6,188 @@
 //                                                                        ngpus=N  (one host thread per GPU, multi_gpu.hpp)
 //                                                                        transport=peer|slab  (with ngpus=N: peer links +
 //                                                                        packed slabs, or packed slabs only)
+//                                                                        infiles=a b c  (a series of plotfiles in one run,
+//                                                                        series.hpp; every other key applies to each file)
 #include <chrono>
 
 #include "multi_gpu.hpp"
-#include "tool_common.hpp"
+#include "series.hpp"
 
 static void print_usage(char** argv) {
     std::cerr << "usage:\n" << argv[0] << " infile=<plotfilename> \n\tOptions:\n\tis_per=<L M N> gradVar=<name>\n";
     std::exit(1);
 }
 
+struct GradOpts {                                      // the keys every file of a run shares
+    int finestLevel = 1000;
+    std::vector<std::string> gvars, aux;
+    std::vector<int> is_per;
+    int bck[3];
+};
+
+struct GradFile {                                      // one plotfile, checked
+    std::string infile, outfile;
+    pltio::Header H;
+    int Nlev = 0;
+    std::vector<std::string> names;
+    int nv = 0, nIn = 0, nOut = 0;
+};
+
+// the checks of a single run on one plotfile; `who` prefixes every abort message (a series names the file)
+static GradFile grad_file(const GradOpts& o, const std::string& infile, const std::string& who) {
+    GradFile F;
+    F.infile = infile;
+    try { F.H = pltio::read_header(infile); } catch (std::exception& e) { pa_abort(who + std::string("cannot read plotfile: ") + e.what()); }
+    F.Nlev = std::min(o.finestLevel, F.H.finest_level) + 1;
+    for (auto& v : o.gvars)
+        if (F.H.comp(v) < 0) { std::cout << "Cannot find " << v << " data in pltfile \n"; pa_abort(who + "Cannot find " + v + " data in pltfile"); }
+    for (auto& a : o.aux)
+        if (F.H.comp(a) < 0) pa_abort(who + "Unknown auxiliary variable name: " + a);
+    F.nv = (int)o.gvars.size();
+    F.nIn = F.nv + (int)o.aux.size();
+    F.nOut = F.nIn + 4 * F.nv;
+    for (auto& v : o.gvars) F.names.push_back(v);
+    for (auto& a : o.aux) F.names.push_back(a);
+    for (auto& v : o.gvars) { F.names.push_back(v + "_gx"); F.names.push_back(v + "_gy"); F.names.push_back(v + "_gz"); F.names.push_back("||grad" + v + "||"); }
+    F.outfile = file_root(infile) + "_gt";
+    return F;
+}
+
+// disk -> in[l] components 0 .. nIn-1 (gradient variables, then pass-through variables); ncomp = the components to allocate
+static void grad_read(const GradOpts& o, const GradFile& F, HostSet& in, int ncomp, bool talk) {
+    ensure_levels(in, F.Nlev);
+    for (int l = 0; l < F.Nlev; ++l) {
+        if (talk) std::cout << "Reading data for level: " << l << std::endl;
+        in[l].alloc(F.H.levels[l].ncells(), ncomp);
+        for (int v = 0; v < F.nv; ++v) pltio::read_level_comp(F.infile, F.H, l, F.H.comp(o.gvars[v]), in[l].comp(v));
+        for (size_t a = 0; a < o.aux.size(); ++a) pltio::read_level_comp(F.infile, F.H, l, F.H.comp(o.aux[a]), in[l].comp(F.nv + (int)a));
+    }
+}
+
+// the gradient variables to the device, pa_grad, the results into out[l] components nIn .. nOut-1 (the inputs copied over
+// when out is another set)
+static void grad_gpu(const GradOpts& o, const GradFile& F, HostSet& in, HostSet& out, StagedDownloader& dl) {
+    const int Nlev = F.Nlev, nv = F.nv;
+    HierInput hi;
+    make_level_descs(F.H, Nlev, hi);
+    pa_hier* h = nullptr;
+    check(pa_hier_create(&h, Nlev, hi.lv.data(), o.is_per.data(), o.bck, 0, 1), "pa_hier_create");
+    pa_field *fin = nullptr, *fout = nullptr;
+    check(pa_field_alloc(h, nv, 1, &fin), "pa_field_alloc");
+    check(pa_field_alloc(h, 4 * nv, 0, &fout), "pa_field_alloc");
+    for (int l = 0; l < Nlev; ++l)
+        for (int v = 0; v < nv; ++v) check(pa_field_upload_level(fin, l, v, in[l].comp(v)), "upload");
+    check(pa_grad(fin, 0, nv, fout, 0), "pa_grad");
+    ensure_levels(out, Nlev);
+    long long mx = 0;
+    for (int l = 0; l < Nlev; ++l) {
+        mx = std::max(mx, F.H.levels[l].ncells());
+        if (&out != &in) {
+            out[l].alloc(F.H.levels[l].ncells(), F.nOut);
+            std::memcpy(out[l].comp(0), in[l].comp(0), (size_t)F.nIn * F.H.levels[l].ncells() * 8);
+        }
+    }
+    dl.reserve(mx);
+    for (int l = 0; l < Nlev; ++l)
+        for (int c = 0; c < 4 * nv; ++c) dl.download(fout, l, c, out[l].comp(F.nIn + c), F.H.levels[l].ncells());
+    dl.flush();
+    check(pa_sync(), "pa_sync");
+    pa_field_free(fin); pa_field_free(fout); pa_hier_destroy(h);
+}
+
+static void grad_write(const GradFile& F, const HostSet& out) {
+    std::vector<std::vector<const double*>> data(F.Nlev);
+    for (int l = 0; l < F.Nlev; ++l) for (int c = 0; c < F.nOut; ++c) data[l].push_back(out[l].comp(c));
+    std::vector<int> rr(std::max(F.Nlev - 1, 0), 2);          // the reference hard-codes refRatios = 2 (grad.cpp:255)
+    pltio::Header meta = F.H;
+    meta.time = 0.0;                                           // WriteMultiLevelPlotfile(..., 0.0, ...) (grad.cpp:256)
+    try { pltio::write_plotfile(F.outfile, meta, F.names, data, rr); } catch (std::exception& e) { pa_abort(e.what()); }
+}
+
 int main(int argc, char** argv) {
     if (argc < 2) print_usage(argv);
     ParmParse pp(argc, argv);
     if (pp.contains("help")) print_usage(argv);
+    GradOpts o;
     std::string infile, gradVar = "temp";
-    int finestLevel = 1000, verbose = 0;
-    pp.get("infile", infile);
+    int verbose = 0;
+    const bool series = pp.contains("infiles");
+    std::vector<std::string> infiles;
+    if (series) infiles = series_inputs(pp);
+    else pp.get("infile", infile);
     pp.query("gradVar", gradVar);
-    pp.query("finestLevel", finestLevel);
+    pp.query("finestLevel", o.finestLevel);
     pp.query("verbose", verbose);
 
-    pltio::Header H;
-    try { H = pltio::read_header(infile); } catch (std::exception& e) { pa_abort(std::string("cannot read plotfile: ") + e.what()); }
-    finestLevel = std::min(finestLevel, H.finest_level);
-    const int Nlev = finestLevel + 1;
-
-    std::vector<std::string> gvars;
     int ng = pp.countval("gradVars");
-    if (ng > 0) { gvars.resize(ng); for (int i = 0; i < ng; ++i) pp.get("gradVars", gvars[i], i); }
-    else gvars.push_back(gradVar);
-    for (auto& v : gvars)
-        if (H.comp(v) < 0) { std::cout << "Cannot find " << v << " data in pltfile \n"; pa_abort("Cannot find " + v + " data in pltfile"); }
-    int nAux = pp.countval("Aux_Variables");
-    std::vector<std::string> aux(nAux);
-    for (int i = 0; i < nAux; ++i) {
-        pp.get("Aux_Variables", aux[i], i);
-        if (H.comp(aux[i]) < 0) pa_abort("Unknown auxiliary variable name: " + aux[i]);
-    }
-    std::vector<int> sym_dir(3, 0), is_per(3, 1);
+    if (ng > 0) { o.gvars.resize(ng); for (int i = 0; i < ng; ++i) pp.get("gradVars", o.gvars[i], i); }
+    else o.gvars.push_back(gradVar);
+    o.aux.resize(pp.countval("Aux_Variables"));
+    for (size_t i = 0; i < o.aux.size(); ++i) pp.get("Aux_Variables", o.aux[i], (int)i);
+    std::vector<int> sym_dir(3, 0);
+    o.is_per.assign(3, 1);
     pp.queryarr("sym_dir", sym_dir, 0, 3);
-    pp.queryarr("is_per", is_per, 0, 3);
-    std::cout << "Periodicity assumed for this case: ";
-    for (int d = 0; d < 3; ++d) std::cout << is_per[d] << " ";
-    std::cout << "\n";
-
+    pp.queryarr("is_per", o.is_per, 0, 3);
+    for (int d = 0; d < 3; ++d) o.bck[d] = sym_dir[d] ? PA_BC_REFLECT_ODD : PA_BC_NEUMANN;
     int ngpus = 1;
     pp.query("ngpus", ngpus);
+
+    if (series) {
+        // every header read and checked before anything is computed or written
+        std::vector<GradFile> files;
+        for (auto& f : infiles) files.push_back(grad_file(o, f, f + ": "));
+        check_distinct_outputs(files);
+        std::cout << "Periodicity assumed for this case: ";
+        for (int d = 0; d < 3; ++d) std::cout << o.is_per[d] << " ";
+        std::cout << "\n";
+        SeriesBody<GradFile> body;
+        body.read = [&](const GradFile& F, HostSet& in) { grad_read(o, F, in, F.nIn, false); };
+        body.gpu = [&](const GradFile& F, HostSet& in, HostSet& out, StagedDownloader& dl) { grad_gpu(o, F, in, out, dl); };
+        body.write = grad_write;
+        run_series(ngpus, files, body, verbose != 0);
+        return 0;
+    }
+
+    GradFile F = grad_file(o, infile, "");
+    std::cout << "Periodicity assumed for this case: ";
+    for (int d = 0; d < 3; ++d) std::cout << o.is_per[d] << " ";
+    std::cout << "\n";
+    pp.query("outfile", F.outfile);
+
     std::string transport = "peer";
     pp.query("transport", transport);
     if (transport != "peer" && transport != "slab") pa_abort("transport must be peer or slab (got " + transport + ")");
     if (ngpus > 1) {
         GradJob J;
-        J.infile = infile; J.H = &H; J.Nlev = Nlev; J.gvars = gvars; J.aux = aux; J.is_per = is_per;
+        J.infile = infile; J.H = &F.H; J.Nlev = F.Nlev; J.gvars = o.gvars; J.aux = o.aux; J.is_per = o.is_per;
         J.peer = transport == "peer";
         J.verbose = verbose != 0;
-        for (int d = 0; d < 3; ++d) J.bck[d] = sym_dir[d] ? PA_BC_REFLECT_ODD : PA_BC_NEUMANN;
-        for (auto& v : gvars) J.names.push_back(v);
-        for (auto& a : aux) J.names.push_back(a);
-        for (auto& v : gvars) { J.names.push_back(v + "_gx"); J.names.push_back(v + "_gy"); J.names.push_back(v + "_gz"); J.names.push_back("||grad" + v + "||"); }
-        J.outfile = file_root(infile) + "_gt";
-        pp.query("outfile", J.outfile);
+        for (int d = 0; d < 3; ++d) J.bck[d] = o.bck[d];
+        J.names = F.names;
+        J.outfile = F.outfile;
         std::cout << "Writing new data to " << J.outfile << std::endl;
         run_grad_multi(ngpus, J);
         return 0;
     }
-    auto t0 = std::chrono::steady_clock::now();
     auto tnow = [] { return std::chrono::steady_clock::now(); };
     auto secs = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) { return std::chrono::duration<double>(b - a).count(); };
-    double t_init = 0, t_pin = 0, t_read = 0;
+    auto t0 = tnow();
     check(pa_init(0), "pa_init");
-    t_init = secs(t0, tnow());
-    HierInput hi;
-    make_level_descs(H, Nlev, hi);
-    int bck[3];
-    for (int d = 0; d < 3; ++d) bck[d] = sym_dir[d] ? PA_BC_REFLECT_ODD : PA_BC_NEUMANN;
-    pa_hier* h = nullptr;
-    check(pa_hier_create(&h, Nlev, hi.lv.data(), is_per.data(), bck, 0, 1), "pa_hier_create");
-    const int nv = (int)gvars.size();
-    pa_field *fin = nullptr, *fout = nullptr;
-    check(pa_field_alloc(h, nv, 1, &fin), "pa_field_alloc");
-    check(pa_field_alloc(h, 4 * nv, 0, &fout), "pa_field_alloc");
-
-    // read: gradient variables go to the device, pass-through variables stay on the host
-    const int nIn = nv + nAux, nOut = nIn + 4 * nv;
-    std::vector<PinnedLevel> buf(Nlev);
-    for (int l = 0; l < Nlev; ++l) {
-        std::cout << "Reading data for level: " << l << std::endl;
-        auto ta = tnow();
-        buf[l].alloc(H.levels[l].ncells(), nOut);
-        auto tb = tnow();
-        for (int v = 0; v < nv; ++v) {
-            pltio::read_level_comp(infile, H, l, H.comp(gvars[v]), buf[l].comp(v));
-            check(pa_field_upload_level(fin, l, v, buf[l].comp(v)), "upload");
-        }
-        for (int a = 0; a < nAux; ++a) pltio::read_level_comp(infile, H, l, H.comp(aux[a]), buf[l].comp(nv + a));
-        t_pin += secs(ta, tb); t_read += secs(tb, tnow());
-    }
-    auto t1 = std::chrono::steady_clock::now();
-    check(pa_grad(fin, 0, nv, fout, 0), "pa_grad");
+    auto t1 = tnow();
+    // one buffer set holds the inputs and receives the results
+    HostSet buf;
+    grad_read(o, F, buf, F.nOut, true);
+    auto t2 = tnow();
     {
-        long long mx = 0;
-        for (int l = 0; l < Nlev; ++l) mx = std::max(mx, H.levels[l].ncells());
-        StagedDownloader dl(mx);
-        for (int l = 0; l < Nlev; ++l)
-            for (int c = 0; c < 4 * nv; ++c) dl.download(fout, l, c, buf[l].comp(nIn + c), H.levels[l].ncells());
-        dl.flush();
+        StagedDownloader dl(0);
+        grad_gpu(o, F, buf, buf, dl);
     }
-    check(pa_sync(), "pa_sync");
-    auto t2 = std::chrono::steady_clock::now();
-
-    std::vector<std::string> names;
-    for (auto& v : gvars) names.push_back(v);
-    for (auto& a : aux) names.push_back(a);
-    for (auto& v : gvars) { names.push_back(v + "_gx"); names.push_back(v + "_gy"); names.push_back(v + "_gz"); names.push_back("||grad" + v + "||"); }
-    std::string outfile = file_root(infile) + "_gt";
-    pp.query("outfile", outfile);
-    std::cout << "Writing new data to " << outfile << std::endl;
-    std::vector<std::vector<const double*>> data(Nlev);
-    for (int l = 0; l < Nlev; ++l) for (int c = 0; c < nOut; ++c) data[l].push_back(buf[l].comp(c));
-    std::vector<int> rr(std::max(Nlev - 1, 0), 2);            // the reference hard-codes refRatios = 2 (grad.cpp:255)
-    pltio::Header meta = H;
-    meta.time = 0.0;                                           // WriteMultiLevelPlotfile(..., 0.0, ...) (grad.cpp:256)
-    try { pltio::write_plotfile(outfile, meta, names, data, rr); } catch (std::exception& e) { pa_abort(e.what()); }
     auto t3 = tnow();
-    if (verbose) {
-        auto s = [](auto a, auto b) { return std::chrono::duration<double>(b - a).count(); };
-        std::cout << "[b200] read+upload " << s(t0, t1) << " s, hot path+download " << s(t1, t2) << " s, kernels " << pa_kernel_launches() << "\n";
-        std::cout << "[b200] phases: cuda init " << t_init << " s, pinned alloc " << t_pin << " s, file read + upload " << t_read
-                  << " s, hierarchy + fields " << s(t0, t1) - t_init - t_pin - t_read << " s, plotfile write " << s(t2, t3) << " s\n";
-    }
-    pa_field_free(fin); pa_field_free(fout); pa_hier_destroy(h);
+    std::cout << "Writing new data to " << F.outfile << std::endl;
+    grad_write(F, buf);
+    auto t4 = tnow();
+    if (verbose)
+        std::cout << "[b200] phases: cuda init " << secs(t0, t1) << " s, file read " << secs(t1, t2) << " s, hierarchy + upload + hot path + download "
+                  << secs(t2, t3) << " s, plotfile write " << secs(t3, t4) << " s, kernels " << pa_kernel_launches() << "\n";
     return 0;
 }

@@ -55,17 +55,26 @@ inline void make_level_descs(const pltio::Header& h, int nlev, HierInput& out) {
 // host buffer holding [comp][level cells].  Pageable by default: measured on the B200 box (profiles/r02_tool_walltime.txt),
 // cudaHostAlloc of the tools' buffers costs 0.4 s per GB and as much again to release at exit -- more than the pinned DMA saves on
 // data that crosses PCIe once (2 GB pinned for a 50 M-cell grad run: 0.9 s to pin, against 0.2 s of slower copies).  PA_TOOL_PIN=1
-// pins them (worth it when the same buffers are reused many times).
+// pins them (worth it when the same buffers are reused many times).  alloc() keeps the memory it already holds when that is
+// large enough, so a series of plotfiles reuses one buffer per level and grows it only for a larger file.
 struct PinnedLevel {
     double* p = nullptr;
     long long ncells = 0;
     int ncomp = 0;
     bool pinned = false;
+    size_t cap = 0;                                    // bytes held
+    PinnedLevel() = default;
+    PinnedLevel(PinnedLevel&& o) noexcept : p(o.p), ncells(o.ncells), ncomp(o.ncomp), pinned(o.pinned), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+    PinnedLevel(const PinnedLevel&) = delete;
+    PinnedLevel& operator=(const PinnedLevel&) = delete;
     void alloc(long long cells, int comps) {
         ncells = cells; ncomp = comps;
+        const size_t bytes = (size_t)cells * comps * 8;
+        if (p && bytes <= cap) return;
+        release();
         const char* e = std::getenv("PA_TOOL_PIN");
         pinned = e && e[0] == '1';
-        const size_t bytes = (size_t)cells * comps * 8;
+        cap = bytes;
         if (pinned) {
             void* q = nullptr;
             check(pa_host_alloc(&q, bytes), "pa_host_alloc");
@@ -77,7 +86,9 @@ struct PinnedLevel {
         }
     }
     double* comp(int c) { return p + (long long)c * ncells; }
-    ~PinnedLevel() { if (p) { if (pinned) pa_host_free(p); else std::free(p); } }
+    const double* comp(int c) const { return p + (long long)c * ncells; }
+    void release() { if (p) { if (pinned) pa_host_free(p); else std::free(p); } p = nullptr; cap = 0; }
+    ~PinnedLevel() { release(); }
 };
 
 // Device -> pageable host memory through a pair of pinned bounce buffers: the DMA runs at full PCIe speed into pinned memory and
@@ -86,14 +97,20 @@ struct PinnedLevel {
 // costs 0.4 s per GB to pin and as much to release.  The two buffers hold one component of the largest level each.
 class StagedDownloader {
 public:
-    explicit StagedDownloader(long long max_cells) : cap_(max_cells) {
+    explicit StagedDownloader(long long max_cells) { reserve(max_cells); }
+    ~StagedDownloader() { flush(); free_buffers(); }
+    // bounce buffers for levels of up to max_cells cells: kept when they are large enough (a series reuses one downloader)
+    void reserve(long long max_cells) {
+        if (b_[0] && max_cells <= cap_) return;
+        flush();
+        free_buffers();
+        cap_ = max_cells;
         for (int i = 0; i < 2; ++i) {
             void* q = nullptr;
             check(pa_host_alloc(&q, (size_t)std::max<long long>(cap_, 1) * 8), "pa_host_alloc");
             b_[i] = (double*)q;
         }
     }
-    ~StagedDownloader() { flush(); for (int i = 0; i < 2; ++i) if (b_[i]) pa_host_free(b_[i]); }
     StagedDownloader(const StagedDownloader&) = delete;
     StagedDownloader& operator=(const StagedDownloader&) = delete;
     // queue: component `comp` of level `lev` of `f` -> dst (ncells doubles, pageable or pinned)
@@ -108,8 +125,9 @@ public:
     }
     void flush() { if (pend_dst_) copy_out(); }
 private:
+    void free_buffers() { for (int i = 0; i < 2; ++i) if (b_[i]) { pa_host_free(b_[i]); b_[i] = nullptr; } }
     void copy_out() { std::memcpy(pend_dst_, pend_src_, (size_t)pend_n_ * 8); pend_dst_ = nullptr; }
-    long long cap_;
+    long long cap_ = 0;
     double* b_[2] = {nullptr, nullptr};
     double* pend_dst_ = nullptr;
     const double* pend_src_ = nullptr;

@@ -8,6 +8,12 @@
     python -m peleanalysis_b200.mgtools filter    infile=plt00100 [variables=a b] [max_filter_level=N] [filter_type=1] [base_fgr=2]
                                                   [same_fgr_all_levels=0] [max_grid_size=32] [interp_type=1]
     python -m torch.distributed.run --nproc-per-node 8 -m peleanalysis_b200.mgtools grad infile=... [transport=peer|slab]
+    python -m torch.distributed.run --nproc-per-node 8 -m peleanalysis_b200.mgtools grad infiles=plt00100 plt00200 ... [keys]
+
+infiles= processes a series of plotfiles in one process per rank, so `import torch` and the CUDA context are paid once: at
+world size W, rank r takes files r, r+W, ... and runs each as the world-size-1 run of that file on its own GPU (do_smooth
+included), with no communication except a final barrier.  Every other key applies to each file; each output has the name a
+single run writes by default.  infiles cannot be combined with infile, outfile or transport.
 
 Same keys, same output variable names and the same plotfile format as R/Src/grad.cpp / curvature.cpp / filterPlt.cpp (and
 as the C++ shells in host/).  filter spreads the boxes re-chopped to max_grid_size over the ranks; the FillPatch sources of
@@ -93,11 +99,12 @@ def read_boxes(path: str, hd, lev: int, meta, box_ids: Sequence[int], comp_ids: 
 
 
 class _Dist:
-    """torch.distributed if this is a multi-process run (RANK / WORLD_SIZE from torchrun), else a single rank."""
+    """torch.distributed if this is a multi-process run (RANK / WORLD_SIZE from torchrun), else a single rank.  solo=True: one
+    rank of world size 1 whatever the environment (one file of a series)."""
 
-    def __init__(self, backend: str, device: int):
-        self.rank = int(os.environ.get("RANK", "0"))
-        self.world = int(os.environ.get("WORLD_SIZE", "1"))
+    def __init__(self, backend: str, device: int, solo: bool = False):
+        self.rank = 0 if solo else int(os.environ.get("RANK", "0"))
+        self.world = 1 if solo else int(os.environ.get("WORLD_SIZE", "1"))
         self.dist = None
         self.own_group = False
         if self.world > 1:
@@ -137,10 +144,48 @@ def run(tool: str, argv: Sequence[str], capi=None, multigpu=None, wrap=None, bac
         from . import capi as _capi
         capi = _capi
     pp = parse_args(argv)
+    if "infiles" in pp and tool in ("grad", "curvature", "filter"):
+        return _series(tool, pp, capi, backend, device)
     if tool not in ("grad", "curvature", "filter") or "infile" not in pp:
         raise SystemExit(__doc__)
     dev = device if device is not None else int(os.environ.get("LOCAL_RANK", "0"))
+    return _run_one(tool, pp, capi, multigpu, wrap, backend, dev, _Dist(backend, dev))
+
+
+def _series(tool: str, pp, capi, backend: str, device: int | None) -> str:
+    """infiles=: this rank's files of the list, each as a world-size-1 run; returns the last output of this rank ('' if none)."""
+    infiles = pp.pop("infiles")
+    if not infiles:
+        raise SystemExit("amrex::Abort::0::infiles needs at least one plotfile !!!")
+    for k in ("infile", "outfile", "transport"):
+        if k in pp:
+            raise SystemExit("amrex::Abort::0::infiles cannot be combined with %s (each file's output has its default name) !!!" % k)
+    suffix = {"grad": "_gt", "curvature": "_K", "filter": "_filtered"}[tool]
+    seen = {}
+    for f in infiles:                                          # before anything is computed: one output name per input
+        out = file_root(f) + suffix
+        if out in seen:
+            raise SystemExit("amrex::Abort::0::infiles: %s and %s both write %s !!!" % (seen[out], f, out))
+        seen[out] = f
+        try:
+            plotfile.read_header(f)
+        except Exception as e:                                 # noqa: BLE001  (any unreadable header stops the run up front)
+            raise SystemExit("amrex::Abort::0::%s: cannot read plotfile: %s !!!" % (f, e))
+    dev = device if device is not None else int(os.environ.get("LOCAL_RANK", "0"))
     D = _Dist(backend, dev)
+    out = ""
+    try:
+        for f in infiles[D.rank::D.world]:
+            one = dict(pp)
+            one["infile"] = [f]
+            out = _run_one(tool, one, capi, None, None, backend, dev, _Dist(backend, dev, solo=True))
+    finally:
+        D.barrier()
+        D.close()
+    return out
+
+
+def _run_one(tool: str, pp, capi, multigpu, wrap, backend: str, dev: int, D: "_Dist") -> str:
     if multigpu is None and D.world > 1:
         from . import multigpu as _mg
         multigpu = _mg
