@@ -22,7 +22,7 @@ struct CurvKeys {                                      // the keys every file of
 
 struct CurvFile {                                      // one plotfile, checked: its inputs, output slots and names
     std::string infile, outfile;
-    pltio::Header H;
+    pltio::Header H, meta;                             // the plotfile; the output's header (time 0)
     int Nlev = 0;
     std::vector<std::string> inNames, velNames{"x_velocity", "y_velocity", "z_velocity"}, names;
     bool need_vel = false;
@@ -105,40 +105,45 @@ static CurvFile curv_file(const CurvKeys& k, const std::string& infile, const st
     if (!k.do_smooth) F.zero_slots.push_back(idSmProg);
     if (!k.do_gaussCurv) F.zero_slots.push_back(idKg);
     if (k.getStrainTensor && !k.do_strain) for (int i = 0; i < 9; ++i) F.zero_slots.push_back(idROST + i);
+    F.meta = H;
+    F.meta.time = 0.0;
     return F;
 }
 
-// disk -> in[l]: components 0 .. nCompIn-1 the pass-through inputs (progress variable first); with velocities, the last three
-// of the ncomp (+ 3) allocated components
-static void curv_read(const CurvFile& F, HostSet& in, int ncomp, bool talk) {
+// disk -> in[l] of the rank's boxes: components 0 .. nCompIn-1 the pass-through inputs (progress variable first); in_place:
+// room for the results as well; with velocities, three more components last
+static void curv_read(const CurvFile& F, const RankCtx& R, HostSet& in, bool in_place, bool talk) {
     ensure_levels(in, F.Nlev);
-    const int nalloc = ncomp + (F.need_vel ? 3 : 0);
+    const int nalloc = (in_place ? F.nCompOut : F.nCompIn) + (F.need_vel ? 3 : 0);
     for (int l = 0; l < F.Nlev; ++l) {
         if (talk) std::cout << "Reading data for level " << l << "\n";
-        in[l].alloc(F.H.levels[l].ncells(), nalloc);
-        for (int c = 0; c < F.nCompIn; ++c) pltio::read_level_comp(F.infile, F.H, l, F.H.comp(F.inNames[c]), in[l].comp(c));
+        in[l].alloc(R.cells(F.H, l), nalloc);
+        for (int c = 0; c < F.nCompIn; ++c) pltio::read_boxes_comp(F.infile, F.H, l, F.H.comp(F.inNames[c]), R.mine[l], in[l].comp(c));
         if (F.need_vel)
-            for (int d = 0; d < 3; ++d) pltio::read_level_comp(F.infile, F.H, l, F.H.comp(F.velNames[d]), in[l].comp(nalloc - 3 + d));
+            for (int d = 0; d < 3; ++d) pltio::read_boxes_comp(F.infile, F.H, l, F.H.comp(F.velNames[d]), R.mine[l], in[l].comp(nalloc - 3 + d));
     }
 }
 
-static void curv_gpu(const CurvKeys& k, const CurvFile& F, HostSet& in, HostSet& out, StagedDownloader& dl, bool talk) {
+static void curv_gpu(const CurvKeys& k, const CurvFile& F, const RankCtx& R, HostSet& in, HostSet& out, StagedDownloader& dl, bool talk) {
     const int Nlev = F.Nlev, nres = F.nres;
-    HierInput hi;
-    make_level_descs(F.H, Nlev, hi);
-    pa_hier* h = nullptr;
-    check(pa_hier_create(&h, Nlev, hi.lv.data(), k.is_per.data(), k.bck, 0, 1), "pa_hier_create");
-    pa_field *st = nullptr, *res = nullptr;
+    pa_hier* h = R.hier(F.H, Nlev, k.is_per.data(), k.bck, 0);
+    pa_field *st = nullptr, *res = nullptr, *scratch = nullptr;
     // do_smooth: two more state components, c and the smoothed phi, which the curvature then reads as its scalar
     const int nst = F.need_vel ? 4 : 1, comp_c = nst, comp_phi = nst + 1;
     check(pa_field_alloc(h, k.do_smooth ? nst + 2 : nst, 1, &st), "pa_field_alloc");
     check(pa_field_alloc(h, nres, 1, &res), "pa_field_alloc");
+    if (F.o.do_gauss) check(pa_curvature_scratch(h, 0, &scratch), "pa_curvature_scratch");
     for (int l = 0; l < Nlev; ++l) {
         check(pa_field_upload_level(st, l, 0, in[l].comp(0)), "upload");
         if (F.need_vel)
             for (int d = 0; d < 3; ++d) check(pa_field_upload_level(st, l, 1 + d, in[l].comp(in[l].ncomp - 3 + d)), "upload");
     }
+    std::vector<pa_field*> fields{st, res};
+    if (scratch) fields.push_back(scratch);
+    R.map_peers(Nlev, fields);
     std::vector<int> slot = F.slot;
+    pa_curv_opts o = F.o;
+    int comp_S = 0;
     if (k.do_smooth) {
         pa_smooth_opts so{};
         so.smoothing_time = k.smooth_time;
@@ -150,17 +155,39 @@ static void curv_gpu(const CurvKeys& k, const CurvFile& F, HostSet& in, HostSet&
                             << " iterations, max|c - A phi| / max|c| = " << resid << "\n";
         // the curvature of phi with the identity normalisation (curvature.cpp:328-406 hands the solution on as the progress
         // variable); its Progress output is phi itself and goes to SmoothedProgress, Progress is c
-        pa_curv_opts os = F.o;
-        os.prog_min = 0.0; os.prog_max = 1.0;
+        o.prog_min = 0.0; o.prog_max = 1.0;
         slot[0] = F.idSmProg;
-        check(pa_curvature(st, comp_phi, 1, &os, res, 0), "pa_curvature");
-    } else {
-        check(pa_curvature(st, 0, 1, &F.o, res, 0), "pa_curvature");
+        comp_S = comp_phi;
     }
+    // the steps of pa_curvature, each behind the cross-rank step it needs
+    auto step = [&](int steps, int lev) { check(pa_curvature_steps(st, comp_S, 1, &o, res, 0, steps, lev, lev), "pa_curvature"); };
+    R.exchange(st, comp_S, 1);
+    step(PA_CURV_PASS1, -1);
+    if (o.do_threshold) {
+        for (int l = 0; l < Nlev; ++l) {
+            R.exchange(res, 2, 3);
+            step(PA_CURV_DIV, l);
+            // the clip zeroes n(l) in place; with peer links every rank's DIV(l) reads its peers' UNCLIPPED n(l) over the links
+            // first (curvature.cpp:487-567: FillBoundary of n precedes the clip).  With transport=slab the peers' cells of n(l)
+            // were copied inside the exchange, which ends in a barrier: nothing reads n(l) in place.
+            if (R.peer_links) {
+                check(pa_sync(), "pa_sync");
+                R.barrier();
+            }
+            step(PA_CURV_CLIP, l);
+        }
+    } else {
+        R.exchange(res, 2, 3);
+        step(PA_CURV_DIV, -1);
+    }
+    if (o.do_gauss) { R.exchange(scratch, 0, 3); step(PA_CURV_GAUSS, -1); }
+    if (o.do_strain) { R.exchange(st, 1, 3); step(PA_CURV_STRAIN, -1); }
+    if (o.do_velnormal) step(PA_CURV_VELN, -1);
+
     ensure_levels(out, Nlev);
     long long mx = 0;
     for (int l = 0; l < Nlev; ++l) {
-        const long long nc = F.H.levels[l].ncells();
+        const long long nc = in[l].ncells;
         mx = std::max(mx, nc);
         if (&out != &in) {
             out[l].alloc(nc, F.nCompOut);
@@ -176,16 +203,8 @@ static void curv_gpu(const CurvKeys& k, const CurvFile& F, HostSet& in, HostSet&
     }
     dl.flush();
     check(pa_sync(), "pa_sync");
+    R.barrier();                                       // nobody frees a slab a peer may still be reading
     pa_field_free(st); pa_field_free(res); pa_hier_destroy(h);
-}
-
-static void curv_write(const CurvFile& F, const HostSet& out) {
-    std::vector<std::vector<const double*>> data(F.Nlev);
-    for (int l = 0; l < F.Nlev; ++l) for (int c = 0; c < F.nCompOut; ++c) data[l].push_back(out[l].comp(c));
-    std::vector<int> rr(std::max(F.Nlev - 1, 0), 2);          // curvature.cpp:842
-    pltio::Header meta = F.H;
-    meta.time = 0.0;
-    try { pltio::write_plotfile(F.outfile, meta, F.names, data, rr); } catch (std::exception& e) { pa_abort(e.what()); }
 }
 
 int main(int argc, char** argv) {
@@ -225,15 +244,16 @@ int main(int argc, char** argv) {
     int ngpus = 1;
     pp.query("ngpus", ngpus);
 
+    // the threads of ngpus=N and the files of a series print no progress lines
+    ToolBody<CurvFile> body;
+    body.read = [&](const CurvFile& F, const RankCtx& R, HostSet& in, bool in_place) { curv_read(F, R, in, in_place, false); };
+    body.gpu = [&](const CurvFile& F, const RankCtx& R, HostSet& in, HostSet& out, StagedDownloader& dl) { curv_gpu(k, F, R, in, out, dl, false); };
+
     if (series) {
         // every header read and checked before anything is computed or written; each file runs on one GPU, so do_smooth too
         std::vector<CurvFile> files;
         for (auto& f : infiles) files.push_back(curv_file(k, f, f + ": ", false));
         check_distinct_outputs(files);
-        SeriesBody<CurvFile> body;
-        body.read = [&](const CurvFile& F, HostSet& in) { curv_read(F, in, F.nCompIn, false); };
-        body.gpu = [&](const CurvFile& F, HostSet& in, HostSet& out, StagedDownloader& dl) { curv_gpu(k, F, in, out, dl, false); };
-        body.write = curv_write;
         run_series(ngpus, files, body, verbose != 0);
         return 0;
     }
@@ -250,27 +270,21 @@ int main(int argc, char** argv) {
     if (ngpus > 1 && k.do_smooth)
         pa_abort("do_smooth=1 runs on one GPU only: the smoothing solve has no multi-GPU path (use ngpus=1)");
     if (ngpus > 1) {
-        CurvJob J;
-        J.peer = transport == "peer";
-        J.verbose = verbose != 0;
-        J.infile = plotFileName; J.outfile = F.outfile; J.H = &F.H; J.Nlev = F.Nlev;
-        J.inNames = F.inNames; J.velNames = F.velNames; J.names = F.names; J.need_vel = F.need_vel; J.o = F.o;
-        J.slot = F.slot; J.zero_slots = F.zero_slots; J.nCompOut = F.nCompOut; J.is_per = k.is_per;
-        for (int d = 0; d < 3; ++d) J.bck[d] = k.bck[d];
         std::cout << "Writing new data to " << F.outfile << "\n";
-        run_curv_multi(ngpus, J);
+        run_ranks(ngpus, F, body, transport == "peer", verbose != 0);
         return 0;
     }
 
     check(pa_init(0), "pa_init");
+    const RankCtx R(F.meta, F.Nlev);
     // one buffer set holds the inputs and receives the results
     HostSet buf;
-    curv_read(F, buf, F.nCompOut, verbose != 0);
+    curv_read(F, R, buf, true, verbose != 0);
     {
         StagedDownloader dl(0);
-        curv_gpu(k, F, buf, buf, dl, verbose != 0);
+        curv_gpu(k, F, R, buf, buf, dl, verbose != 0);
     }
     std::cout << "Writing new data to " << F.outfile << "\n";
-    curv_write(F, buf);
+    R.write(F, buf);
     return 0;
 }

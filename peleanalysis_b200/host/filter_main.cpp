@@ -36,8 +36,7 @@ struct FilterFile {                                    // one plotfile, checked,
     std::string infile, outfile;
     pltio::Header H;                                   // the plotfile
     pltio::Header meta;                                // its grids re-chopped to max_grid_size (the output's boxes)
-    std::vector<std::vector<std::vector<pltio::BoxI>>> chunks;   // [level][original box] -> its chunks
-    std::vector<std::vector<int>> parent;              // [level][chunk] -> original box
+    std::vector<std::vector<int>> parent;              // [level][chunk] -> original box (ascending)
     int Nlev = 0, ngmax = 0;
     std::vector<int> fgr, ngrow;
     std::vector<std::string> names;
@@ -61,7 +60,7 @@ static FilterFile filter_file(const FilterKeys& k, const std::string& infile, co
     // filter-to-grid ratio and ghost width of every level (filterPlt.cpp:138-148), grids re-chopped to max_grid_size (:153)
     F.fgr.resize(Nlev); F.ngrow.resize(Nlev);
     F.meta = H;
-    F.chunks.resize(Nlev); F.parent.resize(Nlev);
+    F.parent.resize(Nlev);
     int fgr_lev = k.base_fgr;
     for (int l = 0; l < Nlev; ++l) {
         if (!k.same_fgr && l > 0) {
@@ -73,7 +72,6 @@ static FilterFile filter_file(const FilterKeys& k, const std::string& infile, co
         if (nw < 0) pa_abort(who + std::string("filter weights: ") + pa_last_error());
         F.ngmax = std::max(F.ngmax, F.ngrow[l]);
         F.meta.levels[l].boxes.clear();
-        F.chunks[l].resize(H.levels[l].boxes.size());
         for (size_t b = 0; b < H.levels[l].boxes.size(); ++b) {
             const pltio::BoxI& B = H.levels[l].boxes[b];
             int one[6] = {B.lo[0], B.lo[1], B.lo[2], B.hi[0], B.hi[1], B.hi[2]};
@@ -84,7 +82,6 @@ static FilterFile filter_file(const FilterKeys& k, const std::string& infile, co
             for (int c = 0; c < n; ++c) {
                 pltio::BoxI C;
                 for (int d = 0; d < 3; ++d) { C.lo[d] = out[6 * c + d]; C.hi[d] = out[6 * c + 3 + d]; }
-                F.chunks[l][b].push_back(C);
                 F.meta.levels[l].boxes.push_back(C);
                 F.parent[l].push_back((int)b);
             }
@@ -93,8 +90,8 @@ static FilterFile filter_file(const FilterKeys& k, const std::string& infile, co
     return F;
 }
 
-// disk -> in[l], every variable cut into the output boxes
-static void filter_read(const FilterFile& F, HostSet& in, bool talk) {
+// disk -> in[l], every variable on the rank's output boxes, cut from the plotfile boxes they lie in (only those are read)
+static void filter_read(const FilterFile& F, const RankCtx& R, HostSet& in, bool talk) {
     const pltio::Header& H = F.H;
     const int ncomp = (int)F.names.size();
     ensure_levels(in, F.Nlev);
@@ -102,18 +99,27 @@ static void filter_read(const FilterFile& F, HostSet& in, bool talk) {
     std::vector<double> tmp;
     for (int l = 0; l < F.Nlev; ++l) {
         if (talk) std::cout << "on level " << l << std::endl;
-        const long long nc = H.levels[l].ncells();
-        in[l].alloc(nc, ncomp);
-        tmp.resize((size_t)nc);
+        const std::vector<int>& mine = R.mine[l];
+        std::vector<int> parents;                      // chunk ids ascend with their parent's
+        long long np = 0;
+        for (int c : mine)
+            if (parents.empty() || parents.back() != F.parent[l][c]) {
+                parents.push_back(F.parent[l][c]);
+                np += H.levels[l].boxes[parents.back()].npts();
+            }
+        in[l].alloc(R.cells(F.meta, l), ncomp);
+        tmp.resize((size_t)np);
         for (int v = 0; v < ncomp; ++v) {
-            pltio::read_level_comp(F.infile, H, l, H.comp(F.names[v]), tmp.data());
-            // the plotfile's FABs cut into the output boxes: each original box becomes its chunks, in place
+            pltio::read_boxes_comp(F.infile, H, l, H.comp(F.names[v]), parents, tmp.data());
+            // each plotfile box becomes the rank's chunks of it, in place
             const double* src = tmp.data();
             double* dst = in[l].comp(v);
-            for (size_t b = 0; b < H.levels[l].boxes.size(); ++b) {
-                const pltio::BoxI& B = H.levels[l].boxes[b];
+            size_t i = 0;
+            for (int pb : parents) {
+                const pltio::BoxI& B = H.levels[l].boxes[pb];
                 const long long nx = B.hi[0] - B.lo[0] + 1, ny = B.hi[1] - B.lo[1] + 1;
-                for (const pltio::BoxI& C : F.chunks[l][b]) {
+                for (; i < mine.size() && F.parent[l][mine[i]] == pb; ++i) {
+                    const pltio::BoxI& C = F.meta.levels[l].boxes[mine[i]];
                     const int cx = C.hi[0] - C.lo[0] + 1;
                     for (int kk = C.lo[2]; kk <= C.hi[2]; ++kk)
                         for (int j = C.lo[1]; j <= C.hi[1]; ++j) {
@@ -127,24 +133,23 @@ static void filter_read(const FilterFile& F, HostSet& in, bool talk) {
     }
 }
 
-static void filter_gpu(const FilterKeys& k, const FilterFile& F, HostSet& in, HostSet& out, StagedDownloader& dl, bool talk) {
+static void filter_gpu(const FilterKeys& k, const FilterFile& F, const RankCtx& R, HostSet& in, HostSet& out, StagedDownloader& dl, bool talk) {
     const int Nlev = F.Nlev, ncomp = (int)F.names.size();
-    HierInput hi;
-    make_level_descs(F.meta, Nlev, hi);
     const int no_per[3] = {0, 0, 0}, bck[3] = {PA_BC_NEUMANN, PA_BC_NEUMANN, PA_BC_NEUMANN};   // PltFileManager.cpp:118-120: never periodic
-    pa_hier* h = nullptr;
-    check(pa_hier_create2(&h, Nlev, hi.lv.data(), no_per, bck, 0, 1, PA_HIER_FILTER_ONLY), "pa_hier_create");
+    pa_hier* h = R.hier(F.meta, Nlev, no_per, bck, PA_HIER_FILTER_ONLY);
     pa_field *fin = nullptr, *fout = nullptr;
     check(pa_field_alloc(h, ncomp, F.ngmax, &fin), "pa_field_alloc");
     check(pa_field_alloc(h, ncomp, 0, &fout), "pa_field_alloc");
     for (int l = 0; l < Nlev; ++l)
         for (int v = 0; v < ncomp; ++v) check(pa_field_upload_level(fin, l, v, in[l].comp(v)), "upload");
     check(pa_sync(), "pa_sync");
+    R.barrier();
     if (talk) std::cout << "Done!" << std::endl;
 
     if (talk) std::cout << "FillPatching data..." << std::endl;
     for (int l = 0; l < Nlev; ++l) {
         if (talk) std::cout << "on level " << l << std::endl;
+        R.fill_patch_exchange(fin, ncomp, l, F.ngrow[l], k.interp_type);
         check(pa_fill_patch(fin, 0, ncomp, l, F.ngrow[l], k.interp_type), "pa_fill_patch");
     }
     if (talk) std::cout << "Done!" << std::endl;
@@ -164,15 +169,10 @@ static void filter_gpu(const FilterKeys& k, const FilterFile& F, HostSet& in, Ho
         for (int c = 0; c < ncomp; ++c) dl.download(fout, l, c, out[l].comp(c), out[l].ncells);
     dl.flush();
     check(pa_sync(), "pa_sync");
+    R.barrier();                                       // nobody frees a send slab a peer may still be reading
     if (talk) std::cout << "Done!" << std::endl;
+    if (talk) std::cout << "Saving filtered data..." << std::endl;      // the plotfile write follows
     pa_field_free(fin); pa_field_free(fout); pa_hier_destroy(h);
-}
-
-static void filter_write(const FilterFile& F, const HostSet& out) {
-    std::vector<std::vector<const double*>> data(F.Nlev);
-    for (int l = 0; l < F.Nlev; ++l) for (size_t c = 0; c < F.names.size(); ++c) data[l].push_back(out[l].comp((int)c));
-    std::vector<int> rr(std::max(F.Nlev - 1, 0), 2);          // write_plotfile hard-codes ref_ratio 2 (filterPlt.cpp:50)
-    try { pltio::write_plotfile(F.outfile, F.meta, F.names, data, rr); } catch (std::exception& e) { pa_abort(e.what()); }
 }
 
 int main(int argc, char** argv) {
@@ -199,15 +199,17 @@ int main(int argc, char** argv) {
     k.variables.resize(pp.countval("variables"));
     for (size_t i = 0; i < k.variables.size(); ++i) pp.get("variables", k.variables[i], (int)i);
 
+    // progress lines in a single run and from rank 0 of ngpus=N; a series prints none
+    const bool talk = !series;
+    ToolBody<FilterFile> body;
+    body.read = [&](const FilterFile& F, const RankCtx& R, HostSet& in, bool) { filter_read(F, R, in, talk && R.r == 0); };
+    body.gpu = [&](const FilterFile& F, const RankCtx& R, HostSet& in, HostSet& out, StagedDownloader& dl) { filter_gpu(k, F, R, in, out, dl, talk && R.r == 0); };
+
     if (series) {
         // every header read and checked before anything is computed or written; each file runs on one GPU
         std::vector<FilterFile> files;
         for (auto& f : infiles) files.push_back(filter_file(k, f, f + ": "));
         check_distinct_outputs(files);
-        SeriesBody<FilterFile> body;
-        body.read = [&](const FilterFile& F, HostSet& in) { filter_read(F, in, false); };
-        body.gpu = [&](const FilterFile& F, HostSet& in, HostSet& out, StagedDownloader& dl) { filter_gpu(k, F, in, out, dl, false); };
-        body.write = filter_write;
         run_series(ngpus, files, body, verbose != 0);
         return 0;
     }
@@ -216,24 +218,22 @@ int main(int argc, char** argv) {
     auto t0 = std::chrono::steady_clock::now();
     check(pa_init(0), "pa_init");
     if (ngpus > 1) {
-        FilterJob J;
-        J.infile = infile; J.outfile = F.outfile; J.H = &F.H; J.meta = &F.meta; J.parent = F.parent; J.Nlev = F.Nlev;
-        J.filter_type = k.filter_type; J.interp_type = k.interp_type; J.ngmax = F.ngmax; J.fgr = F.fgr; J.ngrow = F.ngrow; J.names = F.names;
-        run_filter_multi(ngpus, J);
+        run_ranks(ngpus, F, body, false, false);
+        std::cout << "Done!" << std::endl;
         return 0;
     }
+    const RankCtx R(F.meta, F.Nlev);
     // one buffer set holds the inputs and receives the results
     HostSet buf;
-    filter_read(F, buf, true);
+    body.read(F, R, buf, true);
     auto t1 = std::chrono::steady_clock::now();
     {
         StagedDownloader dl(0);
-        filter_gpu(k, F, buf, buf, dl, true);
+        body.gpu(F, R, buf, buf, dl);
     }
     auto t2 = std::chrono::steady_clock::now();
 
-    std::cout << "Saving filtered data..." << std::endl;
-    filter_write(F, buf);
+    R.write(F, buf);
     std::cout << "Done!" << std::endl;
     if (verbose) {
         auto s = [](auto a, auto b) { return std::chrono::duration<double>(b - a).count(); };

@@ -27,7 +27,7 @@ struct GradOpts {                                      // the keys every file of
 
 struct GradFile {                                      // one plotfile, checked
     std::string infile, outfile;
-    pltio::Header H;
+    pltio::Header H, meta;                             // the plotfile; the output's header (time 0, grad.cpp:256)
     int Nlev = 0;
     std::vector<std::string> names;
     int nv = 0, nIn = 0, nOut = 0;
@@ -50,58 +50,53 @@ static GradFile grad_file(const GradOpts& o, const std::string& infile, const st
     for (auto& a : o.aux) F.names.push_back(a);
     for (auto& v : o.gvars) { F.names.push_back(v + "_gx"); F.names.push_back(v + "_gy"); F.names.push_back(v + "_gz"); F.names.push_back("||grad" + v + "||"); }
     F.outfile = file_root(infile) + "_gt";
+    F.meta = F.H;
+    F.meta.time = 0.0;                                 // WriteMultiLevelPlotfile(..., 0.0, ...) (grad.cpp:256)
     return F;
 }
 
-// disk -> in[l] components 0 .. nIn-1 (gradient variables, then pass-through variables); ncomp = the components to allocate
-static void grad_read(const GradOpts& o, const GradFile& F, HostSet& in, int ncomp, bool talk) {
+// disk -> in[l] components 0 .. nIn-1 (gradient variables, then pass-through variables) of the rank's boxes; in_place: room
+// for the results as well
+static void grad_read(const GradOpts& o, const GradFile& F, const RankCtx& R, HostSet& in, bool in_place, bool talk) {
     ensure_levels(in, F.Nlev);
     for (int l = 0; l < F.Nlev; ++l) {
         if (talk) std::cout << "Reading data for level: " << l << std::endl;
-        in[l].alloc(F.H.levels[l].ncells(), ncomp);
-        for (int v = 0; v < F.nv; ++v) pltio::read_level_comp(F.infile, F.H, l, F.H.comp(o.gvars[v]), in[l].comp(v));
-        for (size_t a = 0; a < o.aux.size(); ++a) pltio::read_level_comp(F.infile, F.H, l, F.H.comp(o.aux[a]), in[l].comp(F.nv + (int)a));
+        in[l].alloc(R.cells(F.H, l), in_place ? F.nOut : F.nIn);
+        for (int v = 0; v < F.nv; ++v) pltio::read_boxes_comp(F.infile, F.H, l, F.H.comp(o.gvars[v]), R.mine[l], in[l].comp(v));
+        for (size_t a = 0; a < o.aux.size(); ++a) pltio::read_boxes_comp(F.infile, F.H, l, F.H.comp(o.aux[a]), R.mine[l], in[l].comp(F.nv + (int)a));
     }
 }
 
 // the gradient variables to the device, pa_grad, the results into out[l] components nIn .. nOut-1 (the inputs copied over
 // when out is another set)
-static void grad_gpu(const GradOpts& o, const GradFile& F, HostSet& in, HostSet& out, StagedDownloader& dl) {
+static void grad_gpu(const GradOpts& o, const GradFile& F, const RankCtx& R, HostSet& in, HostSet& out, StagedDownloader& dl) {
     const int Nlev = F.Nlev, nv = F.nv;
-    HierInput hi;
-    make_level_descs(F.H, Nlev, hi);
-    pa_hier* h = nullptr;
-    check(pa_hier_create(&h, Nlev, hi.lv.data(), o.is_per.data(), o.bck, 0, 1), "pa_hier_create");
+    pa_hier* h = R.hier(F.H, Nlev, o.is_per.data(), o.bck, 0);
     pa_field *fin = nullptr, *fout = nullptr;
     check(pa_field_alloc(h, nv, 1, &fin), "pa_field_alloc");
     check(pa_field_alloc(h, 4 * nv, 0, &fout), "pa_field_alloc");
     for (int l = 0; l < Nlev; ++l)
         for (int v = 0; v < nv; ++v) check(pa_field_upload_level(fin, l, v, in[l].comp(v)), "upload");
+    R.map_peers(Nlev, {fin});
+    R.exchange(fin, 0, nv);
     check(pa_grad(fin, 0, nv, fout, 0), "pa_grad");
     ensure_levels(out, Nlev);
     long long mx = 0;
     for (int l = 0; l < Nlev; ++l) {
-        mx = std::max(mx, F.H.levels[l].ncells());
+        const long long nc = in[l].ncells;
+        mx = std::max(mx, nc);
         if (&out != &in) {
-            out[l].alloc(F.H.levels[l].ncells(), F.nOut);
-            std::memcpy(out[l].comp(0), in[l].comp(0), (size_t)F.nIn * F.H.levels[l].ncells() * 8);
+            out[l].alloc(nc, F.nOut);
+            std::memcpy(out[l].comp(0), in[l].comp(0), (size_t)F.nIn * nc * 8);
         }
     }
     dl.reserve(mx);
     for (int l = 0; l < Nlev; ++l)
-        for (int c = 0; c < 4 * nv; ++c) dl.download(fout, l, c, out[l].comp(F.nIn + c), F.H.levels[l].ncells());
+        for (int c = 0; c < 4 * nv; ++c) dl.download(fout, l, c, out[l].comp(F.nIn + c), out[l].ncells);
     dl.flush();
     check(pa_sync(), "pa_sync");
+    R.barrier();                                       // nobody frees a slab (or send slab) a peer may still be reading
     pa_field_free(fin); pa_field_free(fout); pa_hier_destroy(h);
-}
-
-static void grad_write(const GradFile& F, const HostSet& out) {
-    std::vector<std::vector<const double*>> data(F.Nlev);
-    for (int l = 0; l < F.Nlev; ++l) for (int c = 0; c < F.nOut; ++c) data[l].push_back(out[l].comp(c));
-    std::vector<int> rr(std::max(F.Nlev - 1, 0), 2);          // the reference hard-codes refRatios = 2 (grad.cpp:255)
-    pltio::Header meta = F.H;
-    meta.time = 0.0;                                           // WriteMultiLevelPlotfile(..., 0.0, ...) (grad.cpp:256)
-    try { pltio::write_plotfile(F.outfile, meta, F.names, data, rr); } catch (std::exception& e) { pa_abort(e.what()); }
 }
 
 int main(int argc, char** argv) {
@@ -132,6 +127,11 @@ int main(int argc, char** argv) {
     int ngpus = 1;
     pp.query("ngpus", ngpus);
 
+    // the threads of ngpus=N and the files of a series print no progress lines
+    ToolBody<GradFile> body;
+    body.read = [&](const GradFile& F, const RankCtx& R, HostSet& in, bool in_place) { grad_read(o, F, R, in, in_place, false); };
+    body.gpu = [&](const GradFile& F, const RankCtx& R, HostSet& in, HostSet& out, StagedDownloader& dl) { grad_gpu(o, F, R, in, out, dl); };
+
     if (series) {
         // every header read and checked before anything is computed or written
         std::vector<GradFile> files;
@@ -140,10 +140,6 @@ int main(int argc, char** argv) {
         std::cout << "Periodicity assumed for this case: ";
         for (int d = 0; d < 3; ++d) std::cout << o.is_per[d] << " ";
         std::cout << "\n";
-        SeriesBody<GradFile> body;
-        body.read = [&](const GradFile& F, HostSet& in) { grad_read(o, F, in, F.nIn, false); };
-        body.gpu = [&](const GradFile& F, HostSet& in, HostSet& out, StagedDownloader& dl) { grad_gpu(o, F, in, out, dl); };
-        body.write = grad_write;
         run_series(ngpus, files, body, verbose != 0);
         return 0;
     }
@@ -158,15 +154,8 @@ int main(int argc, char** argv) {
     pp.query("transport", transport);
     if (transport != "peer" && transport != "slab") pa_abort("transport must be peer or slab (got " + transport + ")");
     if (ngpus > 1) {
-        GradJob J;
-        J.infile = infile; J.H = &F.H; J.Nlev = F.Nlev; J.gvars = o.gvars; J.aux = o.aux; J.is_per = o.is_per;
-        J.peer = transport == "peer";
-        J.verbose = verbose != 0;
-        for (int d = 0; d < 3; ++d) J.bck[d] = o.bck[d];
-        J.names = F.names;
-        J.outfile = F.outfile;
-        std::cout << "Writing new data to " << J.outfile << std::endl;
-        run_grad_multi(ngpus, J);
+        std::cout << "Writing new data to " << F.outfile << std::endl;
+        run_ranks(ngpus, F, body, transport == "peer", verbose != 0);
         return 0;
     }
     auto tnow = [] { return std::chrono::steady_clock::now(); };
@@ -174,17 +163,18 @@ int main(int argc, char** argv) {
     auto t0 = tnow();
     check(pa_init(0), "pa_init");
     auto t1 = tnow();
+    const RankCtx R(F.meta, F.Nlev);
     // one buffer set holds the inputs and receives the results
     HostSet buf;
-    grad_read(o, F, buf, F.nOut, true);
+    grad_read(o, F, R, buf, true, true);
     auto t2 = tnow();
     {
         StagedDownloader dl(0);
-        grad_gpu(o, F, buf, buf, dl);
+        grad_gpu(o, F, R, buf, buf, dl);
     }
     auto t3 = tnow();
     std::cout << "Writing new data to " << F.outfile << std::endl;
-    grad_write(F, buf);
+    R.write(F, buf);
     auto t4 = tnow();
     if (verbose)
         std::cout << "[b200] phases: cuda init " << secs(t0, t1) << " s, file read " << secs(t1, t2) << " s, hierarchy + upload + hot path + download "

@@ -7,6 +7,7 @@
 //   GPU     (the worker thread) runs the tool's per-file body on its device: hierarchy and fields created, upload, the
 //           library calls, download into a free output set, hierarchy and fields freed;
 //   writer  writes the output set as the file's plotfile.
+// All three run the body with a one-rank RankCtx (multi_gpu.hpp), as a single run does.
 // Host memory: 2 input sets and 2 output sets per worker, each one PinnedLevel per level, allocated on first use and grown
 // only when a larger file arrives, so a worker holds at most 4 buffer sets of the largest file.  They stay pageable
 // (tool_common.hpp: pinning costs more than it saves on data that crosses PCIe once); the pinned bounce buffers of the
@@ -17,27 +18,11 @@
 #include <chrono>
 #include <condition_variable>
 #include <deque>
-#include <functional>
 #include <map>
 #include <mutex>
 #include <thread>
 
-#include "tool_common.hpp"
-
-using HostSet = std::vector<PinnedLevel>;              // [level] -> [comp][level cells]
-
-inline void ensure_levels(HostSet& s, int nlev) {       // never shrinks: the buffers of deeper levels stay for later files
-    if ((int)s.size() < nlev) s.resize(nlev);
-}
-
-// What a tool supplies: its single-run body cut at the two host buffer hand-overs.  gpu() runs on a thread that called
-// pa_init for its device, leaves nothing allocated on the device, and fills `out` (which may be `in` itself in a single run).
-template <class File>
-struct SeriesBody {
-    std::function<void(const File&, HostSet& in)> read;
-    std::function<void(const File&, HostSet& in, HostSet& out, StagedDownloader& dl)> gpu;
-    std::function<void(const File&, const HostSet& out)> write;
-};
+#include "multi_gpu.hpp"
 
 // infiles=...: the list.  The keys that name one file cannot be combined with it, and transport only concerns box
 // distribution of one file over several GPUs.
@@ -86,7 +71,7 @@ struct SeriesShared {
 };
 
 template <class File>
-void series_worker(int dev, SeriesShared& S, const std::vector<File>& files, const SeriesBody<File>& body, bool verbose) {
+void series_worker(int dev, SeriesShared& S, const std::vector<File>& files, const ToolBody<File>& body, bool verbose) {
     struct Item { int file, set; double read_s, gpu_s; int64_t dev_bytes; };
     using clk = std::chrono::steady_clock;
     auto since = [](clk::time_point t) { return std::chrono::duration<double>(clk::now() - t).count(); };
@@ -105,7 +90,7 @@ void series_worker(int dev, SeriesShared& S, const std::vector<File>& files, con
             if (k >= (int)files.size()) { to_gpu.push(Item{-1, -1, 0, 0, 0}); return; }
             const int s = free_in.pop();
             const auto t0 = clk::now();
-            stage(files[k], [&] { body.read(files[k], in[s]); });
+            stage(files[k], [&] { body.read(files[k], RankCtx(files[k].meta, files[k].Nlev), in[s], false); });
             to_gpu.push(Item{k, s, since(t0), 0, 0});
         }
     });
@@ -115,7 +100,7 @@ void series_worker(int dev, SeriesShared& S, const std::vector<File>& files, con
             if (it.file < 0) return;
             const File& F = files[it.file];
             const auto t0 = clk::now();
-            stage(F, [&] { body.write(F, out[it.set]); });
+            stage(F, [&] { RankCtx(F.meta, F.Nlev).write(F, out[it.set]); });
             const double write_s = since(t0);
             free_out.push(it.set);
             if (verbose) {
@@ -132,7 +117,8 @@ void series_worker(int dev, SeriesShared& S, const std::vector<File>& files, con
         if (it.file < 0) { to_write.push(it); break; }
         const int o = free_out.pop();
         const auto t0 = clk::now();
-        stage(files[it.file], [&] { body.gpu(files[it.file], in[it.set], out[o], dl); });
+        const File& F = files[it.file];
+        stage(F, [&] { body.gpu(F, RankCtx(F.meta, F.Nlev), in[it.set], out[o], dl); });
         it.gpu_s = since(t0);
         free_in.push(it.set);
         check(pa_debug_device_bytes(&it.dev_bytes), "pa_debug_device_bytes");
@@ -145,7 +131,7 @@ void series_worker(int dev, SeriesShared& S, const std::vector<File>& files, con
 
 // returns after every output plotfile is complete; ngpus workers (one per GPU) share the list
 template <class File>
-void run_series(int ngpus, const std::vector<File>& files, const SeriesBody<File>& body, bool verbose) {
+void run_series(int ngpus, const std::vector<File>& files, const ToolBody<File>& body, bool verbose) {
     if (ngpus < 1) pa_abort("ngpus must be >= 1");
     SeriesShared S;
     const int nw = std::min<int>(ngpus, (int)files.size());

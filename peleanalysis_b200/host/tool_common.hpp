@@ -77,7 +77,7 @@ struct PinnedLevel {
         cap = bytes;
         if (pinned) {
             void* q = nullptr;
-            check(pa_host_alloc(&q, bytes), "pa_host_alloc");
+            check(pa_host_alloc(&q, bytes ? bytes : 8), "pa_host_alloc");   // a rank may own no box of a level
             p = (double*)q;
         } else {
             void* q = nullptr;
@@ -90,6 +90,12 @@ struct PinnedLevel {
     void release() { if (p) { if (pinned) pa_host_free(p); else std::free(p); } p = nullptr; cap = 0; }
     ~PinnedLevel() { release(); }
 };
+
+using HostSet = std::vector<PinnedLevel>;              // [level] -> [comp][level cells]
+
+inline void ensure_levels(HostSet& s, int nlev) {       // never shrinks: the buffers of deeper levels stay for later files
+    if ((int)s.size() < nlev) s.resize(nlev);
+}
 
 // Device -> pageable host memory through a pair of pinned bounce buffers: the DMA runs at full PCIe speed into pinned memory and
 // the host-side copy of one (level, component) overlaps the transfer of the next.  Measured on the B200 box: a direct download
