@@ -11,6 +11,7 @@ from typing import List, Optional, Sequence
 import numpy as np
 
 from .plotfile import Level, Plotfile
+from .stencilrun import download_level
 
 
 def level_fgr(base_fgr: int, ratios: Sequence[int], same_fgr_all_levels: bool, lev: int) -> int:
@@ -44,7 +45,8 @@ class FilterRun:
 
     rank / nranks > 1: the re-chopped boxes of every level are spread over the ranks by pa_sfc_distribute, only this rank's
     boxes are uploaded and returned, and every fill is preceded by its slab exchange (multigpu.FillPatchExchange over the
-    current torch.distributed group; `multigpu` / `wrap` let tests hand in another binding and host-memory slabs)."""
+    current torch.distributed group; `multigpu` / `wrap` let tests hand in another binding and host-memory slabs).
+    out_names: the filtered variables in file order; download_level(l): this rank's share of level l in that order."""
 
     def __init__(self, P, pf: Plotfile, filter_type: int = 1, base_fgr: int = 2, same_fgr_all_levels: bool = False,
                  max_grid_size: int = 32, interp_type: int = 1, variables: Optional[Sequence[str]] = None,
@@ -63,6 +65,8 @@ class FilterRun:
         self.ncomp = len(comps)
         self.fin = P.Field(self.hier, self.ncomp, max(self.ngrow))
         self.fout = P.Field(self.hier, self.ncomp, 0)
+        self.out_names = self.names
+        self.outputs = [(self.fout, c) for c in range(self.ncomp)]
         self.exchanges = []
         if nranks > 1:
             if multigpu is None:
@@ -87,6 +91,9 @@ class FilterRun:
         per_comp = [self.fout.download_fabs(c) for c in range(self.ncomp)]
         return [[np.stack([per_comp[c][l][b] for c in range(self.ncomp)]) if per_comp[0][l][b] is not None else None
                  for b in range(len(lv.boxes))] for l, lv in enumerate(self.levels)]
+
+    def download_level(self, lev: int) -> np.ndarray:
+        return download_level(self.P, self.hier, self.outputs, lev)
 
     def grown_input(self, lev: int, box: int, comp: int) -> np.ndarray:
         """the input FAB with the field's ghost width; only the level's own ngrow layers are filled"""

@@ -69,15 +69,42 @@ def unique_old_name(path: str) -> str:
     return "%s.old.%d" % (path, int(time.time() * 1e6) % 10**10)
 
 
-def write_plotfile(path: str, pf: Plotfile, nfiles_per_level: int = 1, clean: str = "rename") -> None:
-    """Write `pf` to directory `path`.  clean='rename' mimics the reference (an existing
-    directory is renamed to <path>.old.<unique>); clean='remove' deletes it (benchmarks)."""
+def create_plotfile_dirs(path: str, nlev: int, clean: str = "rename") -> None:
+    """`path` and its Level_l directories.  clean='rename' mimics the reference (an existing directory is renamed to
+    <path>.old.<unique>); clean='remove' deletes it (benchmarks)."""
     if os.path.lexists(path):
         if clean == "remove":
             shutil.rmtree(path)
         else:
             os.rename(path, unique_old_name(path))
     os.makedirs(path)
+    for il in range(nlev):
+        os.makedirs(os.path.join(path, "Level_%d" % il))
+
+
+def write_fab_file(path: str, lev: int, fname: str, level: Level, box_ids: Sequence[int], fabs: Sequence[np.ndarray]) -> list:
+    """Level_<lev>/<fname> holding the FABs of the boxes box_ids of `level`; fabs[i] is the data of box box_ids[i], component
+    first ([ncomp, nz, ny, nx] or [ncomp, cells]).  Returns one record (lev, box, fname, offset, mins, maxs) per box for
+    write_metadata.  No file is created for no boxes."""
+    records = []
+    if not len(box_ids):
+        return records
+    with open(os.path.join(path, "Level_%d" % lev, fname), "wb") as f:
+        for b, fab in zip(box_ids, fabs):
+            lo, hi = level.boxes[b]
+            n = (hi[2] - lo[2] + 1, hi[1] - lo[1] + 1, hi[0] - lo[0] + 1)
+            assert fab.shape[1:] in (n, (n[0] * n[1] * n[2],)), (fname, b, fab.shape)
+            a = np.ascontiguousarray(fab, dtype="<f8").reshape(len(fab), -1)
+            off = f.tell()
+            f.write(("%s%s %d\n" % (_FAB_DESC, _box_str(lo, hi), a.shape[0])).encode())
+            f.write(a.tobytes())
+            records.append((lev, b, fname, off, a.min(axis=1).tolist(), a.max(axis=1).tolist()))
+    return records
+
+
+def write_metadata(path: str, pf: Plotfile, records: Sequence[tuple]) -> None:
+    """Header (WriteGenericPlotfileHeader, AMReX_PlotFileUtil.cpp:73-155) and every Level_l/Cell_H (VisMF header v1) of `pf`
+    (its FABs are not used) from the write_fab_file records of all its boxes."""
     nlev = len(pf.levels)
     with open(os.path.join(path, "Header"), "w") as h:
         h.write("HyperCLaw-V1.1\n%d\n" % len(pf.names))
@@ -103,41 +130,36 @@ def write_plotfile(path: str, pf: Plotfile, nfiles_per_level: int = 1, clean: st
             h.write("Level_%d/Cell\n" % il)
     ncomp = len(pf.names)
     for il, l in enumerate(pf.levels):
-        ldir = os.path.join(path, "Level_%d" % il)
-        os.makedirs(ldir)
         nb = len(l.boxes)
-        nf = max(1, min(nfiles_per_level, nb))
-        fod = []
-        files = [open(os.path.join(ldir, "Cell_D_%05d" % i), "wb") for i in range(nf)]
-        mins = np.empty((nb, ncomp))
-        maxs = np.empty((nb, ncomp))
-        for ib, ((lo, hi), fab) in enumerate(zip(l.boxes, l.fabs)):
-            f = files[ib % nf]
-            fod.append(("Cell_D_%05d" % (ib % nf), f.tell()))
-            f.write(("%s%s %d\n" % (_FAB_DESC, _box_str(lo, hi), ncomp)).encode())
-            a = np.ascontiguousarray(fab, dtype="<f8")
-            assert a.shape == (ncomp, hi[2] - lo[2] + 1, hi[1] - lo[1] + 1, hi[0] - lo[0] + 1), a.shape
-            f.write(a.tobytes())
-            flat = a.reshape(ncomp, -1)
-            mins[ib] = flat.min(axis=1)
-            maxs[ib] = flat.max(axis=1)
-        for f in files:
-            f.close()
-        with open(os.path.join(ldir, "Cell_H"), "w") as c:
+        rec = {r[1]: r for r in records if r[0] == il}
+        assert len(rec) == nb and all(len(r[4]) == ncomp for r in rec.values()), "level %d: %d of %d boxes written" % (il, len(rec), nb)
+        with open(os.path.join(path, "Level_%d" % il, "Cell_H"), "w") as c:
             c.write("1\n1\n%d\n0\n" % ncomp)
             c.write("(%d 0\n" % nb)
             for lo, hi in l.boxes:
                 c.write(_box_str(lo, hi) + "\n")
             c.write(")\n")
             c.write("%d\n" % nb)
-            for name, off in fod:
-                c.write("FabOnDisk: %s %d\n" % (name, off))
+            for b in range(nb):
+                c.write("FabOnDisk: %s %d\n" % rec[b][2:4])
             c.write("\n")
-            for tab in (mins, maxs):
+            for k in (4, 5):                                   # mins, maxs
                 c.write("%d,%d\n" % (nb, ncomp))
-                for row in tab:
-                    c.write("".join("%.17e," % v for v in row) + "\n")
+                for b in range(nb):
+                    c.write("".join("%.17e," % v for v in rec[b][k]) + "\n")
                 c.write("\n")
+
+
+def write_plotfile(path: str, pf: Plotfile, nfiles_per_level: int = 1, clean: str = "rename") -> None:
+    """Write `pf` to directory `path`, box b of a level to file Cell_D_<b mod nfiles_per_level>.  clean: as create_plotfile_dirs."""
+    create_plotfile_dirs(path, len(pf.levels), clean)
+    records = []
+    for il, l in enumerate(pf.levels):
+        nf = max(1, min(nfiles_per_level, len(l.boxes)))
+        for i in range(nf):
+            ids = range(i, len(l.boxes), nf)
+            records += write_fab_file(path, il, "Cell_D_%05d" % i, l, ids, [l.fabs[b] for b in ids])
+    write_metadata(path, pf, records)
 
 
 def _ints(s: str) -> List[int]:
@@ -236,38 +258,50 @@ def parse_fab_header(line: str, where: str = "?"):
     return dt, tuple(b[0:3]), tuple(b[3:6]), b[9]
 
 
+def read_boxes(path: str, lev: int, box_ids: Sequence[int], comp_ids: Sequence[int]) -> List[np.ndarray]:
+    """Components comp_ids of the boxes box_ids of level lev: one float64 [len(comp_ids), nz, ny, nx] array per box (its valid
+    cells).  Only those FABs and components are read; consecutive components are one read per FAB."""
+    hd = read_header(path)
+    _, boxes, fod, _, _ = read_cell_h(path, hd["paths"][lev])
+    ldir = os.path.dirname(os.path.join(path, hd["paths"][lev]))
+    comp_ids = list(comp_ids)
+    one_read = bool(comp_ids) and comp_ids == list(range(comp_ids[0], comp_ids[0] + len(comp_ids)))
+    out = []
+    for b in box_ids:
+        (lo, hi), (fn, off) = boxes[b], fod[b]
+        with open(os.path.join(ldir, fn), "rb") as f:
+            f.seek(off)
+            dt, flo, fhi, fnc = parse_fab_header(f.readline().decode("ascii", "replace"), fn)
+            base = f.tell()
+            if any(flo[d] > lo[d] or fhi[d] < hi[d] for d in range(3)) or max(comp_ids, default=-1) >= fnc:
+                raise ValueError("FAB in %s does not cover box %s / components %s" % (fn, (lo, hi), comp_ids))
+            m = [fhi[d] - flo[d] + 1 for d in range(3)]
+            npts = m[0] * m[1] * m[2]
+            sl = tuple(slice(lo[d] - flo[d], hi[d] - flo[d] + 1) for d in (2, 1, 0))
+            if one_read:
+                f.seek(base + np.dtype(dt).itemsize * npts * comp_ids[0])
+                a = np.fromfile(f, dt, npts * len(comp_ids)).reshape(len(comp_ids), m[2], m[1], m[0])[(slice(None),) + sl].astype("<f8")
+            else:
+                a = np.empty((len(comp_ids), hi[2] - lo[2] + 1, hi[1] - lo[1] + 1, hi[0] - lo[0] + 1))
+                for k, c in enumerate(comp_ids):
+                    f.seek(base + np.dtype(dt).itemsize * npts * c)
+                    a[k] = np.fromfile(f, dt, npts).reshape(m[2], m[1], m[0])[sl]
+        out.append(a)
+    return out
+
+
 def read_plotfile(path: str, comps: Sequence[str] | None = None, finest_level: int | None = None,
                   load_data: bool = True) -> Plotfile:
-    """Read a plotfile.  comps=None reads every component; otherwise only the named ones, in that order."""
+    """Read a plotfile.  comps=None reads every component; otherwise only the named ones, in that order.  load_data=False
+    reads the metadata only (levels without FABs)."""
     hd = read_header(path)
     nlev = hd["finest"] + 1 if finest_level is None else min(finest_level, hd["finest"]) + 1
     names = hd["names"] if comps is None else list(comps)
     idx = [hd["names"].index(n) for n in names]
     levels = []
     for lev in range(nlev):
-        ncomp, boxes, fod, _, _ = read_cell_h(path, hd["paths"][lev])
-        ldir = os.path.dirname(os.path.join(path, hd["paths"][lev]))
-        fabs = []
-        if load_data:
-            for (lo, hi), (fn, off) in zip(boxes, fod):
-                n = [hi[d] - lo[d] + 1 for d in range(3)]
-                with open(os.path.join(ldir, fn), "rb") as f:
-                    f.seek(off)
-                    dt, flo, fhi, fnc = parse_fab_header(f.readline().decode("ascii", "replace"), fn)
-                    base = f.tell()
-                    m = [fhi[d] - flo[d] + 1 for d in range(3)]
-                    if any(flo[d] > lo[d] or fhi[d] < hi[d] for d in range(3)) or fnc < ncomp:
-                        raise ValueError("FAB in %s does not cover box %s with %d components" % (fn, (lo, hi), ncomp))
-                    npts = m[0] * m[1] * m[2]
-                    sl = tuple(slice(lo[d] - flo[d], lo[d] - flo[d] + n[d]) for d in (2, 1, 0))
-                    if len(idx) == ncomp and idx == list(range(ncomp)):
-                        a = np.fromfile(f, dt, npts * ncomp).reshape(ncomp, m[2], m[1], m[0])[(slice(None),) + sl].astype("<f8")
-                    else:
-                        a = np.empty((len(idx), n[2], n[1], n[0]))
-                        for o, c in enumerate(idx):
-                            f.seek(base + np.dtype(dt).itemsize * npts * c)
-                            a[o] = np.fromfile(f, dt, npts).reshape(m[2], m[1], m[0])[sl]
-                fabs.append(a)
+        _, boxes, _, _, _ = read_cell_h(path, hd["paths"][lev])
+        fabs = read_boxes(path, lev, range(len(boxes)), idx) if load_data else []
         dlo, dhi = hd["domains"][lev]
         levels.append(Level(dlo, dhi, hd["dx"][lev], boxes, fabs))
     return Plotfile(names, hd["prob_lo"], hd["prob_hi"], hd["ref_ratio"][: nlev - 1], levels, hd["time"], hd["coord"])

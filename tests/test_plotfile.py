@@ -111,6 +111,19 @@ def test_other_on_disk_formats(tmp_path, dtype, grow):
     got = np.concatenate([f[g.comp("temp")].ravel() for l in g.levels for f in l.fabs])
     want = np.concatenate([f[0].astype(dtype).astype("<f8").ravel() for l in pf.levels for f in l.fabs])
     assert np.array_equal(got, want)
+    # mgtools reads through plotfile.read_boxes: the executable's plotfile, value for value
+    import importlib.util
+    from peleanalysis_b200 import capi as product_capi, mgtools
+    spec = importlib.util.spec_from_file_location("capi_emulated_formats", product_capi.__file__)
+    emu = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(emu)
+    emu.LIB_PATH = lib
+    mgtools.run("grad", ["infile=" + d, "gradVar=temp", "outfile=" + str(tmp_path / "m")], capi=emu, device=0)
+    m = plotfile.read_plotfile(str(tmp_path / "m"))
+    assert m.names == g.names
+    for n in g.names:
+        assert np.array_equal(np.concatenate([f[m.comp(n)].ravel() for l in m.levels for f in l.fabs]),
+                              np.concatenate([f[g.comp(n)].ravel() for l in g.levels for f in l.fabs])), n
     if O.have_ref():
         O.run_ref("grad", d, str(tmp_path / "gref"), gradVar="temp")
         q = subprocess.run([O.ref_exe("fcompare.ref.ex"), str(tmp_path / "g"), str(tmp_path / "gref")], capture_output=True, text=True)
