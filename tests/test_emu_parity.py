@@ -29,7 +29,8 @@ def emu():
     m = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(m)
     m.LIB_PATH = lib                     # a private module instance: the product binding itself is untouched
-    old = {k: os.environ.get(k) for k in ("PA_NORMAL_MATH", "PA_STENCIL", "PA_TMA_SMALL", "PA_CURV_FUSED", "PA_NORMAL_F3", "PA_NORMAL_W", "CUEMU_SEED")}
+    old = {k: os.environ.get(k) for k in ("PA_NORMAL_MATH", "PA_STENCIL", "PA_TMA_SMALL", "PA_CURV_FUSED", "PA_NORMAL_F3", "PA_NORMAL_W", "PA_CURV_UNFUSED",
+                                       "CUEMU_SEED")}
     os.environ["PA_NORMAL_MATH"] = "fast"   # no device self-test: the emulator has no MUFU (sqrt_fast == sqrt there)
     m.init(0)
     yield m

@@ -34,7 +34,7 @@ def _random_boxes(rng, lo, hi, nmax, min_size=2, max_size=10):
     return out
 
 
-def random_case(seed, curvature):
+def random_case(seed, curvature, names=("temp",)):
     rng = np.random.default_rng(seed)
     base = tuple(int(rng.choice([8, 10, 12, 16, 20])) for _ in range(3))
     mgs = int(rng.choice([6, 8, 12, 16, 32]))
@@ -63,7 +63,7 @@ def random_case(seed, curvature):
                 regions.append(refined(c2, 2))
                 ratios.append(2)
     prob_hi = (1.0, 1.0, 1.0) if rng.random() < 0.7 else (0.7, 0.35, 1.3)
-    pf = synth.make_hierarchy(base, regions, ratios, mgs, ("temp",), prob_hi=prob_hi, header_ratio=None)
+    pf = synth.make_hierarchy(base, regions, ratios, mgs, names, prob_hi=prob_hi, header_ratio=None)
     return pf, is_per, sym
 
 

@@ -24,8 +24,10 @@ def _flat(pf, name):
 def _set_stencil(stencil):
     """tma: TMA pipeline, CTA shape by tile size (small boxes -> 2 / 4 consumer warps); tma_big: TMA pipeline in the 8 /
     16-warp shapes whatever the tile size; tma_fused: curvature through the fused kernel + shell pass where the hierarchy is
-    eligible (PA_CURV_FUSED=1, opt-in; tma_fused3: the later fused kernel); simple: the plain-load kernels."""
+    eligible (PA_CURV_FUSED=1, opt-in; tma_fused3: the later fused kernel); simple: the plain-load kernels; unfused: curvature's
+    progress pass as a kernel of its own, then the flame normal from the materialised Progress (PA_CURV_UNFUSED=1)."""
     os.environ["PA_STENCIL"] = "simple" if stencil == "simple" else "tma"
+    os.environ["PA_CURV_UNFUSED"] = "1" if stencil == "unfused" else "0"
     os.environ["PA_TMA_SMALL"] = "0" if stencil.startswith("tma_big") else "1"
     os.environ["PA_CURV_FUSED"] = {"tma_fused": "1", "tma_fused3": "3"}.get(stencil, "0")
     os.environ["PA_NORMAL_F3"] = "1" if stencil == "tma_n3" else "0"      # flame normal through curv_f3.cu's kernel without its K part
