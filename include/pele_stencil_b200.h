@@ -13,7 +13,8 @@
  * PA_ERR_CUDA when no sm_100 device is usable.
  *
  * Host buffers are FArrayBox-ordered: the VALID region of one box, one component, i fastest
- * ([nz][ny][nx] doubles) -- what FArrayBox::dataPtr(comp) addresses for a 0-ghost FAB.
+ * ([nz][ny][nx] doubles) -- what FArrayBox::dataPtr(comp) addresses for a 0-ghost FAB.  Data that is already in device
+ * memory (a GPU MultiFab, a CUDA tensor) goes in and out through pa_array4 descriptors (pa_field_upload_device).
  */
 #ifndef PELE_STENCIL_B200_H
 #define PELE_STENCIL_B200_H
@@ -148,6 +149,31 @@ int pa_field_download(const pa_field *f, int lev, int box, int comp, double *hos
 int pa_field_upload_level(pa_field *f, int lev, int comp, const double *host_concat);
 int pa_field_download_level(const pa_field *f, int lev, int comp, double *host_concat);
 int pa_field_set_val(pa_field *f, int comp, int ncomp, double v);     /* MultiFab::setVal incl. ghost cells */
+/* ---- data already on the GPU: device arrays <-> field, no host round trip -------------------------------------------------
+ * pa_array4 has the fields of amrex::Array4<double> (AX/Base/AMReX_Array4.H), so an AMReX caller fills it field for field from
+ * fab.array() / mf.const_array(mfi): cell (i,j,k), component n lives at p[(i-begin[0]) + (j-begin[1])*jstride +
+ * (k-begin[2])*kstride + n*nstride].  A ghost-free dense box has begin = the box's lo; a FAB with nGrow ghost cells has
+ * begin = lo - nGrow.  p is device (or managed) memory of the calling thread's device. */
+typedef struct {
+    double *p;                          /* device (or managed) memory of the calling thread's device */
+    int64_t jstride, kstride, nstride;  /* in doubles; the i stride is 1 */
+    int begin[3], end[3];               /* index box the array covers, end exclusive (Array4::begin / end) */
+    int ncomp;
+} pa_array4;
+/* src[k] / dst[k] belongs to this rank's k-th box of the level in ascending global box id (the order of pa_field_upload_level);
+ * nsrc / ndst must equal the number of those boxes.  Upload copies components 0..ncomp-1 of every array into components
+ * comp..comp+ncomp-1 of f; download the other way.  Only the box's VALID cells move: the field's ghost cells are not written,
+ * and bytes of a destination array outside its valid box keep their values.  One kernel launch per call for all boxes and
+ * components.  PA_ERR_ARG (the message names the problem) for a null pointer, a wrong array count, begin / end that do not
+ * contain the box, ncomp beyond an array's ncomp or a component range outside the field, strides too small for the array's
+ * extents (rows, planes or components overlapping), download destinations whose written address ranges overlap, and memory
+ * that cudaPointerGetAttributes reports as host memory (use pa_field_upload_level / pa_field_download_level for host data)
+ * or as memory of another device.  A level with no local boxes is a no-op.
+ * Streams: both calls are asynchronous on the library stream (pa_set_stream) and never synchronise it.  The CALLER orders
+ * whatever produces src before pa_field_upload_device and whatever consumes dst after pa_field_download_device -- simplest by
+ * making its own stream the library stream, or with an event. */
+int pa_field_upload_device(pa_field *f, int lev, int comp, int ncomp, const pa_array4 *src, int nsrc);
+int pa_field_download_device(const pa_field *f, int lev, int comp, int ncomp, const pa_array4 *dst, int ndst);
 /* Fingerprint of the valid cells of comps [comp, comp+ncomp) of this rank's boxes: sum mod 2^64 of a mix of every cell's bit
  * pattern with (level, GLOBAL box id, component, cell index).  Adding the ranks' values (wrapping) gives a number that does
  * not depend on the box -> rank map: equal fingerprints for 1, 2, 4, 8 ranks <=> bit-identical outputs (with overwhelming

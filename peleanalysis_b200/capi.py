@@ -38,6 +38,60 @@ class SmoothOpts(C.Structure):
                 ("reserved", C.c_int * 7)]
 
 
+class Array4(C.Structure):
+    """pa_array4: the fields of amrex::Array4<double> -- a device array covering the index box [begin, end) (end exclusive),
+    cell (i,j,k) component n at p[(i-begin0) + (j-begin1)*jstride + (k-begin2)*kstride + n*nstride], strides in doubles."""
+    _fields_ = [("p", C.c_void_p), ("jstride", C.c_int64), ("kstride", C.c_int64), ("nstride", C.c_int64),
+                ("begin", C.c_int * 3), ("end", C.c_int * 3), ("ncomp", C.c_int)]
+
+
+def array4_of(obj, box, nghost: int = 0) -> Array4:
+    """Array4 of a CUDA array (anything with __cuda_array_interface__: torch, CuPy, pyAMReX) that holds box (lo, hi) grown by
+    nghost cells, starting at its first element: [nz][ny][nx] or [ncomp][nz][ny][nx] float64 with unit x stride.  Views with
+    other strides are fine (a component chosen by slicing, a sub-box of a bigger array).  ValueError for anything else."""
+    if isinstance(obj, Array4):
+        return obj
+    if getattr(obj, "is_cuda", False) and hasattr(obj, "data_ptr"):      # torch tensor: the same fields, without building the dict
+        if str(obj.dtype) != "torch.float64":
+            raise ValueError("array4_of needs float64 data, got %s" % obj.dtype)
+        cai = {"shape": tuple(obj.shape), "typestr": "<f8", "strides": tuple(8 * s for s in obj.stride()), "data": (obj.data_ptr(), False)}
+    else:
+        cai = getattr(obj, "__cuda_array_interface__", None)
+    if cai is None:
+        raise ValueError("array4_of needs an object with __cuda_array_interface__ (a CUDA array), got %s" % type(obj).__name__)
+    shape = tuple(int(s) for s in cai["shape"])
+    if cai.get("typestr") != "<f8":
+        raise ValueError("array4_of needs float64 ('<f8') data, got %r" % cai.get("typestr"))
+    if cai.get("mask") is not None:
+        raise ValueError("array4_of: masked arrays are not supported")
+    if len(shape) not in (3, 4):
+        raise ValueError("array4_of needs a 3-D [nz][ny][nx] or 4-D [ncomp][nz][ny][nx] array, got shape %s" % (shape,))
+    strides = cai.get("strides")
+    if strides is None:                                    # C-contiguous
+        strides, s = [], 8
+        for n in reversed(shape):
+            strides.insert(0, s)
+            s *= n
+    strides = [int(s) for s in strides]
+    if any(s % 8 for s in strides):
+        raise ValueError("array4_of: strides %s are not whole doubles" % (strides,))
+    if shape[-1] > 1 and strides[-1] != 8:
+        raise ValueError("array4_of needs unit x stride (the last dimension contiguous), got %d bytes" % strides[-1])
+    if len(shape) == 3:
+        shape, strides = (1,) + shape, [shape[0] * strides[0]] + strides
+    ptr = int(cai["data"][0])
+    if ptr == 0 and any(n > 0 for n in shape):
+        raise ValueError("array4_of: null data pointer")
+    lo = box[0]
+    a = Array4()
+    a.p = ptr
+    a.nstride, a.kstride, a.jstride = strides[0] // 8, strides[1] // 8, strides[2] // 8
+    a.begin[:] = [int(lo[d]) - nghost for d in range(3)]
+    a.end[:] = [int(lo[d]) - nghost + shape[3 - d] for d in range(3)]
+    a.ncomp = shape[0]
+    return a
+
+
 PA_ERR_UNSUPPORTED, PA_ERR_NOCONV = -4, -6
 PA_SMOOTH_PRECOND_JACOBI, PA_SMOOTH_PRECOND_MG = 0, 1
 SMOOTH_PRECONDS = {"jacobi": PA_SMOOTH_PRECOND_JACOBI, "mg": PA_SMOOTH_PRECOND_MG}
@@ -64,6 +118,8 @@ SYMBOLS = {
     "pa_field_upload": (_i, [_vp, _i, _i, _i, _vp]), "pa_field_download": (_i, [_vp, _i, _i, _i, _vp]),
     "pa_field_upload_level": (_i, [_vp, _i, _i, _vp]), "pa_field_download_level": (_i, [_vp, _i, _i, _vp]),
     "pa_field_set_val": (_i, [_vp, _i, _i, _d]),
+    "pa_field_upload_device": (_i, [_vp, _i, _i, _i, C.POINTER(Array4), _i]),
+    "pa_field_download_device": (_i, [_vp, _i, _i, _i, C.POINTER(Array4), _i]),
     "pa_field_hash": (_i, [_vp, _i, _i, C.POINTER(C.c_uint64)]),
     "pa_fill_boundary": (_i, [_vp, _i, _i, _i]), "pa_fill_ghosts": (_i, [_vp, _i, _i, _i, _i]),
     "pa_grad": (_i, [_vp, _i, _i, _vp, _i]), "pa_grad_phases": (_i, [_vp, _i, _i, _vp, _i, _i]),
@@ -340,6 +396,28 @@ class Field:
     def download_level(self, lev: int, comp: int, host: np.ndarray) -> None:
         assert host.dtype == np.float64 and host.flags.c_contiguous and host.size == self.hier.local_cells[lev]
         check(lib().pa_field_download_level(self.f, lev, comp, _ptr(host)))
+
+    def _arrays(self, lev: int, arrays, nghost: int):
+        boxes = [self.hier.levels[lev].boxes[b] for b in self.hier.local_boxes[lev]]
+        if len(arrays) != len(boxes):
+            raise ValueError("level %d: %d arrays for the %d boxes this rank owns" % (lev, len(arrays), len(boxes)))
+        descs = (Array4 * max(len(boxes), 1))()
+        for k, (a, bx) in enumerate(zip(arrays, boxes)):
+            descs[k] = array4_of(a, bx, nghost)
+        return descs, len(boxes)
+
+    def upload_level_device(self, lev: int, comp: int, arrays, nghost: int = 0, ncomp: int = 1) -> None:
+        """Components 0..ncomp-1 of one CUDA array (or Array4) per local box of the level, in box order, into components
+        comp..comp+ncomp-1; each array holds its box grown by nghost cells.  Asynchronous on the library stream: order the
+        arrays' producer before this call (e.g. set_stream(torch.cuda.current_stream().cuda_stream))."""
+        descs, n = self._arrays(lev, arrays, nghost)
+        check(lib().pa_field_upload_device(self.f, lev, comp, ncomp, descs, n))
+
+    def download_level_device(self, lev: int, comp: int, arrays, nghost: int = 0, ncomp: int = 1) -> None:
+        """The valid cells of components comp..comp+ncomp-1 into one CUDA array per local box (the inverse of
+        upload_level_device); cells of the arrays outside the valid box are left alone."""
+        descs, n = self._arrays(lev, arrays, nghost)
+        check(lib().pa_field_download_device(self.f, lev, comp, ncomp, descs, n))
 
     def upload_box(self, lev: int, box: int, comp: int, host: np.ndarray) -> None:
         host = np.ascontiguousarray(host, dtype=np.float64)

@@ -94,6 +94,10 @@ struct LevelDev {
     DevBuf<long long> host_off;                        // nlocal+1 prefix of valid cells (host concat order)
     DevBuf<int> gid;                                   // global box id of every local box
     std::vector<long long> host_off_h;
+    // device-array copies (pa_field_upload_device): row items of the local boxes and the lanes per row, built on first use
+    std::vector<PaRowItem> io_items_h;
+    DevBuf<PaRowItem> io_items;
+    int io_lg_s = 0;
 };
 
 // Tiles are stored class-major, level-minor: a "class" groups the boxes one CTA shape of the TMA pipeline serves
@@ -162,6 +166,7 @@ struct pa_hier {
     DevBuf<int> shell_level, shell_box;
     long long shell_begin[PA_MAX_LEVELS + 1] = {0};
     std::map<cudaStream_t, std::unique_ptr<DevBuf<double>>> staging;   // upload / download staging, one per stream
+    std::map<cudaStream_t, std::unique_ptr<DevBuf<PaA4Dev>>> a4;       // per-box array records of device copies, one per stream
     DevBuf<double> send_slab, recv_slab;               // multi-rank exchange, [cell][comp]
     pa_field* recv_owner = nullptr;                    // the field whose exchanged data the (shared) recv slab holds right now
     int slab_ncomp = 0;
@@ -1059,6 +1064,117 @@ int pa_field_download_level(const pa_field* f, int lev, int comp, double* host) 
     CU(cudaMemcpyAsync(host, stg, (size_t)n * 8, cudaMemcpyDeviceToHost, t_stream));
     return PA_OK;
 }
+// ---- caller's device arrays (pa_array4) <-> valid cells of a level, one kernel launch per call ---------------------------
+// Row items: a box is cut into runs of whole rows of about 4096 cells; the lanes sharing a row are the power of two (4..32)
+// that the narrowest local box of the level fills, so 16-wide boxes keep all 32 lanes of a warp busy (two rows per warp).
+static int device_io_items(pa_hier* h, int lev) {
+    LevelDev& D = *h->lev[lev];
+    if (!D.io_items_h.empty()) return PA_OK;
+    const Level& V = h->H.lev[lev];
+    int minx = 1 << 30;
+    for (size_t lb = 0; lb < V.local.size(); ++lb) {
+        const Box& B = V.boxes[V.local[lb]];
+        minx = std::min(minx, B.len(0));
+        const int rows = B.len(1) * B.len(2), per = std::max(1, 4096 / B.len(0));
+        for (int r = 0; r < rows; r += per) D.io_items_h.push_back(PaRowItem{(int)lb, r, std::min(per, rows - r), 0});
+    }
+    D.io_lg_s = minx >= 32 ? 5 : minx >= 16 ? 4 : minx >= 8 ? 3 : 2;
+    CU(D.io_items.upload(D.io_items_h, t_stream));      // the host vector lives as long as the hierarchy
+    return PA_OK;
+}
+
+// Validates the arrays of one call and resolves them against the local boxes (records in local box order).
+static int resolve_array4(const pa_field* f, int lev, int comp, int ncomp, const pa_array4* a, int na, bool is_dst, const char* who,
+                          std::vector<PaA4Dev>& rec) {
+    auto bad = [&](const std::string& m) { return fail(PA_ERR_ARG, std::string(who) + ": " + m); };
+    if (!f || !f->h) return bad("null field");
+    pa_hier* h = f->h;
+    if (lev < 0 || lev >= h->H.nlev) return bad("level out of range");
+    if (comp < 0 || ncomp < 1 || comp + ncomp > f->ncomp)
+        return bad("field components [" + std::to_string(comp) + ", " + std::to_string(comp + ncomp) + ") out of [0, " + std::to_string(f->ncomp) + ")");
+    const Level& V = h->H.lev[lev];
+    if (na != (int)V.local.size())
+        return bad("got " + std::to_string(na) + " arrays for the " + std::to_string(V.local.size()) + " boxes this rank owns on level " + std::to_string(lev));
+    if (na > 0 && !a) return bad("null array list");
+    int dev = 0;
+    CU(cudaGetDevice(&dev));
+    std::vector<std::pair<uintptr_t, uintptr_t>> ranges;
+    rec.resize(na);
+    for (int k = 0; k < na; ++k) {
+        const pa_array4& A = a[k];
+        const Box& B = V.boxes[V.local[k]];
+        const std::string at = "array " + std::to_string(k) + " (global box " + std::to_string(V.local[k]) + "): ";
+        if (!A.p) return bad(at + "null data pointer");
+        for (int d = 0; d < 3; ++d)
+            if (A.begin[d] > B.lo[d] || A.end[d] <= B.hi[d]) return bad(at + "begin / end do not contain the box");
+        if (ncomp > A.ncomp) return bad(at + "ncomp " + std::to_string(ncomp) + " exceeds the array's " + std::to_string(A.ncomp) + " components");
+        const long long lx = A.end[0] - A.begin[0], ly = A.end[1] - A.begin[1], lz = A.end[2] - A.begin[2];
+        if (A.jstride < 0 || A.kstride < 0 || A.nstride < 0) return bad(at + "negative stride");
+        if ((ly > 1 && A.jstride < lx) || (lz > 1 && A.kstride < (ly - 1) * A.jstride + lx) ||
+            (A.ncomp > 1 && A.nstride < (lz - 1) * A.kstride + (ly - 1) * A.jstride + lx))
+            return bad(at + "strides too small for the extents: rows, planes or components of the array overlap");
+#if !defined(PA_HOST_EMULATION) || defined(PA_EMU_POINTER_ATTRIBUTES)
+        cudaPointerAttributes pa;
+        std::memset(&pa, 0, sizeof(pa));
+        cudaError_t e = cudaPointerGetAttributes(&pa, A.p);
+        if (e != cudaSuccess) { cudaGetLastError(); return bad(at + "cudaPointerGetAttributes failed: " + cudaGetErrorString(e)); }
+        if (pa.type != cudaMemoryTypeDevice && pa.type != cudaMemoryTypeManaged)
+            return bad(at + "the pointer is host memory; host data goes through pa_field_upload_level / pa_field_download_level");
+        if (pa.type == cudaMemoryTypeDevice && pa.device != dev)
+            return bad(at + "the pointer is memory of device " + std::to_string(pa.device) + ", the calling thread's device is " + std::to_string(dev));
+#else
+        // a CPU test build whose runtime stand-in cannot tell device from host memory: refuse rather than guess
+        return fail(PA_ERR_UNSUPPORTED, std::string(who) + ": this build cannot query pointer attributes");
+#endif
+        PaA4Dev& r = rec[k];
+        r.p = A.p + (B.lo[0] - A.begin[0]) + (long long)(B.lo[1] - A.begin[1]) * A.jstride + (long long)(B.lo[2] - A.begin[2]) * A.kstride;
+        r.js = A.jstride; r.ks = A.kstride; r.ns = A.nstride;
+        if (is_dst) {
+            const long long last = (B.len(0) - 1) + (long long)(B.len(1) - 1) * r.js + (long long)(B.len(2) - 1) * r.ks + (long long)(ncomp - 1) * r.ns;
+            ranges.emplace_back((uintptr_t)r.p, (uintptr_t)(r.p + last + 1));
+        }
+    }
+    if (is_dst) {
+        std::vector<std::pair<uintptr_t, uintptr_t>> s = ranges;
+        std::sort(s.begin(), s.end());
+        for (size_t i = 1; i < s.size(); ++i)
+            if (s[i].first < s[i - 1].second) return bad("destination arrays overlap: their written address ranges intersect");
+    }
+    return PA_OK;
+}
+
+static int device_copy(const pa_field* f, int lev, int comp, int ncomp, const pa_array4* a, int na, bool to_field, const char* who) {
+    std::vector<PaA4Dev> rec;
+    CHK(resolve_array4(f, lev, comp, ncomp, a, na, !to_field, who, rec));
+    if (rec.empty()) return PA_OK;
+    pa_hier* h = f->h;
+    CHK(ensure_device(h));
+    CHK(device_io_items(h, lev));
+    auto& slot = h->a4[t_stream];
+    if (!slot) {                       // sized for the level with the most local boxes: never reallocated afterwards
+        slot = std::make_unique<DevBuf<PaA4Dev>>();
+        size_t most = 1;
+        for (const Level& V : h->H.lev) most = std::max(most, V.local.size());
+        CU(slot->reserve(most));
+    }
+    // rec dies when this returns: a copy from pageable memory has been staged by the time cudaMemcpyAsync returns
+    CU(cudaMemcpyAsync(slot->p, rec.data(), rec.size() * sizeof(PaA4Dev), cudaMemcpyHostToDevice, t_stream));
+    int err = PA_OK;
+    const PaLayDev* ly = dev_layout(h, lev, f->ng, &err);
+    if (!ly) return err;
+    LevelDev& D = *h->lev[lev];
+    double* base = f->slab[lev] + (long long)comp * f->cs[lev];
+    if (to_field) CU(launch_array4_to_field(D.io_items.p, (int)D.io_items_h.size(), D.boxes.p, ly, slot->p, ncomp, base, f->cs[lev], D.io_lg_s, t_stream));
+    else CU(launch_field_to_array4(D.io_items.p, (int)D.io_items_h.size(), D.boxes.p, ly, slot->p, ncomp, base, f->cs[lev], D.io_lg_s, t_stream));
+    return PA_OK;
+}
+int pa_field_upload_device(pa_field* f, int lev, int comp, int ncomp, const pa_array4* src, int nsrc) {
+    return device_copy(f, lev, comp, ncomp, src, nsrc, true, "pa_field_upload_device");
+}
+int pa_field_download_device(const pa_field* f, int lev, int comp, int ncomp, const pa_array4* dst, int ndst) {
+    return device_copy(f, lev, comp, ncomp, dst, ndst, false, "pa_field_download_device");
+}
+
 int pa_field_set_val(pa_field* f, int comp, int ncomp, double v) {
     CHK(check_field(f, comp, ncomp, "pa_field_set_val"));
     for (int l = 0; l < f->h->H.nlev; ++l)

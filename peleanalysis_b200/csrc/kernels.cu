@@ -73,6 +73,81 @@ cudaError_t launch_pack_valid(const PaBoxDev* boxes, const PaLayDev* lay, const 
     return cudaGetLastError();
 }
 
+// ------------------------------------------------------------------------------------------------------------
+// caller's device arrays (pa_array4: AMReX FABs with or without ghost cells, strided tensor views) <-> valid cells of a
+// level.  Work item = a run of rows of one box; blockIdx.y = component.  2^lg_s lanes share a row and walk it in chunks
+// of 2^lg_s cells (lg_s >= 2), so every store into the field covers whole 32-byte sectors: the field's valid rows start
+// on a sector (PaLayDev::xoff) and a chunk is a multiple of 4 doubles -- only a row's tail can be partial, as with any
+// copy of that row.  The caller's rows may start at any 8-byte offset; its loads stay coalesced along the row.  Four
+// rows per group are in flight at once.
+// ------------------------------------------------------------------------------------------------------------
+template <bool TO_FIELD>
+__global__ void __launch_bounds__(256) k_array4_copy(const PaRowItem* __restrict__ items, int nitems, const PaBoxDev* __restrict__ boxes,
+                                                     const PaLayDev* __restrict__ lay, const PaA4Dev* __restrict__ arr,
+                                                     double* __restrict__ comp_base, long long cs, int lg_s) {
+    constexpr int U = 4;
+    const int m = (int)blockIdx.y;
+    const int S = 1 << lg_s;
+    const int lane = (int)threadIdx.x & (S - 1);
+    const int g = (int)threadIdx.x >> lg_s, G = (int)blockDim.x >> lg_s;
+    for (int it = (int)blockIdx.x; it < nitems; it += (int)gridDim.x) {
+        const PaRowItem w = items[it];
+        const PaBoxDev b = boxes[w.box];
+        const PaLayDev y = lay[w.box];
+        const PaA4Dev a = arr[w.box];
+        const int nx = b.n[0], ny = b.n[1];
+        double* fld = comp_base + (long long)m * cs + y.off + (long long)y.ng * y.PS + (long long)y.ng * y.P + (y.ng + y.xoff);
+        double* usr = a.p + (long long)m * a.ns;
+        // (j, k) of this group's first row; later rows advance by G without a division
+        int j = (w.row0 + g) % ny, k = (w.row0 + g) / ny;
+        for (int r0 = g; r0 < w.nrows; r0 += U * G) {
+            long long fo[U], uo[U];
+            int nr = 0;
+#pragma unroll
+            for (int u = 0; u < U; ++u) {
+                if (r0 + u * G < w.nrows) {
+                    fo[u] = (long long)k * y.PS + (long long)j * y.P;
+                    uo[u] = (long long)k * a.ks + (long long)j * a.js;
+                    nr = u + 1;
+                } else {
+                    fo[u] = 0; uo[u] = 0;
+                }
+                j += G;
+                while (j >= ny) { j -= ny; ++k; }
+            }
+            for (int x0 = 0; x0 < nx; x0 += S) {
+                const int x = x0 + lane;
+                if (x >= nx) continue;
+                double v[U];
+#pragma unroll
+                for (int u = 0; u < U; ++u)
+                    if (u < nr) v[u] = TO_FIELD ? usr[uo[u] + x] : fld[fo[u] + x];
+#pragma unroll
+                for (int u = 0; u < U; ++u)
+                    if (u < nr) { if (TO_FIELD) fld[fo[u] + x] = v[u]; else usr[uo[u] + x] = v[u]; }
+            }
+        }
+    }
+}
+
+static int array4_grid(int nitems) { return nitems < 148 * 16 ? nitems : 148 * 16; }
+
+cudaError_t launch_array4_to_field(const PaRowItem* items, int nitems, const PaBoxDev* boxes, const PaLayDev* lay, const PaA4Dev* arr,
+                                   int ncomp, double* comp_base, long long cs, int lg_s, cudaStream_t st) {
+    if (nitems <= 0 || ncomp <= 0) return cudaSuccess;
+    PA_LAUNCH(dim3(array4_grid(nitems), ncomp), 256, 0, st, k_array4_copy<true>)(items, nitems, boxes, lay, arr, comp_base, cs, lg_s);
+    ++g_launches;
+    return cudaGetLastError();
+}
+cudaError_t launch_field_to_array4(const PaRowItem* items, int nitems, const PaBoxDev* boxes, const PaLayDev* lay, const PaA4Dev* arr,
+                                   int ncomp, const double* comp_base, long long cs, int lg_s, cudaStream_t st) {
+    if (nitems <= 0 || ncomp <= 0) return cudaSuccess;
+    PA_LAUNCH(dim3(array4_grid(nitems), ncomp), 256, 0, st, k_array4_copy<false>)(items, nitems, boxes, lay, arr, const_cast<double*>(comp_base),
+                                                                                cs, lg_s);
+    ++g_launches;
+    return cudaGetLastError();
+}
+
 __global__ void k_fill(double* __restrict__ p, long long n, double v) {
     for (long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x; c < n; c += (long long)gridDim.x * blockDim.x) p[c] = v;
 }

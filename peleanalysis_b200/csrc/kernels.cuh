@@ -81,6 +81,12 @@ cudaError_t launch_unpack_valid(const PaBoxDev* boxes, const PaLayDev* lay, cons
                                 long long ncells, const double* staging, double* comp_base, cudaStream_t st);
 cudaError_t launch_pack_valid(const PaBoxDev* boxes, const PaLayDev* lay, const long long* host_off, int nboxes,
                               long long ncells, const double* comp_base, double* staging, cudaStream_t st);
+// caller's device arrays <-> valid cells of comps [0, ncomp) of a level (comp_base = the field's first copied component):
+// one launch over every row item of the level and every component; lg_s = log2 of the lanes that share one row
+cudaError_t launch_array4_to_field(const PaRowItem* items, int nitems, const PaBoxDev* boxes, const PaLayDev* lay, const PaA4Dev* arr,
+                                   int ncomp, double* comp_base, long long cs, int lg_s, cudaStream_t st);
+cudaError_t launch_field_to_array4(const PaRowItem* items, int nitems, const PaBoxDev* boxes, const PaLayDev* lay, const PaA4Dev* arr,
+                                   int ncomp, const double* comp_base, long long cs, int lg_s, cudaStream_t st);
 cudaError_t launch_fill(double* p, long long n, double v, cudaStream_t st);
 
 // halo tags [tag0, tag1) covering cells [cell0, cell1) of the table's flattened enumeration; `comp0` = first component

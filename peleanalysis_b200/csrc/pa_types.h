@@ -109,6 +109,19 @@ struct PaFaceBlock {
     int cell0;        // first plane cell of the chunk, relative to the record's start
 };
 
+// a caller's device array (pa_array4) resolved against one local box: cell (i,j,k) relative to the box's low corner,
+// component m of the copied range, lives at p[i + j*js + k*ks + m*ns]
+struct PaA4Dev {
+    double* p;
+    long long js, ks, ns;
+};
+// device <-> field copy work item (pa_field_upload_device): rows [row0, row0+nrows) of local box `box`, row = k*ny + j
+struct PaRowItem {
+    int box;
+    int row0, nrows;
+    int pad;
+};
+
 // stencil work item: rows [y0, y0+ny) x planes [z0, z0+nz) of a local box, full x extent
 struct PaTile {
     int lev;

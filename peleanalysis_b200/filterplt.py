@@ -11,7 +11,7 @@ from typing import List, Optional, Sequence
 import numpy as np
 
 from .plotfile import Level, Plotfile
-from .stencilrun import download_level
+from .stencilrun import download_level, result_device, upload_device
 
 
 def level_fgr(base_fgr: int, ratios: Sequence[int], same_fgr_all_levels: bool, lev: int) -> int:
@@ -94,6 +94,17 @@ class FilterRun:
 
     def download_level(self, lev: int) -> np.ndarray:
         return download_level(self.P, self.hier, self.outputs, lev)
+
+    def upload_device(self, name: str, arrays_per_level, nghost: int = 0) -> None:
+        """variable `name` from device memory: per level, one CUDA array per box this rank owns of the RE-CHOPPED grids
+        (self.levels, self.hier.local_boxes); no host copy.  Asynchronous on the library stream."""
+        if name not in self.names:
+            raise ValueError("%r is not a filtered variable of this run (%s)" % (name, ", ".join(self.names)))
+        upload_device(self.hier, self.fin, self.names.index(name), arrays_per_level[:self.nlev], nghost)
+
+    def result_device(self, alloc=None):
+        """per level, per box of the re-chopped grids: torch CUDA tensor [ncomp][nz][ny][nx] (None for boxes of other ranks)"""
+        return result_device(self.hier, self.levels, self.outputs, alloc)
 
     def grown_input(self, lev: int, box: int, comp: int) -> np.ndarray:
         """the input FAB with the field's ghost width; only the level's own ngrow layers are filled"""

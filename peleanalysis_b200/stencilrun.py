@@ -34,6 +34,48 @@ def download_level(P, hier, outputs, lev: int) -> np.ndarray:
     return out
 
 
+def upload_device(hier, field, comp: int, arrays_per_level, nghost: int = 0) -> None:
+    """arrays_per_level[l]: one CUDA array per box this rank owns on level l (hier.local_boxes[l] order), [nz][ny][nx] or a
+    FAB [ncomp][nz][ny][nx] whose component 0 is taken (pick another by slicing), each holding its box grown by nghost cells"""
+    for l, arrays in enumerate(arrays_per_level):
+        if hier.local_boxes[l] or len(arrays):
+            field.upload_level_device(l, comp, arrays, nghost)
+
+
+def _torch_empty(shape):
+    import torch
+    return torch.empty(shape, dtype=torch.float64, device="cuda")
+
+
+def result_device(hier, levels, outputs, alloc=None):
+    """per level, per box: a torch CUDA tensor [len(outputs)][nz][ny][nx] (None for boxes of other ranks); row k is
+    component outputs[k] = (field, comp), zeros where outputs[k] is None.  Written on the library stream.  alloc(shape) may
+    supply other CUDA arrays (sliceable along the first axis, with zero_() on a row)."""
+    alloc = alloc or _torch_empty
+    res = []
+    for l, lv in enumerate(levels):
+        row: List[Optional[object]] = [None] * len(lv.boxes)
+        loc = hier.local_boxes[l]
+        for b in loc:
+            lo, hi = lv.boxes[b]
+            row[b] = alloc((len(outputs), hi[2] - lo[2] + 1, hi[1] - lo[1] + 1, hi[0] - lo[0] + 1))
+        k = 0
+        while loc and k < len(outputs):
+            if outputs[k] is None:
+                for b in loc:
+                    row[b][k].zero_()
+                k += 1
+                continue
+            f, c = outputs[k]
+            n = 1                  # one call per run of consecutive components of one field
+            while k + n < len(outputs) and outputs[k + n] is not None and outputs[k + n][0] is f and outputs[k + n][1] == c + n:
+                n += 1
+            f.download_level_device(l, c, [row[b][k:k + n] for b in loc], ncomp=n)
+            k += n
+        res.append(row)
+    return res
+
+
 class _Run:
     def __init__(self, P, pf: Plotfile, is_per, sym_dir, rank: int, nranks: int, multigpu, wrap, peer_links: bool):
         self.P, self.pf = P, pf
@@ -60,6 +102,18 @@ class _Run:
     def download_level(self, lev: int) -> np.ndarray:
         return download_level(self.P, self.hier, self.outputs, lev)
 
+    def upload_device(self, name: str, arrays_per_level, nghost: int = 0) -> None:
+        """input variable `name` from device memory: per level, one CUDA array per box this rank owns (see
+        stencilrun.upload_device); no host copy.  Asynchronous on the library stream."""
+        if name not in self.names:
+            raise ValueError("%r is not an input of this run (%s)" % (name, ", ".join(self.names)))
+        upload_device(self.hier, self._input, self.names.index(name), arrays_per_level, nghost)
+
+    def result_device(self, alloc=None):
+        """per level, per box: torch CUDA tensor [len(out_names)][nz][ny][nx] in out_names order (zeros in the slots the
+        tool does not write; None for boxes of other ranks); no host copy.  Enqueued on the library stream."""
+        return result_device(self.hier, self.levels, self.outputs, alloc)
+
     def cells(self) -> int:
         return self.hier.num_cells
 
@@ -76,6 +130,7 @@ class GradRun(_Run):
         self.fout = P.Field(self.hier, 4 * self.nvar, 0)
         self.out_names = [s for v in self.names for s in (v + "_gx", v + "_gy", v + "_gz", "||grad" + v + "||")]
         self.outputs = [(self.fout, k) for k in range(4 * self.nvar)]
+        self._input = self.fin
         if peer_links and nranks > 1:
             self.mg.map_peers(self.fin)
         self.exchange = self.mg.SlabExchange(self.fin, self.nvar, **self.kw) if nranks > 1 else None
@@ -126,6 +181,7 @@ class CurvatureRun(_Run):
             self.opts_phi = P.CurvOpts.from_buffer_copy(opts)
             self.opts_phi.prog_min, self.opts_phi.prog_max = 0.0, 1.0
         self.state = P.Field(self.hier, nst + 2 if self.do_smooth else nst, 1)
+        self._input = self.state
         self.nout = P.curvature_num_outputs(opts)
         self.fout = P.Field(self.hier, self.nout, 1)
         v = progress
